@@ -2,10 +2,11 @@
 """Benchmark of the KD training hot path (BASELINE.json: "KD-train samples/sec (Glow 32x32x3, ...); logp delta").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B | --global-batch G] [--impl reference]
-                    [--workload NAME]
+                    [--workload NAME] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1). A step = one KD training step (student fwd, teacher fwd, multi-level
-latent MSE, backward, clip 30, Adam) on one synthetic CIFAR-shaped batch per rank. Prints ONE JSON line.
+latent MSE, backward, clip 30, Adam) on one synthetic CIFAR-shaped batch per rank, from the seeded initial student.
+Prints ONE JSON line.
 
 --impl reference times the reference's CPU algorithm (oracle/ port; the reference is a Python script tree that does not
 travel to the GPU box) and imports NOTHING from the product package.
@@ -71,6 +72,33 @@ def synthetic_images(n, shape, seed):
     g = torch.Generator().manual_seed(seed)
     H, W, C = shape
     return torch.floor(torch.rand(n, C, H, W, generator=g) * 256.0) / 256.0 - 0.5
+
+
+DUMP_BYTES = 64 << 20
+
+
+def host_outputs(arrays):
+    """The arrays --dump-outputs writes, copied to the host as float32 (float64 stays float64). An array larger than its
+    share of DUMP_BYTES is replaced by a fixed sample of its flattened elements (seeded, sorted indices), so that two
+    builds run with the same arguments can be compared element for element."""
+    share = DUMP_BYTES // len(arrays)
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach()
+        a = a.double() if a.dtype == torch.float64 else a.float()
+        cap = share // a.element_size()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.flatten()[idx.to(a.device)]
+        out[name] = a.cpu()
+    return out
+
+
+def dump_outputs(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.numpy())
 
 
 def peaks():
@@ -412,7 +440,7 @@ def run_fwd_inv(args, wl, cfg_desc, warmup):
         with torch.no_grad():
             outs, bpd, _ = model(x.clone(), None)
             rev = model(z=outs[-1], temperature=0.0, reverse=True)
-            res["bpd"], res["x"] = bpd, rev[-1]
+            res["bpd"], res["z"], res["x"] = bpd, outs[-1], rev[-1]
             res["stat"] = torch.stack([bpd.mean(), rev[-1].abs().mean()])
 
     x.copy_(dev_pool[0])
@@ -449,6 +477,8 @@ def run_fwd_inv(args, wl, cfg_desc, warmup):
     barrier()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1) / args.steps
+    # the last timed step's per-sample bpd / nll, final latent and reconstruction
+    outputs = host_outputs({k: res[k] for k in ("bpd", "z", "x")}) if args.dump_outputs and rank == 0 else None
     # end to end: pinned host batch -> H2D -> both passes -> D2H of (mean bpd, mean |x|)
     barrier()
     t0 = time.perf_counter()
@@ -467,6 +497,8 @@ def run_fwd_inv(args, wl, cfg_desc, warmup):
         delta = logp_delta(model, cfg if not maf else None, maf, wl, device)
         v, cms, cores, sample = cpu_fwd_inv(wl, args.cpu_batch, 1)
         cpu_base = {"value": v, "unit": "samples/s", "cores": cores, "kind": "port", "sample": sample}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         gb = B * world
         cfg_desc.update(per_gpu_batch=B, global_batch=gb, parallelism=f"dp{world}", cuda_graphs=True,
@@ -607,7 +639,7 @@ def cpu_batch_for(args, wl):
 def run_reference_arm(args, wl, cfg_desc):
     """bench.py --impl reference: the reference's CPU algorithm for this workload (oracle/ port) on the box's host
     cores, bounded sample per step; rank 0 only. No product code is imported on this path."""
-    n = max(1, min(args.steps, 3))
+    n = args.steps
     if wl.get("mode") == "fwd_inv":
         metric = "fwd_inv_samples_per_sec"
         value, ms, cores, sample = cpu_fwd_inv(wl, args.cpu_batch, n)
@@ -669,7 +701,12 @@ def main():
     ap.add_argument("--ncu-step", action="store_true",
                     help="profiling aid: warm up, then run ONE eager step between cudaProfilerStart/Stop and exit "
                          "(use with ncu --profile-from-start off); prints no bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy "
+                         "(float32, at most 64 MB; a seeded sample of an array too large for its share)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "native" or args.ncu_step):
+        ap.error("--dump-outputs applies to the timed native path")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -740,6 +777,19 @@ def main():
         torch.cuda.profiler.stop()
         print(json.dumps({"ncu_step": True, "batch": B, "losses": trainer.losses.cpu().tolist()}))
         return
+    # Every warm-up and timed step trains the seeded initial student with fresh optimiser state. The kernels reduce with
+    # float atomics, so a step's results vary from run to run in the last bits; a step that continued from the previous
+    # step's weights would take that variation as input, and Adam's early updates (about lr * sign(g)) move a weight
+    # whose gradient is within rounding of zero by up to 2 lr. Restarting keeps the inputs of every step identical from
+    # run to run, and its results equal up to rounding; the work of a step is unchanged. The restart (one copy of the
+    # flat parameters, memsets of the optimiser state) is timed with the step: 47 us of a 38 ms step of the default
+    # workload (B200, 1000 W).
+    p0 = trainer.opt.p.clone()
+
+    def restart():
+        trainer.opt.p.copy_(p0)
+        trainer.reset_state()
+
     # logp delta of the student as initialised, before any step (rank 0, single GPU, with the CPU legs)
     delta = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -763,6 +813,7 @@ def main():
     # ---- device-resident timing (value)
     for i in range(warmup):
         trainer.x.copy_(dev_pool[i % n_pool])
+        restart()
         trainer.step_device()
     sampler = ClockSampler(device.index or 0)
     barrier()
@@ -771,12 +822,20 @@ def main():
     e0.record()
     for i in range(args.steps):
         trainer.x.copy_(dev_pool[i % n_pool])
+        restart()
         trainer.step_device()
     e1.record()
     barrier()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1) / args.steps
     losses = trainer.losses.cpu().tolist()
+    # the last timed step's loss scalars (nll, kd, perceptual, loss) and the student's averaged gradient before clipping,
+    # flat in student.parameters() order. The updated weights are left out: Adam's first update is about lr * sign(g),
+    # not a result that agrees up to rounding.
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = host_outputs({"losses": trainer.losses,
+                                "student_grads": torch.cat([g.flatten() for g in trainer.opt.g_views])})
 
     # ---- end-to-end timing through the public API: pinned host batch -> H2D -> step -> D2H of the loss scalars
     for i in range(2):
@@ -809,6 +868,8 @@ def main():
                     "sample": f"2 KD train steps of {cb} samples, same model/config "
                               f"(oracle/ on torch CPU fp32, {cores} threads), {cms:.0f} ms/step"}
 
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         gb = B * world
         cfg_desc.update(per_gpu_batch=B, global_batch=gb, parallelism=f"dp{world}",
@@ -816,7 +877,9 @@ def main():
                         teacher_prefetch=("1 batch: the frozen teacher's forward of batch t+1 runs beside the student's "
                                           "step on batch t (same updates; one batch consumed and one update made per "
                                           "step)") if pipelined else "off",
-                        l2="per-step working set (activations ~GBs) exceeds the 126 MB L2; inputs rotate over 4 batches")
+                        l2="per-step working set (activations ~GBs) exceeds the 126 MB L2; inputs rotate over 4 batches",
+                        step_start="every warm-up and timed step starts from the seeded initial student and fresh Adam "
+                                   "state; the restart (parameter copy + optimiser-state memsets) is timed with it")
         out = {"metric": METRIC, "value": gb / (ms * 1e-3), "unit": "samples/s", "n_gpus": world,
                "steps": args.steps, "warmup": warmup, "ms_per_step": ms, "higher_is_better": True,
                "scaling": scaling_kind(args), "vs_baseline": None, "dtype": dtype,

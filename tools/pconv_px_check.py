@@ -1,6 +1,6 @@
 """The pixel-major Conv2dZeros + coupling kernel of the 4x4-map level (csrc/pconv_px.cu) against pconv_coupling_kernel<48>
 (NFK_PCONV_PX=0, run in a child process): outputs, saved conv outputs and log-dets must be bit-identical; then timing."""
-import os, subprocess, sys
+import os, subprocess, sys, tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch
@@ -30,10 +30,11 @@ if __name__ == "__main__":
         torch.save([run(*c) for c in CASES], sys.argv[2])
         sys.exit(0)
     mine = [run(*c) for c in CASES]
-    path = "/tmp/pconv_px_ref.pt"
-    subprocess.run([sys.executable, os.path.abspath(__file__), "child", path], env=dict(os.environ, NFK_PCONV_PX="0"),
-                   check=True, timeout=300)
-    ref = torch.load(path)
+    with tempfile.TemporaryDirectory() as tmp:
+        path = os.path.join(tmp, "pconv_px_ref.pt")
+        subprocess.run([sys.executable, os.path.abspath(__file__), "child", path],
+                       env=dict(os.environ, NFK_PCONV_PX="0"), check=True, timeout=300)
+        ref = torch.load(path)
     ok = True
     for c, a, b in zip(CASES, mine, ref):
         eq_y = torch.equal(a[0], b[0])
