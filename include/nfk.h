@@ -149,6 +149,18 @@ int nfk_coupling_bwd(const float* g_out, const float* g_ld, const float* z_out, 
 int nfk_affine1x1_bwd(const float* dy, const float* dcol, int K1p, const float* x, const float* Wf, float* dx,
                       float* dWf, float* dbf, int B, int C, int H, int W, void* stream);
 
+/* Backward of the INVERSE coupling (models/flows.py:185-193: zc2 = z2 / s - shift, ld -= sum log s), same layout and
+ * shape limits as nfk_coupling_bwd: g_zc = dL/dzc [B,C,H,W] (zc = the post-coupling tensor, z_out of the forward kernel
+ * run with reverse = 1), hsave its saved (shift, logit) pairs, g_ld [B]. Writes dz (z2 half dL/dz2 = g_zc2 / s, z1 half
+ * = g_zc1 -- the coupling net's share is added by nfk_col2im_add), the bf16 im2col of dh = (-g_zc2,
+ * -(g_zc2 * (zc2 + shift) + g_ld) * (1 - s)) [B*H*W, K3p] and dbias3 += sum dh (dbias3 zeroed by the caller). */
+int nfk_coupling_inv_bwd(const float* g_zc, const float* g_ld, const float* zc, const float* hsave, float* dz,
+                         void* dhcol, int K3p, float* dbias3, int B, int C, int H, int W, void* stream);
+
+/* dz[:, :C/2] += col2im(dcol) in place: the input gradient of the coupling net's first conv (3x3, pad 1) from the dgrad
+ * GEMM's output dcol [B*H*W, K1p] fp32 (column = tap*(C/2) + ci), for the inverse pass whose conv reads z1 directly. */
+int nfk_col2im_add(const float* dcol, int K1p, float* dz, int B, int C, int H, int W, void* stream);
+
 /* ---- Split2d (models/layers.py:293-313), prior / bpd (models/kd_flows.py:134-150), KD MSE (pl_module.py:266-282) */
 int nfk_split2d_fwd(const float* x, const float* w, const float* bias, const float* logs, float* z1_out, float* ld,
                     int B, int C, int H, int W, void* stream);

@@ -75,6 +75,8 @@ SIGNATURES: dict[str, list] = {
     "nfk_coupling_fwd": [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "nfk_coupling_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp],
     "nfk_affine1x1_bwd": [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "nfk_coupling_inv_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp],
+    "nfk_col2im_add": [_vp, _i, _vp, _i, _i, _i, _i, _vp],
     "nfk_split2d_fwd": [_vp] * 6 + [_i] * 4 + [_vp],
     "nfk_split2d_rev": [_vp] * 5 + [_f, _vp] + [_i] * 4 + [_vp],
     "nfk_split2d_bwd": [_vp] * 10 + [_i] * 4 + [_vp],

@@ -5,8 +5,10 @@
 //                  and the bf16 im2col matrix of y1 = y[:, :C/2] that feeds the first coupling conv (3x3, pad 1).
 //  coupling_fwd    col2im of the last conv's per-tap products P, + folded bias, then the affine coupling
 //                  z2 = (z2 + shift) * sigmoid(s + 2)  (or its inverse), log-det reduced per sample.
-//  coupling_bwd    gradient of the coupling wrt (z2, h) and the im2col matrix of dh for the dgrad / wgrad GEMMs.
+//  coupling_bwd    gradient of the coupling wrt (z2, h) and the im2col matrix of dh for the dgrad / wgrad GEMMs; the
+//                  same kernel with INV = true is the backward of the inverse coupling (coupling_inv_bwd).
 //  affine1x1_bwd   col2im of the first conv's input gradient, dx = W'^T dy, dW' and db' reductions.
+//  col2im_add      dz1 += col2im of the first conv's input gradient (inverse pass: the conv reads z1 directly).
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cstdint>
@@ -204,6 +206,40 @@ affine1x1_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wf, 
   copy_out_rows(out4, cst, npix, r16, rs16, tid);
 }
 
+// col2im of the first conv's input gradient, UN (pixel, channel) items per thread at a time: item i0 + u*ZT is
+// (pixel pl = i / CH, channel ci = i % CH) of the pixel range starting at global pixel m0, channel fastest so that the
+// CH lanes of a pixel read one contiguous segment of a dcol row per tap. out[u] = sum_tap dcol[m - off(tap), tap*CH+ci]
+// (0 for items >= nitems); all 9*UN loads of the (HBM-resident) dcol rows are in flight before the first add.
+template <int CH, int UN>
+__device__ __forceinline__ void col2im_gather(const float* __restrict__ dcol, int K1p, const Geo& g, long long m0,
+                                              int i0, int nitems, float (&out)[UN]) {
+  const int HWm = g.HW - 1, Wm = g.W - 1;
+  float v[UN][9];
+#pragma unroll
+  for (int u = 0; u < UN; ++u) {
+    const int i = i0 + u * ZT;
+    const bool live = i < nitems;
+    const int pl = live ? i / CH : 0, ci = live ? i - pl * CH : 0;
+    const long long m = m0 + pl;
+    const int rem = static_cast<int>(m & HWm);
+    const int yy = rem >> g.lgW, xx = rem & Wm;
+#pragma unroll
+    for (int tap = 0; tap < 9; ++tap) {
+      const int ddy = tap / 3 - 1, ddx = tap % 3 - 1;
+      const int ny = yy - ddy, nx = xx - ddx;
+      v[u][tap] = (live && ny >= 0 && ny < g.H && nx >= 0 && nx < g.W)
+                      ? __ldg(dcol + (m - ddy * g.W - ddx) * K1p + tap * CH + ci) : 0.f;
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < UN; ++u) {
+    float a = 0.f;
+#pragma unroll
+    for (int tap = 0; tap < 9; ++tap) a += v[u][tap];
+    out[u] = a;
+  }
+}
+
 // ------------------------------------------------------------------------------------------ coupling fwd / inv
 // No shared memory. Thread = (pixel, channel pair j), j fastest: the J lanes of a pixel read one contiguous C*4-byte
 // segment of that pixel's P row per tap (few 128-byte lines per warp request — the L1 wavefront count, not HBM, was
@@ -267,8 +303,10 @@ coupling_fwd_kernel(const float* __restrict__ P, int K3p, const float* __restric
 // wrt (z2, shift, logit) from the saved h; dh goes to a smem tile. Phase 2 (thread = pixel): the im2col matrix of dh
 // for the dgrad / wgrad GEMMs with compile-time (tap, channel) positions, staged and copied out in 16-byte coalesced
 // chunks. Bias-gradient sums stay in smem across groups: one global atomic per channel and CTA.
+// INV = true: backward of the INVERSE coupling zc2 = z2 / s - shift, ld -= sum log s (g_out = dL/dzc, z_out = zc):
+// dz2 = dzc2 / s, dshift = -dzc2, dlogit = -(dzc2 * (zc2 + shift) + g_ld) * (1 - s)   (z2 / s = zc2 + shift).
 // smem: dhs[C*ldp] dbs[C] | cst[tile * (K3p/8 + 1)] 16-byte chunks,  ldp = tile + 2*halo + 1
-template <int C>
+template <int C, bool INV>
 __global__ void __launch_bounds__(ZT)
 coupling_bwd_kernel(const float* __restrict__ g_out, const float* __restrict__ g_ld, const float* __restrict__ z_out,
                     const float* __restrict__ hsave, float* __restrict__ dy, __nv_bfloat16* __restrict__ dhcol,
@@ -342,11 +380,12 @@ coupling_bwd_kernel(const float* __restrict__ g_out, const float* __restrict__ g
         if (inr[u]) {
           float sg, lsv;
           sigmoid_logsigmoid(hh[u].y + 2.f, sg, lsv);
-          dsh = g2[u] * sg;
-          dlg = (g2[u] * o2[u] + glv[u]) * (1.f - sg);
+          dsh = INV ? -g2[u] : g2[u] * sg;
+          dlg = INV ? -(g2[u] * (o2[u] + hh[u].x) + glv[u]) * (1.f - sg) : (g2[u] * o2[u] + glv[u]) * (1.f - sg);
           if (ownv[u]) {
-            dy[lo[u]] = g1[u];  // z1 passes through; the coupling-net gradient is added by affine1x1_bwd
-            dy[lo[u] + (static_cast<long long>(J) << g.lgHW)] = dsh;        // dL/dy2
+            // z1 passes through; the coupling-net gradient is added by affine1x1_bwd (col2im_add in the inverse pass)
+            dy[lo[u]] = g1[u];
+            dy[lo[u] + (static_cast<long long>(J) << g.lgHW)] = INV ? g2[u] / sg : dsh;   // dL/dy2 (dL/dz2)
           }
         }
         const int jj = jjv[u];
@@ -429,7 +468,7 @@ affine1x1_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ dco
   float* xs = dys + C * ldp;
   float* acc = dys + tile_floats;   // tile_floats >= 2*C*ldp, and >= the slice-reduction scratch at the end
   const int tid = threadIdx.x;
-  const int HWm = g.HW - 1, Wm = g.W - 1;
+  const int HWm = g.HW - 1;
   const int ngroups = (g.B + g.ipc - 1) / g.ipc;
 
   for (int i = tid; i < C * C; i += ZT) {
@@ -475,36 +514,17 @@ affine1x1_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ dco
     }
     __syncthreads();
     if (dcol) {
-      // dy1[ci, m] += sum_tap dcol[m - off(tap), tap*CH + ci]; three items per thread at a time so that 27 loads of
-      // the (HBM-resident) dcol rows are in flight before the first add
+      // dy1[ci, m] += sum_tap dcol[m - off(tap), tap*CH + ci], three items per thread at a time
       constexpr int UN = 3;
       for (int i0 = tid; i0 < CH * npix; i0 += UN * ZT) {
-        float v[UN][9];
-#pragma unroll
-        for (int u = 0; u < UN; ++u) {
-          const int i = i0 + u * ZT;
-          const bool live = i < CH * npix;
-          const int pl = live ? i / CH : 0, ci = live ? i - pl * CH : 0;
-          const int rem = pl & HWm;
-          const int yy = rem >> g.lgW, xx = rem & Wm;
-          const long long m = (static_cast<long long>(b0) << g.lgHW) + pl;
-#pragma unroll
-          for (int tap = 0; tap < 9; ++tap) {
-            const int ddy = tap / 3 - 1, ddx = tap % 3 - 1;
-            const int ny = yy - ddy, nx = xx - ddx;
-            v[u][tap] = (live && ny >= 0 && ny < g.H && nx >= 0 && nx < g.W)
-                            ? __ldg(dcol + (m - ddy * g.W - ddx) * K1p + tap * CH + ci) : 0.f;
-          }
-        }
+        float a[UN];
+        col2im_gather<CH, UN>(dcol, K1p, g, static_cast<long long>(b0) << g.lgHW, i0, CH * npix, a);
 #pragma unroll
         for (int u = 0; u < UN; ++u) {
           const int i = i0 + u * ZT;
           if (i < CH * npix) {
             const int pl = i / CH, ci = i - pl * CH;
-            float a = 0.f;
-#pragma unroll
-            for (int tap = 0; tap < 9; ++tap) a += v[u][tap];
-            dys[ci * ldp + pl] += a;
+            dys[ci * ldp + pl] += a[u];
           }
         }
       }
@@ -590,6 +610,33 @@ affine1x1_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ dco
   for (int i = tid; i < C; i += ZT) atomicAdd(dbf + i, acc[C * C + i]);
 }
 
+// ------------------------------------------------------------------------------------------ col2im add
+// dz[:, :C/2] += col2im(dcol) in place. CTA = C2I_UN * ZT / CH consecutive pixels x CH channels = C2I_UN * ZT items,
+// one col2im_gather per thread; no shared memory. Reads dcol once (HBM-bound), read-modify-writes the z1 half of dz.
+constexpr int C2I_UN = 3;
+template <int C>
+__global__ void __launch_bounds__(ZT)
+col2im_add_kernel(const float* __restrict__ dcol, int K1p, float* __restrict__ dz, Geo g) {
+  pdl_launch_dependents();
+  pdl_wait();
+  constexpr int CH = C / 2;
+  constexpr int PPC = C2I_UN * ZT / CH;   // pixels per CTA (C2I_UN * ZT is a multiple of every CH)
+  const long long M = static_cast<long long>(g.B) << g.lgHW;
+  const long long m0 = static_cast<long long>(blockIdx.x) * PPC;
+  const int nitems = static_cast<int>(min(static_cast<long long>(PPC), M - m0)) * CH;
+  float a[C2I_UN];
+  col2im_gather<CH, C2I_UN>(dcol, K1p, g, m0, threadIdx.x, nitems, a);
+#pragma unroll
+  for (int u = 0; u < C2I_UN; ++u) {
+    const int i = threadIdx.x + u * ZT;
+    if (i < nitems) {
+      const int pl = i / CH, ci = i - pl * CH;
+      const long long m = m0 + pl;
+      dz[((((m >> g.lgHW) * C) + ci) << g.lgHW) + (m & (g.HW - 1))] += a[u];
+    }
+  }
+}
+
 static Geo make_geo(int B, int C, int H, int W, bool heavy) {
   Geo g;
   g.B = B; g.H = H; g.W = W; g.HW = H * W;
@@ -672,9 +719,12 @@ extern "C" int nfk_coupling_fwd(const float* P, int K3p, const float* bias3, flo
   return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
 }
 
-extern "C" int nfk_coupling_bwd(const float* g_out, const float* g_ld, const float* z_out, const float* hsave,
-                                float* dy, void* dhcol, int K3p, float* dbias3, int B, int C, int H, int W,
-                                void* stream) {
+namespace nfk {
+// Launch of coupling_bwd_kernel in either direction (the two entry points below share the shape limits and sizing).
+template <bool INV>
+static int coupling_bwd_launch(const float* g_out, const float* g_ld, const float* z_out, const float* hsave,
+                               float* dy, void* dhcol, int K3p, float* dbias3, int B, int C, int H, int W,
+                               void* stream) {
   if (B <= 0 || H <= 0 || W <= 0 || H * W > 4096 || K3p % 64 || K3p < 9 * C || !pow2(H) || !pow2(W))
     return NFK_ERR_SHAPE;
   if (!g_out || !g_ld || !z_out || !hsave || !dy || !dhcol || !dbias3) return NFK_ERR_ARG;
@@ -695,13 +745,26 @@ extern "C" int nfk_coupling_bwd(const float* g_out, const float* g_ld, const flo
   const int grid = groups < 4 * 148 ? groups : 4 * 148;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   NFK_DISPATCH_C(C, {
-    int rc = ensure_smem(coupling_bwd_kernel<CC>, smem);
+    int rc = ensure_smem(coupling_bwd_kernel<CC, INV>, smem);
     if (rc) return rc;
-    if (launch_pdl(coupling_bwd_kernel<CC>, dim3(grid), dim3(ZT), smem, st, g_out, g_ld, z_out, hsave, dy,
+    if (launch_pdl(coupling_bwd_kernel<CC, INV>, dim3(grid), dim3(ZT), smem, st, g_out, g_ld, z_out, hsave, dy,
                    static_cast<__nv_bfloat16*>(dhcol), K3p, dbias3, g, brows) != cudaSuccess)
       return NFK_ERR_LAUNCH;
   });
   return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
+}
+}  // namespace nfk
+
+extern "C" int nfk_coupling_bwd(const float* g_out, const float* g_ld, const float* z_out, const float* hsave,
+                                float* dy, void* dhcol, int K3p, float* dbias3, int B, int C, int H, int W,
+                                void* stream) {
+  return coupling_bwd_launch<false>(g_out, g_ld, z_out, hsave, dy, dhcol, K3p, dbias3, B, C, H, W, stream);
+}
+
+extern "C" int nfk_coupling_inv_bwd(const float* g_zc, const float* g_ld, const float* zc, const float* hsave,
+                                    float* dz, void* dhcol, int K3p, float* dbias3, int B, int C, int H, int W,
+                                    void* stream) {
+  return coupling_bwd_launch<true>(g_zc, g_ld, zc, hsave, dz, dhcol, K3p, dbias3, B, C, H, W, stream);
 }
 
 extern "C" int nfk_affine1x1_bwd(const float* dy, const float* dcol, int K1p, const float* x, const float* Wf,
@@ -722,6 +785,21 @@ extern "C" int nfk_affine1x1_bwd(const float* dy, const float* dcol, int K1p, co
     if (rc) return rc;
     if (launch_pdl(affine1x1_bwd_kernel<CC>, dim3(grid), dim3(ZT), smem, st, dy, dcol, K1p, x, Wf, dx, dWf, dbf, g,
                    tile_floats) != cudaSuccess)
+      return NFK_ERR_LAUNCH;
+  });
+  return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
+}
+
+extern "C" int nfk_col2im_add(const float* dcol, int K1p, float* dz, int B, int C, int H, int W, void* stream) {
+  if (B <= 0 || H <= 0 || W <= 0 || H * W > 4096 || !pow2(H) || !pow2(W) || K1p < 9 * (C / 2)) return NFK_ERR_SHAPE;
+  if (!dcol || !dz) return NFK_ERR_ARG;
+  Geo g = make_geo(B, C, H, W, false);
+  const long long M = static_cast<long long>(B) * H * W;
+  const long long ppc = C2I_UN * ZT / (C / 2);
+  const unsigned grid = static_cast<unsigned>((M + ppc - 1) / ppc);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  NFK_DISPATCH_C(C, {
+    if (launch_pdl(col2im_add_kernel<CC>, dim3(grid), dim3(ZT), 0, st, dcol, K1p, dz, g) != cudaSuccess)
       return NFK_ERR_LAUNCH;
   });
   return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;

@@ -171,12 +171,13 @@ def prep_for(step, reverse):
 
 
 def prepare_steps(layers, reverse):
-    """Batch every trainable LU-decomposed FlowStep in `layers` (called by FlowNet.encode/decode under grad)."""
+    """Batch every trainable FlowStep in `layers` (called by FlowNet.encode/decode under grad); reverse=True builds the
+    inverse-direction matrices, and PrepAllFn.backward then applies the inverse's chain rule."""
     if not torch.is_grad_enabled():
         return None
     steps = [l for l in layers if getattr(l, "_batched_prep_ok", None) is not None and l._batched_prep_ok()
              and l.actnorm.logs.requires_grad]
-    if len(steps) < 2 or (reverse and not steps[0].is_1d):   # gradients through the 2-D inverse are not built
+    if len(steps) < 2:
         return None
     return PrepCtx(steps, reverse).build()
 
@@ -347,23 +348,73 @@ def flowstep2d_forward(x, ld_in, k: StepConsts, hid, keep):
     return y, ld_out, (col, h1, h2 if keep else None, hsave, m1, m2)
 
 
-def flowstep2d_reverse(z, ld_in, k: StepConsts, hid):
+def flowstep2d_reverse(z, ld_in, k: StepConsts, hid, keep=False):
     """FlowStep.reverse_flow (reference models/flows.py:173-202): coupling^-1 -> invconv^-1 -> actnorm^-1.
-    k.Wf / k.bf / k.sl hold the INVERSE affine here."""
+    k.Wf / k.bf / k.sl hold the INVERSE affine here. keep=True (training) also returns what FlowStep2dReverseFn's
+    backward reads: (zc = the post-coupling tensor, col, h1, h2, hsave, m1, m2); the outputs are the same bits."""
     B, C, H, W = z.shape
     M, cin = B * H * W, C // 2
     K1p, K3p = ops.round_up(9 * cin, 64), ops.round_up(9 * C, 64)
     dev = z.device
     col = torch.empty(M, K1p, device=dev, dtype=BF16)
     ops.affine1x1_fwd(z, None, None, None, None, col, K1p, None, None, B, C, H, W)   # im2col of z1 only
-    _, h2, _, _ = _coupling_net(col, k, M, hid, K1p, K3p, keep=False)
+    h1, h2, m1, m2 = _coupling_net(col, k, M, hid, K1p, K3p, keep)
+    hsave = torch.empty(M, C, device=dev, dtype=F32) if keep else None
     zc = z.clone()
     ld_mid = ld_in.clone()
-    _conv3_coupling(h2, k, zc, None, ld_mid, B, C, H, W, hid, K3p, True)
+    _conv3_coupling(h2, k, zc, hsave, ld_mid, B, C, H, W, hid, K3p, True)
     x = torch.empty_like(z)
     ld_out = torch.empty_like(ld_mid)
     ops.affine1x1_fwd(zc, k.Wf, k.bf, k.sl, x, None, 0, ld_mid, ld_out, B, C, H, W)
+    if keep:
+        return x, ld_out, (zc, col, h1, h2, hsave, m1, m2)
     return x, ld_out
+
+
+def _grad_arena(C, hid, K1p, K3p, dev):
+    """One zero-filled arena for every accumulate-into buffer of a 2-D step's backward:
+    (arena, dbias3, dbias2, dbias1, dB3, dB2, dB1, dWf, dbf)."""
+    sizes = [C, hid, hid, K3p * hid, hid * hid, hid * K1p, C * C, C]
+    offs = [0]
+    for s in sizes:
+        offs.append(offs[-1] + ops.round_up(s, 4))
+    arena = torch.zeros(offs[-1], device=dev, dtype=F32)
+    dbias3, dbias2, dbias1, dB3, dB2, dB1, dWf, dbf = (arena[offs[i]:offs[i] + sizes[i]] for i in range(8))
+    return (arena, dbias3, dbias2, dbias1, dB3.view(K3p, hid), dB2.view(hid, hid), dB1.view(hid, K1p),
+            dWf.view(C, C), dbf)
+
+
+def _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena, M, hid,
+                           K1p, K3p):
+    """Backward of the coupling net (direction-independent): from the bf16 im2col of dh [M, K3p] to the first conv's
+    input gradient dcol [M, K1p] fp32 (returned), accumulating the three weight gradients and the two bias gradients.
+    Small batches issue the weight gradients on the second stream (see WGRAD_STREAM_MAX_M)."""
+    dev = dhcol.device
+    dpre2 = torch.empty(M, hid, device=dev, dtype=BF16)
+    dpre1 = torch.empty(M, hid, device=dev, dtype=BF16)
+    if USE_FUSED_CNET_BWD and ops.cnet_fused_supported(hid, K3p) and M >= 8192:
+        # both dgrads of the chain in ONE kernel: dpre2 stays in shared memory as the second GEMM's A operand
+        ops.cnet_bwd_fused(dhcol, K3p, B3T, B2T, m2, m1, dpre2, dpre1, dbias2, dbias1, M, hid)
+    else:
+        ops.gemm_nt(dhcol, B3T, M, hid, K3p, ops.EPI_MASK_BF16, dpre2, aux=m2, colsum=dbias2)
+        ops.gemm_nt(dpre2, B2T, M, hid, hid, ops.EPI_MASK_BF16, dpre1, aux=m1, colsum=dbias1)
+    if 0 < M <= WGRAD_STREAM_MAX_M:
+        cur, side = torch.cuda.current_stream(dev), _wgrad_stream(dev)
+        side.wait_stream(cur)                          # fork: dhcol / dpre2 / dpre1 and the zeroed arena exist
+        with torch.cuda.stream(side):
+            ops.gemm_tn(dhcol, h2, K3p, hid, M, dB3)
+            ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
+            ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
+        _wgrad_keepalive.append((dhcol, dpre2, dpre1, h1, h2, col, arena))
+        dcol = torch.empty(M, K1p, device=dev, dtype=F32)
+        ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
+    else:
+        ops.gemm_tn(dhcol, h2, K3p, hid, M, dB3)
+        ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
+        dcol = torch.empty(M, K1p, device=dev, dtype=F32)
+        ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
+        ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
+    return dcol
 
 
 class FlowStep2dFn(torch.autograd.Function):
@@ -394,42 +445,13 @@ class FlowStep2dFn(torch.autograd.Function):
         _join_wgrads(dev)      # the previous step's weight gradients (before anything here can reuse their buffers)
         g_out = torch.zeros_like(x) if g_out is None else g_out.contiguous()
         g_ld = torch.zeros(B, device=dev, dtype=F32) if g_ld is None else g_ld.contiguous()
-        # one zero-filled arena for every accumulate-into buffer of this step
-        sizes = [C, hid, hid, K3p * hid, hid * hid, hid * K1p, C * C, C]
-        offs = [0]
-        for s in sizes:
-            offs.append(offs[-1] + ops.round_up(s, 4))
-        arena = torch.zeros(offs[-1], device=dev, dtype=F32)
-        dbias3, dbias2, dbias1, dB3, dB2, dB1, dWf, dbf = (arena[offs[i]:offs[i] + sizes[i]] for i in range(8))
-        dB3, dB2, dB1, dWf = dB3.view(K3p, hid), dB2.view(hid, hid), dB1.view(hid, K1p), dWf.view(C, C)
+        arena, dbias3, dbias2, dbias1, dB3, dB2, dB1, dWf, dbf = _grad_arena(C, hid, K1p, K3p, dev)
 
         dy = torch.empty_like(x)
         dhcol = torch.empty(M, K3p, device=dev, dtype=BF16)
         ops.coupling_bwd(g_out, g_ld, z_out, hsave, dy, dhcol, K3p, dbias3, B, C, H, W)
-        dpre2 = torch.empty(M, hid, device=dev, dtype=BF16)
-        dpre1 = torch.empty(M, hid, device=dev, dtype=BF16)
-        if USE_FUSED_CNET_BWD and ops.cnet_fused_supported(hid, K3p) and M >= 8192:
-            # both dgrads of the chain in ONE kernel: dpre2 stays in shared memory as the second GEMM's A operand
-            ops.cnet_bwd_fused(dhcol, K3p, B3T, B2T, m2, m1, dpre2, dpre1, dbias2, dbias1, M, hid)
-        else:
-            ops.gemm_nt(dhcol, B3T, M, hid, K3p, ops.EPI_MASK_BF16, dpre2, aux=m2, colsum=dbias2)
-            ops.gemm_nt(dpre2, B2T, M, hid, hid, ops.EPI_MASK_BF16, dpre1, aux=m1, colsum=dbias1)
-        if 0 < M <= WGRAD_STREAM_MAX_M:
-            cur, side = torch.cuda.current_stream(dev), _wgrad_stream(dev)
-            side.wait_stream(cur)                          # fork: dhcol / dpre2 / dpre1 and the zeroed arena exist
-            with torch.cuda.stream(side):
-                ops.gemm_tn(dhcol, h2, K3p, hid, M, dB3)
-                ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
-                ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
-            _wgrad_keepalive.append((dhcol, dpre2, dpre1, h1, h2, col, arena))
-            dcol = torch.empty(M, K1p, device=dev, dtype=F32)
-            ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
-        else:
-            ops.gemm_tn(dhcol, h2, K3p, hid, M, dB3)
-            ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
-            dcol = torch.empty(M, K1p, device=dev, dtype=F32)
-            ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
-            ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
+        dcol = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
+                                      M, hid, K1p, K3p)
         dx = torch.empty_like(x)
         ops.affine1x1_bwd(dy, dcol, K1p, x, Wf, dx, dWf, dbf, B, C, H, W)
 
@@ -438,6 +460,52 @@ class FlowStep2dFn(torch.autograd.Function):
         ctx.pctx.grads[ctx.idx] = (dWf, C, dbf, g_ld, B, float(H * W))
         ctx.pctx.cgrads[ctx.idx] = (dB1, dbias1, dB2, dbias2, dB3, dbias3)
         return (dx, g_ld, None, None, None, None)
+
+
+class FlowStep2dReverseFn(torch.autograd.Function):
+    """Differentiable 2-D FlowStep INVERSE (reference models/flows.py:173-202), the counterpart of FlowStep2dFn for the
+    perceptual term, whose gradient reaches the student through its inverse pass (pl_module.py:229-243). pctx holds
+    the inverse-direction affine; the deposits feed PrepAllFn.backward's inverse chain rule.
+
+    z = [z1, z2], h = NN(z1), zc2 = z2 / s - shift, x = Wf zc + bf. Backward: dzc = Wf^T g_x (affine1x1_bwd, also dWf,
+    dbf), dz2 = dzc2 / s and dh (coupling_inv_bwd), the coupling net's backward to dcol, dz1 = dzc1 + col2im(dcol)."""
+
+    @staticmethod
+    def forward(ctx, z, ld_in, hid, token, pctx, idx):
+        z = z.contiguous()
+        Wf, bf, sl = pctx.consts[idx]
+        k = StepConsts(Wf, bf, sl, *pctx.cops[idx])
+        x, ld_out, (zc, col, h1, h2, hsave, m1, m2) = flowstep2d_reverse(z, ld_in.contiguous(), k, hid, keep=True)
+        ctx.hid = hid
+        ctx.pctx, ctx.idx = pctx, idx
+        ctx.save_for_backward(zc, col, h1, h2, hsave, m1, m2, Wf, k.B1T, k.B2T, k.B3T)
+        return x, ld_out
+
+    @staticmethod
+    def backward(ctx, g_x, g_ld):
+        (zc, col, h1, h2, hsave, m1, m2, Wf, B1T, B2T, B3T) = ctx.saved_tensors
+        hid = ctx.hid
+        B, C, H, W = zc.shape
+        M, cin = B * H * W, C // 2
+        K1p, K3p = ops.round_up(9 * cin, 64), ops.round_up(9 * C, 64)
+        dev = zc.device
+        _join_wgrads(dev)
+        g_x = torch.zeros_like(zc) if g_x is None else g_x.contiguous()
+        g_ld = torch.zeros(B, device=dev, dtype=F32) if g_ld is None else g_ld.contiguous()
+        arena, dbias3, dbias2, dbias1, dB3, dB2, dB1, dWf, dbf = _grad_arena(C, hid, K1p, K3p, dev)
+
+        dzc = torch.empty_like(zc)
+        ops.affine1x1_bwd(g_x, None, K1p, zc, Wf, dzc, dWf, dbf, B, C, H, W)
+        dz = torch.empty_like(zc)
+        dhcol = torch.empty(M, K3p, device=dev, dtype=BF16)
+        ops.coupling_inv_bwd(dzc, g_ld, zc, hsave, dz, dhcol, K3p, dbias3, B, C, H, W)
+        dcol = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
+                                      M, hid, K1p, K3p)
+        ops.col2im_add(dcol, K1p, dz, B, C, H, W)
+
+        ctx.pctx.grads[ctx.idx] = (dWf, C, dbf, g_ld, B, float(H * W))
+        ctx.pctx.cgrads[ctx.idx] = (dB1, dbias1, dB2, dbias2, dB3, dbias3)
+        return (dz, g_ld, None, None, None, None)
 
 
 # ------------------------------------------------------------------------------------------------ Split2d
@@ -504,6 +572,21 @@ def split2d_reverse(z1, w, bias, logs, eps, temperature):
     out = torch.empty(B, 2 * CH, H, W, device=z1.device, dtype=F32)
     ops.split2d_rev(z1.contiguous(), w, bias, logs, eps, temperature, out, B, 2 * CH, H, W)
     return out
+
+
+class Split2dReverseFn(torch.autograd.Function):
+    """Split2d reverse under autograd: cat(z1, z2) with z2 ~ N(mean(z1), exp(logs(z1)) * T) sampled by the split2d_rev
+    kernel. The reference samples with torch.normal, whose derivative with respect to mean and std is zero, so z2 is a
+    constant to autograd: z1 gets the pass-through half of the gradient and the Split2d parameters get none."""
+
+    @staticmethod
+    def forward(ctx, z1, w, bias, logs, eps, temperature):
+        ctx.ch = z1.shape[1]
+        return split2d_reverse(z1, w.detach(), bias.detach(), logs.detach(), eps, temperature)
+
+    @staticmethod
+    def backward(ctx, g):
+        return g[:, :ctx.ch], None, None, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------ prior -> bpd

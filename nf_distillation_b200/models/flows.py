@@ -233,10 +233,12 @@ class FlowStep(nn.Module):
                                                      self.hidden_channels, keep=False)
         else:
             if needs_grad:
-                raise NotImplementedError("gradients through the 2-D inverse pass are not built (image configs use "
-                                          "perceptual weight 0, conf/training/cifar.yaml:17-20)")
-            z, ld_out = Fn.flowstep2d_reverse(input.contiguous(), ld.contiguous(), self._consts(True),
-                                              self.hidden_channels)
+                # the perceptual term's gradient reaches the student through its inverse pass (pl_module.py:229-243)
+                pctx, idx, token = Fn.prep_for(self, True)
+                z, ld_out = Fn.FlowStep2dReverseFn.apply(input, ld, self.hidden_channels, token, pctx, idx)
+            else:
+                z, ld_out = Fn.flowstep2d_reverse(input.contiguous(), ld.contiguous(), self._consts(True),
+                                                  self.hidden_channels)
         return z, (ld_out if want_ld else None)
 
     def _forward_precise(self, input, ld, want_ld, reverse, needs_grad):
@@ -250,7 +252,8 @@ class FlowStep(nn.Module):
                 z, ld_out = precise.FlowStep2dX3Fn.apply(input, ld, self.hidden_channels, *fp)
             else:
                 if needs_grad:
-                    raise NotImplementedError("gradients through the 2-D inverse pass are not built")
+                    raise NotImplementedError("gradients through the 2-D inverse pass are built for the bf16 "
+                                              "precision only")
                 k = self._consts(True)
                 z, ld_out = precise.flowstep2d_reverse_x3(input.contiguous(), ld.contiguous(), self.hidden_channels,
                                                           (k.Wf, k.bf, k.sl), *fp[3:])

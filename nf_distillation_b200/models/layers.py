@@ -260,8 +260,12 @@ class Split2d(nn.Module):
             eps = None
             if temperature is None or temperature != 0:
                 eps = torch.randn_like(input)
-            out = Fn.split2d_reverse(input, w.detach(), b.detach(), l.detach(), eps,
-                                     1.0 if temperature is None else float(temperature))
+            T = 1.0 if temperature is None else float(temperature)
+            if torch.is_grad_enabled():
+                # z2 is a constant to autograd like the reference's torch.normal draw: only z1's half flows back
+                out = Fn.Split2dReverseFn.apply(input, w.detach(), b.detach(), l.detach(), eps, T)
+            else:
+                out = Fn.split2d_reverse(input, w.detach(), b.detach(), l.detach(), eps, T)
             return out, logdet
         ld = _as_logdet(logdet, B, input.device)
         if ld is None:

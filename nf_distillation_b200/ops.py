@@ -198,6 +198,19 @@ def affine1x1_bwd(dy, dcol, K1p, x, Wf, dx, dWf, dbf, B, C, H, W):
           "nfk_affine1x1_bwd")
 
 
+def coupling_inv_bwd(g_zc, g_ld, zc, hsave, dz, dhcol, K3p, dbias3, B, C, H, W):
+    """Backward of the inverse affine coupling (include/nfk.h: nfk_coupling_inv_bwd)."""
+    _count()
+    check(LIB.nfk_coupling_inv_bwd(_p(g_zc), _p(g_ld), _p(zc), _p(hsave), _p(dz), _p(dhcol), K3p, _p(dbias3), B, C,
+                                   H, W, _st()), "nfk_coupling_inv_bwd")
+
+
+def col2im_add(dcol, K1p, dz, B, C, H, W):
+    """dz[:, :C/2] += col2im(dcol) in place (include/nfk.h: nfk_col2im_add)."""
+    _count()
+    check(LIB.nfk_col2im_add(_p(dcol), K1p, _p(dz), B, C, H, W, _st()), "nfk_col2im_add")
+
+
 def split2d_fwd(x, w, bias, logs, z1_out, ld, B, C, H, W, z1_sq=None):
     """z1_sq (optional): the squeezed copy of z1 written in the same pass (the next level's input)."""
     _count()
