@@ -203,6 +203,19 @@ int nfk_pconv_coupling_supported(int C, int H, int W, int hid);
 int nfk_pconv_coupling_fwd(const void* h2, const void* B3, int K3p, const float* bias3, float* y, float* hsave,
                            float* ld, int B, int C, int H, int W, int hid, int reverse, void* stream);
 
+/* ---- first conv of the coupling net, input gradient, fused with its col2im and nfk_affine1x1_bwd
+ * (csrc/dgrad_col2im.cu): P^T = B1T * dpre1^T on tcgen05 with whole images as the N tile, then per pixel
+ * dys = dy + col2im(P) on the y1 half (dy on the y2 half), dx = W'^T dys, dWf += dys x^T, dbf += sum dys.
+ * dpre1 [B*H*W, hid] bf16 (the masked gradient at the first conv's output), B1T [K1p, hid] bf16 (rows tap*(C/2) + ci,
+ * as built by nfk_coupling_prep), K1p = round_up(9*C/2, 64); dy, x, dx [B,C,H,W] fp32, Wf [C,C]; dWf, dbf are
+ * accumulated (zeroed by the caller). dx is bit-identical to nfk_gemm_nt_bf16 (NFK_EPI_F32) + nfk_affine1x1_bwd.
+ * Supported shapes (nfk_conv1_dgrad_affine_bwd_supported): C = 12 with maps of <= 256 pixels, C = 24 with <= 128,
+ * C = 48 with <= 64; H, W powers of two; hid % 64 == 0. */
+int nfk_conv1_dgrad_affine_bwd_supported(int C, int H, int W, int hid);
+int nfk_conv1_dgrad_affine_bwd(const void* dpre1, const void* B1T, int K1p, const float* dy, const float* x,
+                               const float* Wf, float* dx, float* dWf, float* dbf, int B, int C, int H, int W, int hid,
+                               void* stream);
+
 /* ---- 1-D (tabular) FlowStep, fused (is_1d branches of models/flows.py:37-52,142-202, models/layers.py:410-411) --
  * Weights are packed once per optimiser step by nfk_flow1d_pack from the fused affine (nfk_invconv_prep with
  * transpose=1, forward or inverse direction) and the six nn.Linear layers of get_block_1d:

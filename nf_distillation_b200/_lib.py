@@ -100,6 +100,8 @@ SIGNATURES: dict[str, list] = {
     "nfk_cnet_fwd_fused_ranged": [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _i, _vp],
     "nfk_pconv_coupling_supported": [_i, _i, _i, _i],
     "nfk_pconv_coupling_fwd": [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp],
+    "nfk_conv1_dgrad_affine_bwd_supported": [_i, _i, _i, _i],
+    "nfk_conv1_dgrad_affine_bwd": [_vp] * 9 + [_i] * 5 + [_vp],
     "nfk_made_prep": [_vp] * 5 + [_i] * 4 + [_vp] * 6 + [_i, _vp],
     "nfk_made_prep_bwd": [_vp] * 5 + [_i] * 3 + [_vp] * 3 + [_vp],
     "nfk_rows_to_bf16": [_vp, _i, _i, _i, _vp, _vp],

@@ -298,7 +298,9 @@ typedef CUresult (*EncodeTiledFn3)(CUtensorMap*, CUtensorMapDataType, cuuint32_t
                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static int pc_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows) {
+// bf16 [rows, cols] K-major tensor map, 64-column (128-byte, SWIZZLE_128B) boxes of box_rows rows; also used by
+// dgrad_col2im.cu
+int pc_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows) {
   static EncodeTiledFn3 fn = nullptr;
   if (!fn) {
     void* p = nullptr;

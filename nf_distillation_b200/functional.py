@@ -18,6 +18,7 @@ F32 = torch.float32
 USE_FUSED_CNET = os.environ.get("NFK_FUSED_CNET", "1") != "0"
 USE_FUSED_PCONV = os.environ.get("NFK_FUSED_PCONV", "1") != "0"
 USE_FUSED_CNET_BWD = os.environ.get("NFK_FUSED_CNET_BWD", "1") != "0"
+USE_FUSED_DGRAD1 = os.environ.get("NFK_FUSED_DGRAD1", "1") != "0"
 
 # ---- weight gradients beside the backward chain (small batches) --------------------------------------------------
 # A student FlowStep's backward is a chain of dependent launches: coupling_bwd -> both dgrads -> (3 weight-gradient
@@ -386,8 +387,9 @@ def _grad_arena(C, hid, K1p, K3p, dev):
 
 def _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena, M, hid,
                            K1p, K3p):
-    """Backward of the coupling net (direction-independent): from the bf16 im2col of dh [M, K3p] to the first conv's
-    input gradient dcol [M, K1p] fp32 (returned), accumulating the three weight gradients and the two bias gradients.
+    """Backward of the coupling net (direction-independent): from the bf16 im2col of dh [M, K3p] to the masked
+    gradient at the first conv's output dpre1 [M, hid] bf16 (returned; the first conv's input gradient is left to the
+    caller, see _conv1_dgrad), accumulating the three weight gradients and the two bias gradients.
     Small batches issue the weight gradients on the second stream (see WGRAD_STREAM_MAX_M)."""
     dev = dhcol.device
     dpre2 = torch.empty(M, hid, device=dev, dtype=BF16)
@@ -406,14 +408,17 @@ def _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, db
             ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
             ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
         _wgrad_keepalive.append((dhcol, dpre2, dpre1, h1, h2, col, arena))
-        dcol = torch.empty(M, K1p, device=dev, dtype=F32)
-        ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
     else:
         ops.gemm_tn(dhcol, h2, K3p, hid, M, dB3)
         ops.gemm_tn(dpre2, h1, hid, hid, M, dB2)
-        dcol = torch.empty(M, K1p, device=dev, dtype=F32)
-        ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
         ops.gemm_tn(dpre1, col, hid, K1p, M, dB1)
+    return dpre1
+
+
+def _conv1_dgrad(dpre1, B1T, M, K1p, hid):
+    """The first conv's input gradient as per-tap products dcol [M, K1p] fp32 (column = tap*(C/2) + ci)."""
+    dcol = torch.empty(M, K1p, device=dpre1.device, dtype=F32)
+    ops.gemm_nt(dpre1, B1T, M, K1p, hid, ops.EPI_F32, dcol)
     return dcol
 
 
@@ -450,10 +455,15 @@ class FlowStep2dFn(torch.autograd.Function):
         dy = torch.empty_like(x)
         dhcol = torch.empty(M, K3p, device=dev, dtype=BF16)
         ops.coupling_bwd(g_out, g_ld, z_out, hsave, dy, dhcol, K3p, dbias3, B, C, H, W)
-        dcol = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
-                                      M, hid, K1p, K3p)
+        dpre1 = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
+                                       M, hid, K1p, K3p)
         dx = torch.empty_like(x)
-        ops.affine1x1_bwd(dy, dcol, K1p, x, Wf, dx, dWf, dbf, B, C, H, W)
+        if USE_FUSED_DGRAD1 and ops.conv1_dgrad_affine_bwd_supported(C, H, W, hid):
+            # conv#1 dgrad + col2im + affine1x1_bwd in one kernel: the fp32 dcol never goes through HBM
+            ops.conv1_dgrad_affine_bwd(dpre1, B1T, K1p, dy, x, Wf, dx, dWf, dbf, B, C, H, W, hid)
+        else:
+            dcol = _conv1_dgrad(dpre1, B1T, M, K1p, hid)
+            ops.affine1x1_bwd(dy, dcol, K1p, x, Wf, dx, dWf, dbf, B, C, H, W)
 
         # the parameter-space chain rules (fused affine, folded conv operands) are deferred to PrepAllFn.backward:
         # one batched launch each for all steps of the pass
@@ -499,9 +509,9 @@ class FlowStep2dReverseFn(torch.autograd.Function):
         dz = torch.empty_like(zc)
         dhcol = torch.empty(M, K3p, device=dev, dtype=BF16)
         ops.coupling_inv_bwd(dzc, g_ld, zc, hsave, dz, dhcol, K3p, dbias3, B, C, H, W)
-        dcol = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
-                                      M, hid, K1p, K3p)
-        ops.col2im_add(dcol, K1p, dz, B, C, H, W)
+        dpre1 = _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, dbias1, dB3, dB2, dB1, arena,
+                                       M, hid, K1p, K3p)
+        ops.col2im_add(_conv1_dgrad(dpre1, B1T, M, K1p, hid), K1p, dz, B, C, H, W)
 
         ctx.pctx.grads[ctx.idx] = (dWf, C, dbf, g_ld, B, float(H * W))
         ctx.pctx.cgrads[ctx.idx] = (dB1, dbias1, dB2, dbias2, dB3, dbias3)

@@ -272,6 +272,18 @@ def pconv_coupling_fwd(h2, B3, K3p, bias3, y, hsave, ld, B, C, H, W, hid, revers
                                      int(reverse), _st()), "nfk_pconv_coupling_fwd")
 
 
+def conv1_dgrad_affine_bwd_supported(C, H, W, hid):
+    return bool(LIB.nfk_conv1_dgrad_affine_bwd_supported(C, H, W, hid))
+
+
+def conv1_dgrad_affine_bwd(dpre1, B1T, K1p, dy, x, Wf, dx, dWf, dbf, B, C, H, W, hid):
+    """First conv's input gradient (per-tap tcgen05 products + col2im) fused with affine1x1_bwd; dWf / dbf accumulate."""
+    assert dpre1.dtype == torch.bfloat16 and B1T.dtype == torch.bfloat16
+    _count()
+    check(LIB.nfk_conv1_dgrad_affine_bwd(_p(dpre1), _p(B1T), K1p, _p(dy), _p(x), _p(Wf), _p(dx), _p(dWf), _p(dbf), B,
+                                         C, H, W, hid, _st()), "nfk_conv1_dgrad_affine_bwd")
+
+
 def flow1d_supported(D, Cc, hid, training=False):
     return bool(LIB.nfk_flow1d_supported(D, Cc, hid, int(training)))
 
