@@ -299,6 +299,30 @@ int nfk_made_inverse_resident(const float* u_in, const void* wstream, const floa
                               const float* b3, const int* jobs, int njobs, int push, int N3p, float* x,
                               const float* ld_in, float* ld_out, int B, int D, int H, int Dp, int flip, int mtiles,
                               void* stream);
+/* Gradients of the inverse: given g_x [B,D] (input order) and g_ld [B] (NULL = 0) for x, ld_out = inverse(u_in, ld_in),
+ * ONE reverse sweep d = D-1 .. 0 gives g_u [B,D] (output order), g_ld_in = g_ld, and dout [B,N3p] bf16 =
+ * [mubar | alphabar | 0] with db3 += its column sums; dout is the upstream of the forward's parameter chain at x
+ * (the dgrad / wgrad GEMMs of nfk_made_affine_bwd's dout). out [B,N3p] fp32 and the ReLU masks m1, m2 (word-major
+ * [H/32][B], the EPI_BIAS_RELU_BF16 aux output) come from the forward recomputed at x. db3 must be zeroed.
+ *  nfk_made_inv_bwd_update — pass d of the D-pass form: c [B, ldc] fp32 = the network's input gradient for the dout
+ *     rows finished so far (NULL at d = D-1); writes g_u[:, d], dout[:, d], dout[:, D+d] and adds to db3. dout must be
+ *     zero-initialised before pass D-1.
+ *  nfk_made_inverse_bwd_jobs / _pack / _resident — the one-launch form (csrc/maf_inverse.cu), the mirror of the pull
+ *     kernel with the same three steps: the HOST planner (same cnt1/cnt2 as nfk_made_inverse_jobs, same 8 int32 per
+ *     job; [6] = the job's first 16-wide k-chunk; push form does not exist), the pack of the transposed operands
+ *     B1T [Dp,H], B2T [H,H], B3T [H,N3p] of nfk_made_prep (with_t = 1), and the launch (mtiles as above).
+ *     _supported: 1 if the shapes fit (H, N3p multiples of 64). */
+int nfk_made_inv_bwd_update(const float* c, int ldc, const float* g_x, const float* g_ld, const float* out, int N3p,
+                            const float* u_in, float* g_u, void* dout, float* db3, int B, int D, int d, int flip,
+                            void* stream);
+int nfk_made_inverse_bwd_supported(int D, int H, int N3p);
+int nfk_made_inverse_bwd_jobs(const int* cnt1, const int* cnt2, int D, int H, int N3p, int* jobs, int cap);
+int nfk_made_inverse_bwd_pack(const int* jobs, int njobs, const void* B1T, const void* B2T, const void* B3T, int D,
+                              int H, int N3p, void* wstream, void* stream);
+int nfk_made_inverse_bwd_resident(const float* g_x, const float* g_ld, const float* out, const void* m1,
+                                  const void* m2, const float* u_in, const void* wstream, const int* jobs, int njobs,
+                                  float* g_u, void* dout, float* db3, int B, int D, int H, int N3p, int flip,
+                                  int mtiles, void* stream);
 
 /* Fused conv#1 -> conv#2 of the coupling network: h2 = relu(relu(col*B1^T + b1)*B2^T + b2) in ONE kernel (CTA
  * pairs; h1 stays in shared memory as the tcgen05 A operand of conv#2). col [M,K1p] bf16, B1 [512,K1p], B2 [512,512]

@@ -113,6 +113,11 @@ SIGNATURES: dict[str, list] = {
     "nfk_made_inverse_jobs": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i],
     "nfk_made_inverse_pack": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "nfk_made_inverse_resident": [_vp] * 6 + [_i] * 3 + [_vp] * 3 + [_i] * 6 + [_vp],
+    "nfk_made_inv_bwd_update": [_vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "nfk_made_inverse_bwd_supported": [_i, _i, _i],
+    "nfk_made_inverse_bwd_jobs": [_vp, _vp, _i, _i, _i, _vp, _i],
+    "nfk_made_inverse_bwd_pack": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "nfk_made_inverse_bwd_resident": [_vp] * 8 + [_i] + [_vp] * 3 + [_i] * 6 + [_vp],
     "nfk_kd_nll_loss_scratch_floats": [_i],
     "nfk_kd_nll_loss_fwd": [_vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _vp, _vp, _f, _f, _f, _i, _vp, _vp, _vp, _vp, _vp],
     "nfk_kd_nll_loss_bwd": [_vp, _vp, _i, _vp, _vp, _f, _vp, _f, _f, _f, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],

@@ -163,6 +163,44 @@ __global__ void made_inv_update_kernel(float* __restrict__ x, __nv_bfloat16* __r
   }
 }
 
+// Gradients of the sequential inverse, pass d (d = D-1 .. 0; the mirror of made_inv_update): with c = the input
+// gradient of the network at x for the dout rows finished so far (c[:, d], NULL = zero),
+//   mubar_d = g_x,d + c_d,  v_d = e^{alpha_d} mubar_d,  alphabar_d = v_d u_d + g_ld;  g_u[:, d] = v_d (output order),
+// dout[:, d] and dout[:, D + d] = bf16(mubar_d, alphabar_d), db3[d], db3[D + d] += their column sums (fp32 values,
+// a fixed order within the block, one atomic per block).
+__global__ void made_inv_bwd_update_kernel(const float* __restrict__ c, int ldc, const float* __restrict__ g_x,
+                                           const float* __restrict__ g_ld, const float* __restrict__ out, int N3p,
+                                           const float* __restrict__ u_in, float* __restrict__ g_u,
+                                           __nv_bfloat16* __restrict__ dout, float* __restrict__ db3, int B, int D,
+                                           int d, int flip) {
+  __shared__ float part[2][8];
+  const int b = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  float mub = 0.f, alb = 0.f;
+  if (b < B) {
+    const long long r = b;
+    mub = g_x[r * D + d] + (c ? c[r * ldc + d] : 0.f);
+    const float v = expf(out[r * N3p + D + d]) * mub;
+    alb = v * u_in[r * D + (flip ? D - 1 - d : d)] + (g_ld ? g_ld[b] : 0.f);
+    g_u[r * D + (flip ? D - 1 - d : d)] = v;
+    dout[r * N3p + d] = __float2bfloat16_rn(mub);
+    dout[r * N3p + D + d] = __float2bfloat16_rn(alb);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    mub += __shfl_xor_sync(0xffffffffu, mub, o);
+    alb += __shfl_xor_sync(0xffffffffu, alb, o);
+  }
+  if (lane == 0) {
+    part[0][w] = mub;
+    part[1][w] = alb;
+  }
+  __syncthreads();
+  if (threadIdx.x < 2) {
+    float s = 0.f;
+    for (int i = 0; i < (blockDim.x >> 5); ++i) s += part[threadIdx.x][i];
+    atomicAdd(db3 + (threadIdx.x ? D + d : d), s);
+  }
+}
+
 }  // namespace nfk
 
 using namespace nfk;
@@ -232,5 +270,15 @@ extern "C" int nfk_made_inv_update(float* x, void* xb, int Dp, const float* u_in
   if (!x || !xb || !u_in || !out || (ld_out && !ld_in)) return NFK_ERR_ARG;
   made_inv_update_kernel<<<(B + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(
       x, static_cast<__nv_bfloat16*>(xb), Dp, u_in, out, N3p, ld_in, ld_out, B, D, i, flip, last);
+  return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
+}
+
+extern "C" int nfk_made_inv_bwd_update(const float* c, int ldc, const float* g_x, const float* g_ld, const float* out,
+                                       int N3p, const float* u_in, float* g_u, void* dout, float* db3, int B, int D,
+                                       int d, int flip, void* stream) {
+  if (B <= 0 || D <= 0 || d < 0 || d >= D || N3p < 2 * D || (c && ldc < D)) return NFK_ERR_SHAPE;
+  if (!g_x || !out || !u_in || !g_u || !dout || !db3) return NFK_ERR_ARG;
+  made_inv_bwd_update_kernel<<<(B + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      c, ldc, g_x, g_ld, out, N3p, u_in, g_u, static_cast<__nv_bfloat16*>(dout), db3, B, D, d, flip);
   return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
 }

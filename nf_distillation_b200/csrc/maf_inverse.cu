@@ -629,6 +629,331 @@ __global__ void __launch_bounds__(384) made_inverse_push_kernel(const MiArgs p) 
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// REVERSE SOLVE (gradients of the inverse): the mirror of the pull kernel. With upstream g_x [B, D] and g_ld [B], one
+// sweep d = D-1 .. 0 over the outputs gives every gradient of the inverse:
+//   c_d = sum_{k > d} (dmu_k/dx_d . mubar_k + dalpha_k/dx_d . alphabar_k)    (VJP of the rows already final)
+//   v_d = e^{alpha_d} (g_x,d + c_d),  mubar_d = g_x,d + c_d,  alphabar_d = v_d u_d + g_ld,   g_u = v (output order)
+// c_d is a masked VJP whose order the degrees fix, the exact transpose of the order in which the pull kernel finalises
+// units: layer-2 units of degree d + 1 get g2 = m2 . (dout[:, outputs > d] B3), then layer-1 units of degree d + 1 get
+// g1 = m1 . (g2[:, degree >= d + 1] B2), then c_d = g1[:, degree >= d + 1] B1[:, d]. Every pre-activation gradient
+// is final once (~ one backward pass of work). A warp keeps, for its samples, the bf16 dout rows finished so far and
+// g2 / g1 in shared memory (the roundings the dgrad GEMM epilogues apply); the weights are the transposed operands of
+// nfk_made_prep (B3T, B2T, B1T rows), streamed job by job through the same byte ring as the forward. A job's k range
+// starts at its first k-chunk that can be non-zero (descriptor word w, bits [16,32)). Tiles that straddle two degrees
+// are evaluated at both steps: their not-yet-final columns meet masked-zero weights only.
+struct MibArgs {
+  const float* g_x;             // [B, D] input order
+  const float* g_ld;            // [B] or null
+  const float* out;             // [B, N3p] (mu | alpha) at x, fp32
+  const uint32_t *m1, *m2;      // ReLU masks at x, word-major [H / 32][B]
+  const float* u_in;            // [B, D] layer output order (the inverse's input)
+  const unsigned char* wstream; // nfk_made_inverse_bwd_pack
+  const int4* jobs;
+  int njobs, ring_bytes;
+  float* g_u;                   // [B, D] output order
+  __nv_bfloat16* dout;          // [B, N3p] = [mubar | alphabar | 0]
+  float* db3;                   // [>= 2D] += column sums of dout (fp32 values before rounding)
+  int B, D, H, N3p, flip;
+};
+
+template <int MT>
+__global__ void __launch_bounds__(288) made_inverse_bwd_resident_kernel(const MibArgs p) {
+  extern __shared__ __align__(128) unsigned char mi_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, cwarps = (blockDim.x >> 5) - 1;
+  const int D = p.D, H = p.H, N3p = p.N3p, HW = H >> 5;
+  const int ldo = N3p + 8, ldh = H + 8;
+  constexpr int R = MT * 16;
+  const int act_bytes = R * (ldo + 2 * ldh) * 2;
+  const int per_warp = act_bytes + 2 * HW * R * 4 + N3p * 4;   // + masks [2][HW][R] + column sums [N3p]
+  uint64_t* full = reinterpret_cast<uint64_t*>(mi_smem + p.ring_bytes);
+  uint64_t* empty = full + MI_SLOTS;
+  uint4* jobs_s = reinterpret_cast<uint4*>(mi_smem + p.ring_bytes + 256);
+  unsigned char* act = mi_smem + p.ring_bytes + 256 + p.njobs * 16;
+  const uint32_t ring_s = smem_u32(mi_smem);
+  for (int i = threadIdx.x; i < p.njobs; i += blockDim.x) jobs_s[i] = mi_pack_job(__ldg(p.jobs + 2 * i), __ldg(p.jobs + 2 * i + 1));
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < MI_SLOTS; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], cwarps);
+    }
+    fence_mbar_init();
+  }
+  __syncthreads();
+
+  const int ctiles = (p.B + R * cwarps - 1) / (R * cwarps);
+  const int my_tiles = (ctiles - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
+  const int njobs = p.njobs;
+
+  if (warp == cwarps) {
+    // ---------------- producer: identical to the pull kernel's
+    int slot = 0, par = 0, q = 0;
+    for (int tile = 0; tile < my_tiles; ++tile) {
+      for (int j = 0; j < njobs; ++j, ++q) {
+        const uint4 cur = jobs_s[j];
+        int back = cur.y >> 16;
+        if (back > MI_SLOTS) back = MI_SLOTS;
+        if (q >= back) {
+          const int ws = slot >= back ? slot - back : slot - back + MI_SLOTS;
+          mbar_wait(&empty[ws], slot >= back ? par : par ^ 1);
+        }
+        if (lane == 0) {
+          const uint32_t bytes = (cur.w & 0xffff) * 16;
+          if (bytes == 0) {
+            mbar_arrive(&full[slot]);
+          } else {
+            mbar_expect_tx(&full[slot], bytes);
+            mi_bulk_copy(ring_s + (cur.y & 0xffff) * 16, p.wstream + static_cast<size_t>(cur.z) * 16, bytes, &full[slot]);
+          }
+        }
+        if (++slot == MI_SLOTS) { slot = 0; par ^= 1; }
+      }
+    }
+    return;
+  }
+
+  // ---------------- consumers: warp w owns samples [base, base + R) of the CTA tile
+  const int g = lane >> 2, t = lane & 3;
+  unsigned char* mine = act + static_cast<size_t>(warp) * per_warp;
+  __nv_bfloat16* ds = reinterpret_cast<__nv_bfloat16*>(mine);     // dout rows [R][ldo]
+  __nv_bfloat16* g2 = ds + R * ldo;                               // [R][ldh]
+  __nv_bfloat16* g1 = g2 + R * ldh;                               // [R][ldh]
+  uint32_t* mk = reinterpret_cast<uint32_t*>(mine + act_bytes);   // m1 words [HW][R], then m2 words [HW][R]
+  float* csum = reinterpret_cast<float*>(mk + 2 * HW * R);        // this warp's column sums, every tile
+  for (int i = lane; i < N3p; i += 32) csum[i] = 0.f;
+  const int lrow = lane & 15, lcol = (lane >> 4) * 8;
+  const uint32_t ds_lane = smem_u32(ds + lrow * ldo + lcol);
+  const uint32_t g2_lane = smem_u32(g2 + lrow * ldh + lcol);
+  const uint32_t g1_lane = smem_u32(g1 + lrow * ldh + lcol);
+  const uint32_t b_row = (lane & 7) + ((lane >> 4) << 3), b_col = ((lane >> 3) & 1) * 16;
+
+  int slot = 0, par = 0;
+  for (int tile = 0; tile < my_tiles; ++tile) {
+    const long long base = ((static_cast<long long>(tile) * gridDim.x + blockIdx.x) * cwarps + warp) * R;
+    long long brow[MT][2];       // lanes t == 0: this lane's samples (-1 past the batch end)
+    float gl[MT][2], nx[MT][2][3];   // g_ld; next step's (g_x, alpha, u), requested a whole step ahead
+    {
+      uint4* z = reinterpret_cast<uint4*>(ds);
+      const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+      for (int i = lane; i < act_bytes / 16; i += 32) z[i] = zero;   // scratch columns must be finite
+      for (int i = lane; i < HW * R; i += 32) {
+        const int w = i / R, s = i - w * R;
+        const long long b = base + s;
+        mk[i] = b < p.B ? __ldg(p.m1 + static_cast<long long>(w) * p.B + b) : 0u;
+        mk[HW * R + i] = b < p.B ? __ldg(p.m2 + static_cast<long long>(w) * p.B + b) : 0u;
+      }
+#pragma unroll
+      for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {
+          const long long b = base + mt * 16 + g + 8 * hh;
+          brow[mt][hh] = (t == 0 && b < p.B) ? b : -1;
+          const bool ok = brow[mt][hh] >= 0;
+          gl[mt][hh] = (ok && p.g_ld) ? __ldg(p.g_ld + b) : 0.f;
+          nx[mt][hh][0] = ok ? __ldg(p.g_x + b * D + D - 1) : 0.f;
+          nx[mt][hh][1] = ok ? __ldg(p.out + b * N3p + 2 * D - 1) : 0.f;
+          nx[mt][hh][2] = ok ? __ldg(p.u_in + b * D + (p.flip ? 0 : D - 1)) : 0.f;
+        }
+      __syncwarp();
+    }
+    for (int j = 0; j < njobs; ++j) {
+      const uint4 jd = jobs_s[j];
+      const uint32_t cur = jd.x;
+      const int phase = cur & 3, kch = (cur >> 3) & 255, row0 = cur >> 11, k0 = jd.w >> 16;
+      uint32_t b_addr = ring_s + (jd.y & 0xffff) * 16 + b_row * (kch * 32 + 16) + b_col;
+
+      if (phase < 2) {
+        // phase 1: g2[:, row0 .. row0 + 16) = m2 . (dout . B3T rows); phase 0: g1 = m1 . (g2 . B2T rows)
+        const bool two = (cur & 4) != 0;
+        uint32_t a_addr = (phase == 1 ? ds_lane : g2_lane) + k0 * 32;
+        const int lda_bytes = (phase == 1 ? ldo : ldh) * 2;
+        float acc[MT][2][2][4];
+#pragma unroll
+        for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+          for (int n = 0; n < 2; ++n)
+#pragma unroll
+            for (int c = 0; c < 2; ++c)
+#pragma unroll
+              for (int e = 0; e < 4; ++e) acc[mt][n][c][e] = 0.f;
+        mbar_wait(&full[slot], par);
+        uint32_t a0[MT][4], a1[MT][4], b0[4], b1[4];
+        if (kch > 0) {
+          mi_ldsm_x4<0>(b_addr, b0);
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt) mi_ldsm_x4<0>(a_addr + mt * 16 * lda_bytes, a0[mt]);
+        }
+        int kc = kch;
+        for (; kc >= 2; kc -= 2, a_addr += 64, b_addr += 64) {
+          mi_ldsm_x4<32>(b_addr, b1);
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt) mi_ldsm_x4<32>(a_addr + mt * 16 * lda_bytes, a1[mt]);
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt) {
+            mi_mma(acc[mt][0][0], a0[mt], b0[0], b0[1]);
+            mi_mma(acc[mt][1][0], a0[mt], b0[2], b0[3]);
+          }
+          if (kc > 2) {
+            mi_ldsm_x4<64>(b_addr, b0);
+#pragma unroll
+            for (int mt = 0; mt < MT; ++mt) mi_ldsm_x4<64>(a_addr + mt * 16 * lda_bytes, a0[mt]);
+          }
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt) {
+            mi_mma(acc[mt][0][1], a1[mt], b1[0], b1[1]);
+            mi_mma(acc[mt][1][1], a1[mt], b1[2], b1[3]);
+          }
+        }
+        if (kc) {
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt) {
+            mi_mma(acc[mt][0][0], a0[mt], b0[0], b0[1]);
+            mi_mma(acc[mt][1][0], a0[mt], b0[2], b0[3]);
+          }
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[slot]);
+        __nv_bfloat16* o = (phase == 1 ? g2 : g1) + row0 + 2 * t;
+        const uint32_t* mw = mk + (phase == 1 ? HW * R : 0);
+        const int c0 = row0 + 2 * t, c1 = c0 + 8;
+#pragma unroll
+        for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+          for (int hh = 0; hh < 2; ++hh) {
+            const int s = mt * 16 + g + 8 * hh;
+            const uint32_t w0 = mw[(c0 >> 5) * R + s] >> (c0 & 31);
+            __nv_bfloat162 v = __floats2bfloat162_rn((w0 & 1u) ? acc[mt][0][0][2 * hh] + acc[mt][0][1][2 * hh] : 0.f,
+                                                     (w0 & 2u) ? acc[mt][0][0][2 * hh + 1] + acc[mt][0][1][2 * hh + 1] : 0.f);
+            *reinterpret_cast<__nv_bfloat162*>(o + s * ldh) = v;
+            if (two) {
+              const uint32_t w1 = mw[(c1 >> 5) * R + s] >> (c1 & 31);
+              v = __floats2bfloat162_rn((w1 & 1u) ? acc[mt][1][0][2 * hh] + acc[mt][1][1][2 * hh] : 0.f,
+                                        (w1 & 2u) ? acc[mt][1][0][2 * hh + 1] + acc[mt][1][1][2 * hh + 1] : 0.f);
+              *reinterpret_cast<__nv_bfloat162*>(o + s * ldh + 8) = v;
+            }
+          }
+        __syncwarp();
+      } else {
+        // step d: c_d = g1[:, k0 .. H) . B1T[d, k0 .. H) (job row 0), then row d of every gradient
+        const int d = row0;
+        float cur_v[MT][2][3];
+#pragma unroll
+        for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+          for (int hh = 0; hh < 2; ++hh) {
+            const long long b = brow[mt][hh];
+#pragma unroll
+            for (int e = 0; e < 3; ++e) cur_v[mt][hh][e] = nx[mt][hh][e];
+            const bool ok = b >= 0 && d > 0;
+            nx[mt][hh][0] = ok ? __ldg(p.g_x + b * D + d - 1) : 0.f;
+            nx[mt][hh][1] = ok ? __ldg(p.out + b * N3p + D + d - 1) : 0.f;
+            nx[mt][hh][2] = ok ? __ldg(p.u_in + b * D + (p.flip ? D - d : d - 1)) : 0.f;
+          }
+        float acc[MT][4][4];
+#pragma unroll
+        for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+#pragma unroll
+            for (int e = 0; e < 4; ++e) acc[mt][c][e] = 0.f;
+        uint32_t a_addr = g1_lane + k0 * 32;
+        mbar_wait(&full[slot], par);
+        uint32_t a[2][MT][4][4], b[2][4][2];
+        auto load_group = [&](int buf, int n) {
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            if (c < n) {
+              if (c == 0) mi_ldsm_x2<0>(b_addr, b[buf][0]);
+              if (c == 1) mi_ldsm_x2<32>(b_addr, b[buf][1]);
+              if (c == 2) mi_ldsm_x2<64>(b_addr, b[buf][2]);
+              if (c == 3) mi_ldsm_x2<96>(b_addr, b[buf][3]);
+#pragma unroll
+              for (int mt = 0; mt < MT; ++mt) {
+                if (c == 0) mi_ldsm_x4<0>(a_addr + mt * 16 * ldh * 2, a[buf][mt][0]);
+                if (c == 1) mi_ldsm_x4<32>(a_addr + mt * 16 * ldh * 2, a[buf][mt][1]);
+                if (c == 2) mi_ldsm_x4<64>(a_addr + mt * 16 * ldh * 2, a[buf][mt][2]);
+                if (c == 3) mi_ldsm_x4<96>(a_addr + mt * 16 * ldh * 2, a[buf][mt][3]);
+              }
+            }
+          a_addr += 128;
+          b_addr += 128;
+        };
+        auto mma_group = [&](int buf, int n) {
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            if (c < n) {
+#pragma unroll
+              for (int mt = 0; mt < MT; ++mt) mi_mma(acc[mt][c], a[buf][mt][c], b[buf][c][0], b[buf][c][1]);
+            }
+        };
+        int kc = kch;
+        if (kc > 0) load_group(0, kc < 4 ? kc : 4);
+        while (kc > 0) {
+          const int n0 = kc < 4 ? kc : 4, r1 = kc - n0;
+          if (r1 > 0) load_group(1, r1 < 4 ? r1 : 4);
+          mma_group(0, n0);
+          if (r1 <= 0) break;
+          const int n1 = r1 < 4 ? r1 : 4, r2 = r1 - n1;
+          if (r2 > 0) load_group(0, r2 < 4 ? r2 : 4);
+          mma_group(1, n1);
+          kc = r2;
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[slot]);
+        float smu = 0.f, sal = 0.f;
+        if (t == 0) {   // lanes t == 0 hold column 0 (c_d) of samples g and g + 8
+#pragma unroll
+          for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh) {
+              const float c = (acc[mt][0][2 * hh] + acc[mt][1][2 * hh]) + (acc[mt][2][2 * hh] + acc[mt][3][2 * hh]);
+              const float mub = cur_v[mt][hh][0] + c;
+              const float v = expf(cur_v[mt][hh][1]) * mub;
+              const float alb = v * cur_v[mt][hh][2] + gl[mt][hh];
+              const __nv_bfloat16 bm = __float2bfloat16_rn(mub), ba = __float2bfloat16_rn(alb);
+              const int s = mt * 16 + g + 8 * hh;
+              ds[s * ldo + d] = bm;
+              ds[s * ldo + D + d] = ba;
+              const long long b = brow[mt][hh];
+              if (b >= 0) {
+                p.g_u[b * D + (p.flip ? D - 1 - d : d)] = v;
+                p.dout[b * N3p + d] = bm;
+                p.dout[b * N3p + D + d] = ba;
+                smu += mub;
+                sal += alb;
+              }
+            }
+        }
+        // column sums: a fixed order over the warp's samples, then over its tiles
+#pragma unroll
+        for (int o = 4; o < 32; o <<= 1) {
+          smu += __shfl_xor_sync(0xffffffffu, smu, o);
+          sal += __shfl_xor_sync(0xffffffffu, sal, o);
+        }
+        if (lane == 0) {
+          csum[d] += smu;
+          csum[D + d] += sal;
+        }
+        __syncwarp();
+      }
+      if (++slot == MI_SLOTS) { slot = 0; par ^= 1; }
+    }
+    const int pad = N3p - 2 * D;   // dout's padding columns are zero
+    for (int i = lane; i < R * pad; i += 32) {
+      const int s = i / pad;
+      const long long b = base + s;
+      if (b < p.B) p.dout[b * N3p + 2 * D + (i - s * pad)] = __float2bfloat16_rn(0.f);
+    }
+  }
+  // db3: the consumer warps' sums in warp order, one atomic per column per CTA
+  asm volatile("bar.sync 1, %0;" ::"r"(cwarps * 32) : "memory");
+  for (int i = threadIdx.x; i < 2 * D; i += cwarps * 32) {
+    float s = 0.f;
+    for (int w = 0; w < cwarps; ++w) s += reinterpret_cast<const float*>(act + static_cast<size_t>(w) * per_warp + act_bytes + 2 * HW * R * 4)[i];
+    atomicAdd(p.db3 + i, s);
+  }
+}
+
 // Packed weight stream: every job's bytes exactly as the inverse kernels want them in shared memory — rows of
 // (kch * 32) weight bytes + 16 bytes of padding (zero), rows the job does not own zeroed, for a push-mode layer-2 job
 // followed (128-byte aligned) by its two push-table tiles B3[r][row0 .. row0 + 16) regrouped as [tile][r][8].
@@ -666,7 +991,34 @@ __global__ void made_inverse_pack_kernel(const int4* __restrict__ jobs, const __
   }
 }
 
+// Packed weight stream of the reverse solve: rows of the transposed operands from the job's first k-chunk on (phase
+// 1: B3T [H, N3p], phase 0: B2T [H, H], phase 2: row d of B1T [Dp, H]), same row layout as above.
+__global__ void made_inverse_bwd_pack_kernel(const int4* __restrict__ jobs, const __nv_bfloat16* __restrict__ B1T,
+                                             const __nv_bfloat16* __restrict__ B2T,
+                                             const __nv_bfloat16* __restrict__ B3T, int H, int N3p,
+                                             unsigned char* __restrict__ wstream) {
+  const int4 a = jobs[2 * blockIdx.x], b = jobs[2 * blockIdx.x + 1];
+  if (b.y == 0) return;
+  const int phase = a.x & 3, two = (a.x >> 2) & 1, kch = a.x >> 3, row0 = a.y, k0 = b.z;
+  uint4* dst = reinterpret_cast<uint4*>(wstream + static_cast<size_t>(b.x) * 16);
+  const int per_row = kch * 2 + 1;
+  const int rows = phase == 2 ? 1 : (two ? 16 : 8);
+  const __nv_bfloat16* src = phase == 0 ? B2T + static_cast<size_t>(row0) * H
+                             : phase == 1 ? B3T + static_cast<size_t>(row0) * N3p
+                                          : B1T + static_cast<size_t>(row0) * H;
+  const int ld = phase == 1 ? N3p : H;
+  for (int i = threadIdx.x; i < rows * per_row; i += blockDim.x) {
+    const int r = i / per_row, c = i - r * per_row;
+    dst[i] = c < kch * 2 ? *reinterpret_cast<const uint4*>(src + static_cast<size_t>(r) * ld + k0 * 16 + c * 8)
+                         : make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+
 static inline int mi_per_warp_bytes(int mt, int H, int Dp) { return mt * 16 * ((Dp + 8) + 2 * (H + 8)) * 2; }
+// reverse solve: dout rows, g2, g1 (bf16), the two ReLU masks of the warp's samples, its column sums of dout
+static inline int mib_per_warp_bytes(int mt, int H, int N3p) {
+  return mt * 16 * ((N3p + 8) + 2 * (H + 8)) * 2 + 2 * (H / 32) * mt * 16 * 4 + N3p * 4;
+}
 static inline int mi_per_warp_bytes_push(int H, int Dp) { return 16 * ((Dp + 8) + (H + 8)) * 2; }
 static inline int mi_rows_bytes(int rows, int kch) { return (rows * (kch * 32 + 16) + 127) & ~127; }
 // bytes of a job in the weight ring. pull: its rows (nothing for kch == 0). push: layer-1 job = its rows, layer-2 job =
@@ -690,12 +1042,7 @@ static constexpr int MI_SMEM_MAX = 227 * 1024;
 
 // Weight ring size for a layer shape: what is left after the barriers, the job table (the biases) and as many one-tile
 // warps as fit next to a ring of two or three largest jobs.
-static int mi_ring_bytes(int H, int Dp, int njobs, int push, int N3p) {
-  const int kmax = (H > Dp ? H : Dp) / 16;
-  const int biggest = push ? mi_rows_bytes(16, kmax) + 2 * N3p * 16 : mi_rows_bytes(16, kmax);
-  const int avail = MI_SMEM_MAX - mi_side_bytes(njobs, push ? 2 * H + N3p : 0);
-  const int per_warp = push ? mi_per_warp_bytes_push(H, Dp) : mi_per_warp_bytes(1, H, Dp);
-  const int max_warps = push ? 11 : 8;
+static int mi_ring_fit(int biggest, int avail, int per_warp, int max_warps) {
   // room for four (else three) of the largest jobs when that still leaves 8 warps — with two, the copy of job j + 2
   // cannot start before job j is released and its latency shows when jobs are few and large (D = 6); a ring of exactly
   // three wastes its tail on jobs of unequal size — else for two
@@ -707,6 +1054,52 @@ static int mi_ring_bytes(int H, int Dp, int njobs, int push, int N3p) {
   int ring = (avail - warps * per_warp) & ~127;
   if (ring > (1 << 20) - 128) ring = (1 << 20) - 128;   // offsets are stored in 16 bits of 16-byte units
   return ring;
+}
+
+static int mi_ring_bytes(int H, int Dp, int njobs, int push, int N3p) {
+  const int kmax = (H > Dp ? H : Dp) / 16;
+  const int biggest = push ? mi_rows_bytes(16, kmax) + 2 * N3p * 16 : mi_rows_bytes(16, kmax);
+  const int avail = MI_SMEM_MAX - mi_side_bytes(njobs, push ? 2 * H + N3p : 0);
+  const int per_warp = push ? mi_per_warp_bytes_push(H, Dp) : mi_per_warp_bytes(1, H, Dp);
+  return mi_ring_fit(biggest, avail, per_warp, push ? 11 : 8);
+}
+
+// reverse solve: the largest job multiplies 16 rows over max(H, N3p) columns
+static int mib_ring_bytes(int H, int N3p, int njobs) {
+  const int kmax = (H > N3p ? H : N3p) / 16;
+  return mi_ring_fit(mi_rows_bytes(16, kmax), MI_SMEM_MAX - mi_side_bytes(njobs), mib_per_warp_bytes(1, H, N3p), 8);
+}
+
+// Ring placement of a planned job table (8 int32 per job; [0] descriptor, [2] ring offset, [3] back, [4] stream
+// offset / 16, [5] bytes / 16): consecutive byte ranges, wrapping to 0 when a job does not fit before the end; every
+// tile replays the same offsets, so `back` looks through the cyclic job order (a job of the previous tile counts).
+// Stream placement: job after job.
+template <class Size>
+static int mi_place_jobs(int* jobs, int n, int ring, Size size_of) {
+  int cur = 0;
+  long long soff = 0;
+  for (int j = 0; j < n; ++j) {
+    const int size = size_of(jobs[8 * j]);
+    if (size > ring) return NFK_ERR_SHAPE;
+    if (cur + size > ring) cur = 0;
+    jobs[8 * j + 2] = cur;
+    cur += size;
+    if (soff / 16 > 0x7fffffff) return NFK_ERR_SHAPE;
+    jobs[8 * j + 4] = static_cast<int>(soff / 16);
+    jobs[8 * j + 5] = size / 16;
+    soff += size;
+  }
+  for (int j = 0; j < n; ++j) {
+    const int lo = jobs[8 * j + 2], hi = lo + jobs[8 * j + 5] * 16;
+    int back = n;                                  // nothing overlaps within a whole period: only the slot binds
+    for (int b = 1; b < n && hi > lo; ++b) {
+      const int i = ((j - b) % n + n) % n;
+      const int lo2 = jobs[8 * i + 2], hi2 = lo2 + jobs[8 * i + 5] * 16;
+      if (lo < hi2 && lo2 < hi) { back = b; break; }
+    }
+    jobs[8 * j + 3] = back;
+  }
+  return n;
 }
 
 extern "C" int nfk_made_inverse_resident_supported(int D, int H, int Dp) {
@@ -765,35 +1158,64 @@ extern "C" int nfk_made_inverse_jobs(const int* cnt1, const int* cnt2, int D, in
     }
   }
   if (n > cap) return n;            // sizing call (or a short buffer): offsets need the whole table
-  // ring placement: consecutive byte ranges, wrapping to 0 when a job does not fit before the end; every tile replays
-  // the same offsets, so `back` looks through the cyclic job order (a job of the previous tile counts).
-  // stream placement: job after job.
   const int ring = mi_ring_bytes(H, Dp, n, push, N3p);
   if (ring <= 0) return NFK_ERR_SHAPE;
-  int cur = 0;
-  long long soff = 0;
-  for (int j = 0; j < n; ++j) {
-    const int size = mi_job_bytes(jobs[8 * j], push, N3p);
-    if (size > ring) return NFK_ERR_SHAPE;
-    if (cur + size > ring) cur = 0;
-    jobs[8 * j + 2] = cur;
-    cur += size;
-    if (soff / 16 > 0x7fffffff) return NFK_ERR_SHAPE;
-    jobs[8 * j + 4] = static_cast<int>(soff / 16);
-    jobs[8 * j + 5] = size / 16;
-    soff += size;
-  }
-  for (int j = 0; j < n; ++j) {
-    const int lo = jobs[8 * j + 2], hi = lo + jobs[8 * j + 5] * 16;
-    int back = n;                                  // nothing overlaps within a whole period: only the slot binds
-    for (int b = 1; b < n && hi > lo; ++b) {
-      const int i = ((j - b) % n + n) % n;
-      const int lo2 = jobs[8 * i + 2], hi2 = lo2 + jobs[8 * i + 5] * 16;
-      if (lo < hi2 && lo2 < hi) { back = b; break; }
+  return mi_place_jobs(jobs, n, ring, [&](int desc) { return mi_job_bytes(desc, push, N3p); });
+}
+
+extern "C" int nfk_made_inverse_bwd_supported(int D, int H, int N3p) {
+  if (D <= 0 || D > 4095 || H <= 0 || H % 64 || N3p % 64 || N3p < 2 * D || H > 255 * 16 || N3p > 255 * 16) return 0;
+  return mib_ring_bytes(H, N3p, 4 * D + H / 8) > 0 ? 1 : 0;
+}
+
+// Host-side: the job stream of the reverse solve, steps d = D-1 .. 0, from the same degree counts as the forward's
+// planner. Per step: layer-2 tile pairs of degree d + 1 (k: dout columns of outputs > d), layer-1 tile pairs of
+// degree d + 1 (k: layer-2 units of degree >= d + 1), then the row job of step d (k: layer-1 units of degree >= d + 1).
+// jobs[6] = the job's first 16-wide k-chunk.
+extern "C" int nfk_made_inverse_bwd_jobs(const int* cnt1, const int* cnt2, int D, int H, int N3p, int* jobs, int cap) {
+  if (!cnt1 || !cnt2 || D <= 0 || cap < 0 || (cap > 0 && !jobs)) return NFK_ERR_ARG;
+  if (!nfk_made_inverse_bwd_supported(D, H, N3p)) return NFK_ERR_SHAPE;
+  for (int d = 0; d <= D; ++d)
+    if (cnt1[d] < (d ? cnt1[d - 1] : 0) || cnt2[d] < (d ? cnt2[d - 1] : 0) || cnt1[d] > H || cnt2[d] > H)
+      return NFK_ERR_ARG;
+  int n = 0;
+  auto put = [&](int phase, int row0, int k0, int k1, int two) {
+    if (n < cap) {
+      int* q = jobs + 8 * n;
+      q[0] = phase | (two << 2) | ((k1 > k0 ? k1 - k0 : 0) << 3); q[1] = row0; q[6] = k1 > k0 ? k0 : 0;
+      q[2] = q[3] = q[4] = q[5] = q[7] = 0;
     }
-    jobs[8 * j + 3] = back;
+    ++n;
+  };
+  const int kh = H / 16, ko = (2 * D + 15) / 16;
+  for (int d = D - 1; d >= 0; --d) {
+    if (d + 1 < D) {
+      const int c2p = cnt2[d], c2 = cnt2[d + 1], c1p = cnt1[d], c1 = cnt1[d + 1];
+      for (int nt = c2p >> 3, hi = (c2 + 7) >> 3; c2 > c2p && nt < hi; nt += 2) put(1, nt * 8, (d + 1) >> 4, ko, nt + 1 < hi);
+      for (int nt = c1p >> 3, hi = (c1 + 7) >> 3; c1 > c1p && nt < hi; nt += 2) put(0, nt * 8, c2p >> 4, kh, nt + 1 < hi);
+    }
+    put(2, d, cnt1[d] >> 4, kh, 0);
   }
-  return n;
+  if (n > cap) return n;
+  const int ring = mib_ring_bytes(H, N3p, n);
+  if (ring <= 0) return NFK_ERR_SHAPE;
+  return mi_place_jobs(jobs, n, ring, [](int desc) {
+    const int kch = desc >> 3, rows = (desc & 3) == 2 ? 1 : ((desc & 4) ? 16 : 8);
+    return kch ? mi_rows_bytes(rows, kch) : 0;
+  });
+}
+
+extern "C" int nfk_made_inverse_bwd_pack(const int* jobs, int njobs, const void* B1T, const void* B2T, const void* B3T,
+                                         int D, int H, int N3p, void* wstream, void* stream) {
+  if (njobs <= 0 || !nfk_made_inverse_bwd_supported(D, H, N3p)) return NFK_ERR_SHAPE;
+  if (!jobs || !B1T || !B2T || !B3T || !wstream || (reinterpret_cast<uintptr_t>(jobs) & 15) ||
+      (reinterpret_cast<uintptr_t>(wstream) & 127))
+    return NFK_ERR_ARG;
+  made_inverse_bwd_pack_kernel<<<njobs, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      reinterpret_cast<const int4*>(jobs), static_cast<const __nv_bfloat16*>(B1T),
+      static_cast<const __nv_bfloat16*>(B2T), static_cast<const __nv_bfloat16*>(B3T), H, N3p,
+      static_cast<unsigned char*>(wstream));
+  return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
 }
 
 extern "C" int nfk_made_inverse_pack(const int* jobs, int njobs, const void* B1, const void* B2, const void* B3,
@@ -882,4 +1304,53 @@ extern "C" int nfk_made_inverse_resident(const float* u_in, const void* wstream,
   int mt = mtiles == 0 ? 1 : mtiles;
   if (mt == 2 && ring + mi_side_bytes(njobs) + mi_per_warp_bytes(2, H, Dp) > MI_SMEM_MAX) mt = 1;
   return mt == 2 ? mi_launch<2>(p, st) : mi_launch<1>(p, st);
+}
+
+template <int MT>
+static int mib_launch(MibArgs p, cudaStream_t st) {
+  const int per_warp = mib_per_warp_bytes(MT, p.H, p.N3p);
+  p.ring_bytes = mib_ring_bytes(p.H, p.N3p, p.njobs);
+  if (p.ring_bytes <= 0) return NFK_ERR_SHAPE;
+  const int fixed = p.ring_bytes + mi_side_bytes(p.njobs);
+  int warps = (MI_SMEM_MAX - fixed) / per_warp;
+  if (warps > 8) warps = 8;
+  if (warps < 1) return NFK_ERR_SHAPE;
+  const int wtiles = (p.B + MT * 16 - 1) / (MT * 16);
+  if (warps > wtiles) warps = wtiles;
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int smem = fixed + warps * per_warp;
+  if (cudaFuncSetAttribute(made_inverse_bwd_resident_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) !=
+      cudaSuccess)
+    return NFK_ERR_LAUNCH;
+  int grid = (wtiles + warps - 1) / warps;
+  if (grid > sms) grid = sms;
+  made_inverse_bwd_resident_kernel<MT><<<grid, (warps + 1) * 32, smem, st>>>(p);
+  return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
+}
+
+extern "C" int nfk_made_inverse_bwd_resident(const float* g_x, const float* g_ld, const float* out, const void* m1,
+                                             const void* m2, const float* u_in, const void* wstream, const int* jobs,
+                                             int njobs, float* g_u, void* dout, float* db3, int B, int D, int H,
+                                             int N3p, int flip, int mtiles, void* stream) {
+  if (B <= 0 || njobs <= 0 || njobs > (1 << 20) || !nfk_made_inverse_bwd_supported(D, H, N3p) || mtiles < 0 ||
+      mtiles > 2)
+    return NFK_ERR_SHAPE;
+  if (!g_x || !out || !m1 || !m2 || !u_in || !wstream || !jobs || !g_u || !dout || !db3) return NFK_ERR_ARG;
+  if ((reinterpret_cast<uintptr_t>(jobs) & 15) || (reinterpret_cast<uintptr_t>(wstream) & 15)) return NFK_ERR_ARG;
+  MibArgs p;
+  p.g_x = g_x; p.g_ld = g_ld; p.out = out;
+  p.m1 = static_cast<const uint32_t*>(m1); p.m2 = static_cast<const uint32_t*>(m2);
+  p.u_in = u_in;
+  p.wstream = static_cast<const unsigned char*>(wstream);
+  p.jobs = reinterpret_cast<const int4*>(jobs); p.njobs = njobs; p.ring_bytes = 0;
+  p.g_u = g_u; p.dout = static_cast<__nv_bfloat16*>(dout); p.db3 = db3;
+  p.B = B; p.D = D; p.H = H; p.N3p = N3p; p.flip = flip;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int ring = mib_ring_bytes(H, N3p, njobs);
+  if (ring <= 0) return NFK_ERR_SHAPE;
+  int mt = mtiles == 0 ? 1 : mtiles;
+  if (mt == 2 && ring + mi_side_bytes(njobs) + mib_per_warp_bytes(2, H, N3p) > MI_SMEM_MAX) mt = 1;
+  return mt == 2 ? mib_launch<2>(p, st) : mib_launch<1>(p, st);
 }

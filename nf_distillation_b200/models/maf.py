@@ -77,36 +77,89 @@ class _MadeFn(torch.autograd.Function):
     def backward(ctx, g_u, g_ld, _g_ub):
         made, flip = ctx.made, ctx.flip
         x, xb, h1, h2, m1, m2, out, B1T, B2T, B3T = ctx.saved_tensors
-        D, H, Dp, N3p = made.D, made.H, made.Dp, made.N3p
         B = x.shape[0]
         dev = x.device
         g_u = torch.zeros_like(x) if g_u is None else g_u.contiguous()
         g_ld = torch.zeros(B, device=dev, dtype=F32) if g_ld is None else g_ld.contiguous()
-        sizes = [2 * D, H, H, N3p * H, H * H, H * Dp]
-        offs = [0]
-        for s in sizes:
-            offs.append(offs[-1] + ops.round_up(s, 4))
-        arena = torch.zeros(offs[-1], device=dev, dtype=F32)
-        db3, db2, db1, dB3, dB2, dB1 = (arena[offs[i]:offs[i] + sizes[i]] for i in range(6))
-        dB3, dB2, dB1 = dB3.view(N3p, H), dB2.view(H, H), dB1.view(H, Dp)
+        grads = _made_grad_arena(made, dev)
         dx = torch.empty_like(x)
-        dout = torch.empty(B, N3p, device=dev, dtype=BF16)
-        ops.made_affine_bwd(x, out, N3p, g_u, g_ld, dx, dout, db3, B, D, flip)
-        dpre2 = torch.empty(B, H, device=dev, dtype=BF16)
-        ops.gemm_nt(dout, B3T, B, H, N3p, ops.EPI_MASK_BF16, dpre2, aux=m2, colsum=db2)
-        ops.gemm_tn(dout, h2, N3p, H, B, dB3)
-        dpre1 = torch.empty(B, H, device=dev, dtype=BF16)
-        kb0, kb1 = made._ranges_t
-        ops.gemm_nt_ranged(dpre2, B2T, B, H, H, ops.EPI_MASK_BF16, dpre1, made.bn, kb0, kb1, aux=m1, colsum=db1)
-        ops.gemm_tn(dpre2, h1, H, H, B, dB2)
+        dout = torch.empty(B, made.N3p, device=dev, dtype=BF16)
+        ops.made_affine_bwd(x, out, made.N3p, g_u, g_ld, dx, dout, grads[0], B, made.D, flip)
+        dxn, dw1, dw2, dw3 = _made_net_backward(made, dout, xb, h1, h2, m1, m2, B1T, B2T, B3T, grads, True)
+        dx = dx + dxn[:, :made.D]
+        db3, db2, db1 = grads[:3]
+        return dx, g_ld, None, None, None, dw1, db1, dw2, db2, dw3, db3
+
+
+def _made_grad_arena(made, dev):
+    """Zeroed fp32 accumulators (db3, db2, db1, dB3, dB2, dB1) of one MADE layer's parameter gradients, one allocation."""
+    D, H, Dp, N3p = made.D, made.H, made.Dp, made.N3p
+    sizes = [2 * D, H, H, N3p * H, H * H, H * Dp]
+    offs = [0]
+    for s in sizes:
+        offs.append(offs[-1] + ops.round_up(s, 4))
+    arena = torch.zeros(offs[-1], device=dev, dtype=F32)
+    db3, db2, db1, dB3, dB2, dB1 = (arena[offs[i]:offs[i] + sizes[i]] for i in range(6))
+    return db3, db2, db1, dB3.view(N3p, H), dB2.view(H, H), dB1.view(H, Dp)
+
+
+def _made_net_backward(made, dout, xb, h1, h2, m1, m2, B1T, B2T, B3T, grads, want_dx):
+    """The masked network's backward at the forward's saved activations, from dout = [dmu | dalpha] (bf16 [B, N3p]):
+    accumulates db2, db1 and dB3, dB2, dB1 into `grads` (_made_grad_arena; db3 is the caller's), returns
+    (dxn [B, Dp] fp32 or None, dw1, dw2, dw3)."""
+    D, H, Dp, N3p = made.D, made.H, made.Dp, made.N3p
+    B = dout.shape[0]
+    dev = dout.device
+    _, db2, db1, dB3, dB2, dB1 = grads
+    dpre2 = torch.empty(B, H, device=dev, dtype=BF16)
+    ops.gemm_nt(dout, B3T, B, H, N3p, ops.EPI_MASK_BF16, dpre2, aux=m2, colsum=db2)
+    ops.gemm_tn(dout, h2, N3p, H, B, dB3)
+    dpre1 = torch.empty(B, H, device=dev, dtype=BF16)
+    kb0, kb1 = made._ranges_t
+    ops.gemm_nt_ranged(dpre2, B2T, B, H, H, ops.EPI_MASK_BF16, dpre1, made.bn, kb0, kb1, aux=m1, colsum=db1)
+    ops.gemm_tn(dpre2, h1, H, H, B, dB2)
+    dxn = None
+    if want_dx:
         dxn = torch.empty(B, Dp, device=dev, dtype=F32)
         ops.gemm_nt(dpre1, B1T, B, Dp, H, ops.EPI_F32, dxn)
-        ops.gemm_tn(dpre1, xb, H, Dp, B, dB1)
-        dx = dx + dxn[:, :D]
-        dw1, dw2, dw3 = (torch.empty(H, D, device=dev), torch.empty(H, H, device=dev),
-                         torch.empty(2 * D, H, device=dev))
-        ops.made_prep_bwd(dB1, dB2, dB3, made.deg1, made.deg2, D, H, Dp, dw1, dw2, dw3)
-        return dx, g_ld, None, None, None, dw1, db1, dw2, db2, dw3, db3
+    ops.gemm_tn(dpre1, xb, H, Dp, B, dB1)
+    dw1, dw2, dw3 = (torch.empty(H, D, device=dev), torch.empty(H, H, device=dev),
+                     torch.empty(2 * D, H, device=dev))
+    ops.made_prep_bwd(dB1, dB2, dB3, made.deg1, made.deg2, D, H, Dp, dw1, dw2, dw3)
+    return dxn, dw1, dw2, dw3
+
+
+class _MadeInverseFn(torch.autograd.Function):
+    """The sequential inverse x = MADE^-1(u) with gradients. The forward is the no-grad inverse unchanged (x is
+    bit-identical); the backward recomputes the forward network at x (activations and ReLU masks), runs the reverse
+    solve (MADE._inverse_solve) for g_u and dout = [mubar | alphabar], and the forward's parameter chain from dout."""
+
+    @staticmethod
+    def forward(ctx, u_in, ld_in, made, flip, w1, b1, w2, b2, w3, b3):
+        u_in = u_in.contiguous()
+        x, ld_out = made._run_inverse(u_in, ld_in, True, (w1, b1, w2, b2, w3, b3))
+        ctx.made, ctx.flip = made, flip
+        ctx.save_for_backward(u_in, x, w1, b1, w2, b2, w3, b3)
+        return x, ld_out
+
+    @staticmethod
+    def backward(ctx, g_x, g_ld):
+        made, flip = ctx.made, ctx.flip
+        u_in, x, *params = ctx.saved_tensors
+        B = x.shape[0]
+        dev = x.device
+        g_x = torch.zeros_like(x) if g_x is None else g_x.contiguous()
+        g_ld = None if g_ld is None else g_ld.contiguous()
+        ops_ = made._operands(params, True)
+        xb = made._bf16_rows(x, None)
+        h1, h2, out, m1, m2 = made._net(xb, B, ops_, params[1], params[3], keep=True)
+        grads = _made_grad_arena(made, dev)
+        g_u = torch.empty_like(x)
+        dout = torch.empty(B, made.N3p, device=dev, dtype=BF16)
+        made._inverse_solve(g_x, g_ld, u_in, out, m1, m2, ops_, flip, g_u, dout, grads[0])
+        _, dw1, dw2, dw3 = _made_net_backward(made, dout, xb, h1, h2, m1, m2, ops_[1], ops_[3], ops_[5], grads, False)
+        db3, db2, db1 = grads[:3]
+        return g_u, g_ld, None, None, dw1, db1, dw2, db2, dw3, db3
 
 
 class MADE(nn.Module):
@@ -131,10 +184,11 @@ class MADE(nn.Module):
         self._range_cache = None
         self._cache = None
         self._job_cache = None
+        self._bwd_job_cache = None
         self._stream_cache = None
         self._stream_bytes = 0
         self.push_inverse = True         # False: the pull kernel (h2 kept in shared memory) even for aligned degrees
-        self.resident_inverse = True     # False: the D-pass GEMM inverse (kept as the cross-check in the tests)
+        self.resident_inverse = True     # False: the D-pass GEMM inverse and reverse solve (the cross-checks in the tests)
         self.resident_mtiles = 0         # 16-sample tiles per warp in the resident inverse (0 = chosen by the library)
 
     def _kb_ranges_now(self):
@@ -194,10 +248,14 @@ class MADE(nn.Module):
         """The packed weight stream of the resident inverse for the current operands (rebuilt when they change)."""
         key = (jobs.data_ptr(), push, ops_[0].data_ptr(), ops_[0]._version)
         if self._stream_cache is None or self._stream_cache[0] != key:
-            ws = torch.zeros(max(self._stream_bytes, 128), device=jobs.device, dtype=torch.uint8)
-            ops.made_inverse_pack(jobs, ops_[0], ops_[2], ops_[4], self.N3p, self.D, self.H, self.Dp, push, ws)
+            ws = self._pack_stream(jobs, push, ops_)
             self._stream_cache = (key, ws, ops_[0])   # (keeps B1 alive so the pointer in the key cannot be reused)
         return self._stream_cache[1]
+
+    def _pack_stream(self, jobs, push, ops_):
+        ws = torch.zeros(max(self._stream_bytes, 128), device=jobs.device, dtype=torch.uint8)
+        ops.made_inverse_pack(jobs, ops_[0], ops_[2], ops_[4], self.N3p, self.D, self.H, self.Dp, push, ws)
+        return ws
 
     def _params(self):
         return (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias, self.fc3.weight, self.fc3.bias)
@@ -293,16 +351,28 @@ class MADE(nn.Module):
                 ops.made_affine_fwd(x, out, self.N3p, u, ub, self.Dp, ld.contiguous(), ld_out, Bn, self.D, self.flip)
             u._nfk_bf16 = (ub, u._version)   # bf16 copy for the next MADE layer (saves its conversion pass)
             return u, (ld_out if want else None)
-        if torch.is_grad_enabled() and input.requires_grad:
-            raise NotImplementedError("gradients through the sequential MADE inverse are not built")
-        u_in = input.contiguous()
-        ops_ = self._cached_operands()
+        if torch.is_grad_enabled() and (input.requires_grad or ld.requires_grad or any(p.requires_grad for p in params)):
+            x, ld_out = _MadeInverseFn.apply(input, ld, self, self.flip, *params)
+            return x, (ld_out if want else None)
+        return self._run_inverse(input.contiguous(), ld, want)
+
+    def _run_inverse(self, u_in, ld, want, params=None):
+        """x = MADE^-1(u_in) and (want) ld_out = ld + sum alpha, without gradients. params=None (frozen modules:
+        no-grad calls): the operands and the packed weight stream come from the caches keyed by the parameters'
+        versions and the parameter epoch. Given params (the trainable path): both are rebuilt from them on every call,
+        as the forward's _MadeFn does, because an optimiser that writes the parameters through raw pointers (FlatAdam)
+        bumps no version, and a captured graph must contain the rebuild."""
+        Bn = u_in.shape[0]
+        cached = params is None
+        params = self._params() if cached else tuple(p.detach() for p in params)
+        ops_ = self._cached_operands() if cached else self._operands(params, False)
         jobs, push = self._inverse_jobs(u_in.device)
         if jobs is not None and self.resident_inverse and ops.made_inverse_resident_supported(self.D, self.H, self.Dp):
             # ONE launch: every hidden unit finalised once, in degree order, activations resident in shared memory
             x = torch.empty_like(u_in)
             ld_out = torch.empty(Bn, device=x.device, dtype=F32) if want else None
-            ops.made_inverse_resident(u_in, self._weight_stream(jobs, push, ops_), params[1].detach(),
+            ws = self._weight_stream(jobs, push, ops_) if cached else self._pack_stream(jobs, push, ops_)
+            ops.made_inverse_resident(u_in, ws, params[1].detach(),
                                       params[3].detach(), ops_[6], jobs, push, self.N3p, x,
                                       ld.contiguous() if want else None, ld_out, Bn, self.D, self.H, self.Dp,
                                       self.flip, self.resident_mtiles)
@@ -318,6 +388,52 @@ class MADE(nn.Module):
             ops.made_inv_update(x, xb, self.Dp, u_in, out, self.N3p, ldc, ld_out, Bn, self.D, i, self.flip,
                                 i == self.D - 1)
         return x, (ld_out if want else None)
+
+    def _inverse_bwd_jobs(self, dev):
+        """Job table of the one-launch reverse solve on `dev` (ops.made_inverse_bwd_jobs), planned on the host once
+        per degree assignment; None when the degrees are not sorted ascending or the shape does not fit."""
+        key = (self.deg1.data_ptr(), self.deg1._version, self.deg2.data_ptr(), self.deg2._version, str(dev))
+        if self._bwd_job_cache is None or self._bwd_job_cache[0] != key:
+            d1, d2 = self.deg1.detach().cpu().long(), self.deg2.detach().cpu().long()
+            jobs = None
+            if (bool((d1[1:] >= d1[:-1]).all() and (d2[1:] >= d2[:-1]).all() and d1.min() >= 1 and d2.min() >= 1)
+                    and ops.made_inverse_bwd_supported(self.D, self.H, self.N3p)):
+                edges = torch.arange(self.D + 1)
+                cnt1, cnt2 = ((d[None, :] <= edges[:, None]).sum(1) for d in (d1, d2))
+                jobs = ops.made_inverse_bwd_jobs(cnt1, cnt2, self.D, self.H, self.N3p)
+                jobs = (jobs.to(dev), int(jobs[:, 5].sum()) * 16)
+            self._bwd_job_cache = (key, jobs)
+        return self._bwd_job_cache[1]
+
+    def _inverse_solve(self, g_x, g_ld, u_in, out, m1, m2, ops_, flip, g_u, dout, db3):
+        """Reverse solve of the inverse's gradients at x (out, m1, m2 from the forward network recomputed at x):
+        writes g_u, dout = [mubar | alphabar | 0] and adds dout's column sums to db3. One launch when the degrees are
+        sorted and the shape fits (and resident_inverse is on); else D passes of the three dgrad GEMMs."""
+        B = u_in.shape[0]
+        D, H, Dp, N3p = self.D, self.H, self.Dp, self.N3p
+        _, B1T, _, B2T, _, B3T, _ = ops_
+        plan = self._inverse_bwd_jobs(u_in.device) if self.resident_inverse else None
+        if plan is not None:
+            jobs, nbytes = plan
+            # (no memset: the pack writes every row the kernel multiplies; the bytes it leaves alone are only read
+            # into MMA columns the kernel discards)
+            ws = torch.empty(max(nbytes, 128), device=u_in.device, dtype=torch.uint8)
+            ops.made_inverse_bwd_pack(jobs, B1T, B2T, B3T, D, H, N3p, ws)
+            ops.made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, ws, jobs, g_u, dout, db3, B, D, H, N3p, flip,
+                                          self.resident_mtiles)
+            return
+        dout.zero_()
+        c = torch.empty(B, Dp, device=u_in.device, dtype=F32)
+        dpre2 = torch.empty(B, H, device=u_in.device, dtype=BF16)
+        dpre1 = torch.empty(B, H, device=u_in.device, dtype=BF16)
+        kb0, kb1 = self._ranges_t
+        for d in reversed(range(D)):
+            if d < D - 1:   # c = the network's input gradient for the rows finished so far
+                ops.gemm_nt(dout, B3T, B, H, N3p, ops.EPI_MASK_BF16, dpre2, aux=m2)
+                ops.gemm_nt_ranged(dpre2, B2T, B, H, H, ops.EPI_MASK_BF16, dpre1, self.bn, kb0, kb1, aux=m1)
+                ops.gemm_nt(dpre1, B1T, B, Dp, H, ops.EPI_F32, c)
+            ops.made_inv_bwd_update(c if d < D - 1 else None, Dp, g_x, g_ld, out, N3p, u_in, g_u, dout, db3, B, D, d,
+                                    flip)
 
 
 class MAFNet(nn.Module):

@@ -414,6 +414,48 @@ def made_inverse_resident(u_in, wstream, b1, b2, b3, jobs, push, N3p, x, ld_in, 
                                         int(mtiles), _st()), "nfk_made_inverse_resident")
 
 
+def made_inv_bwd_update(c, ldc, g_x, g_ld, out, N3p, u_in, g_u, dout, db3, B, D, d, flip):
+    """Pass d of the D-pass reverse solve (gradients of the sequential inverse); c = None at d = D-1."""
+    _count()
+    check(LIB.nfk_made_inv_bwd_update(_p(c), ldc, _p(g_x), _p(g_ld), _p(out), N3p, _p(u_in), _p(g_u), _p(dout),
+                                      _p(db3), B, D, d, int(flip), _st()), "nfk_made_inv_bwd_update")
+
+
+def made_inverse_bwd_supported(D, H, N3p) -> bool:
+    return bool(LIB.nfk_made_inverse_bwd_supported(D, H, N3p))
+
+
+def made_inverse_bwd_jobs(cnt1, cnt2, D, H, N3p):
+    """Host-side job table of the one-launch reverse solve (same counts and layout as made_inverse_jobs; column 6 =
+    first k-chunk of the job), steps D-1 .. 0."""
+    import torch
+    cnt1 = cnt1.to(torch.int32).contiguous().cpu()
+    cnt2 = cnt2.to(torch.int32).contiguous().cpu()
+    n = LIB.nfk_made_inverse_bwd_jobs(cnt1.data_ptr(), cnt2.data_ptr(), D, H, N3p, None, 0)
+    if n <= 0:
+        check(n if n < 0 else -1, "nfk_made_inverse_bwd_jobs")
+    jobs = torch.empty(n, 8, dtype=torch.int32)
+    check(0 if LIB.nfk_made_inverse_bwd_jobs(cnt1.data_ptr(), cnt2.data_ptr(), D, H, N3p, jobs.data_ptr(), n) == n
+          else -1, "nfk_made_inverse_bwd_jobs")
+    return jobs
+
+
+def made_inverse_bwd_pack(jobs_dev, B1T, B2T, B3T, D, H, N3p, wstream):
+    """Transposed weights of every reverse-solve job, packed job after job in shared-memory layout."""
+    _count()
+    check(LIB.nfk_made_inverse_bwd_pack(_p(jobs_dev), jobs_dev.shape[0], _p(B1T), _p(B2T), _p(B3T), D, H, N3p,
+                                        _p(wstream), _st()), "nfk_made_inverse_bwd_pack")
+
+
+def made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, wstream, jobs, g_u, dout, db3, B, D, H, N3p, flip,
+                              mtiles=0):
+    """The whole reverse solve of one MADE layer's inverse in one launch (include/nfk.h)."""
+    _count()
+    check(LIB.nfk_made_inverse_bwd_resident(_p(g_x), _p(g_ld), _p(out), _p(m1), _p(m2), _p(u_in), _p(wstream),
+                                            _p(jobs), jobs.shape[0], _p(g_u), _p(dout), _p(db3), B, D, H, N3p,
+                                            int(flip), int(mtiles), _st()), "nfk_made_inverse_bwd_resident")
+
+
 def cnet_fused_supported(hid, K1p) -> bool:
     return hid == 512 and K1p % 64 == 0 and 64 <= K1p <= 512
 
