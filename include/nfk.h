@@ -325,20 +325,24 @@ int nfk_made_inverse_bwd_resident(const float* g_x, const float* g_ld, const flo
                                   int mtiles, void* stream);
 
 /* Fused conv#1 -> conv#2 of the coupling network: h2 = relu(relu(col*B1^T + b1)*B2^T + b2) in ONE kernel (CTA
- * pairs; h1 stays in shared memory as the tcgen05 A operand of conv#2). col [M,K1p] bf16, B1 [512,K1p], B2 [512,512]
- * bf16 (nfk_coupling_prep), h2 [M,512] bf16. Training additionally passes h1 [M,512] and the two 1-bit ReLU mask
- * buffers (word-major, [16][ldmask >= M]); inference passes NULL for them. hid must be 512. */
+ * pairs; h1 stays in tensor memory as the tcgen05 A operand of conv#2; csrc/cnet_ts.cu). col [M,K1p] bf16, B1 [512,K1p],
+ * B2 [512,512] bf16 (nfk_coupling_prep), h2 [M,512] bf16. Training additionally passes h1 [M,512] and the two 1-bit
+ * ReLU mask buffers (word-major, [16][ldmask >= M]); inference passes NULL for them.
+ * nfk_cnet_fused_supported: 1 if the kernels take hidden width hid and first-GEMM depth K (K1p / K3p): hid = 512 and
+ * K a multiple of 64 up to 448 (the GEMM-1 A tile must leave shared memory for a weight ring of two slots). The entry
+ * points return NFK_ERR_SHAPE otherwise; callers run the two nfk_gemm_nt_bf16 GEMMs instead. */
+int nfk_cnet_fused_supported(int hid, int K);
 int nfk_cnet_set_prof(void* buf); /* diagnostics: per-CTA cycle counters of the MMA issuer ([grid][8] int64) or NULL */
 int nfk_cnet_fwd_fused(const void* col, int K1p, const void* B1, const void* B2, const float* bias1,
                        const float* bias2, void* h1, void* h2, void* mask1, void* mask2, long long ldmask, int M,
                        int hid, void* stream);
 /* The same pipeline for the BACKWARD chain of the coupling net (student training): d2 = relu'(h2) .* (dhcol B3T^T) —
- * the Conv2dZeros input gradient through the ReLU mask of h2 — stays in shared memory as the A operand of
+ * the Conv2dZeros input gradient through the ReLU mask of h2 — stays in tensor memory as the A operand of
  * d1 = relu'(h1) .* (d2 B2T^T); both are written out as bf16 [M, 512] (the weight-gradient GEMMs read them) and their
  * column sums are added into dbias2 / dbias1 (fp32 [512], caller-zeroed; NULL = not needed). dhcol [M, K3p] bf16
  * (nfk_coupling_bwd), B3T [512, K3p], B2T [512, 512] bf16 (nfk_coupling_prep, transposed operands), masks as written by
  * nfk_cnet_fwd_fused / nfk_gemm_nt_bf16 (word-major, [16][ldmask >= M]). Replaces two nfk_gemm_nt_bf16 calls with
- * NFK_EPI_MASK_BF16 (autograd of models/flows.py:25-34). hid must be 512, K3p a multiple of 64 up to 512. */
+ * NFK_EPI_MASK_BF16 (autograd of models/flows.py:25-34). Shapes: nfk_cnet_fused_supported(hid, K3p). */
 int nfk_cnet_bwd_fused(const void* dhcol, int K3p, const void* B3T, const void* B2T, const void* mask_h2,
                        const void* mask_h1, long long ldmask, void* dpre2, void* dpre1, float* dbias2, float* dbias1,
                        int M, int hid, void* stream);

@@ -94,6 +94,7 @@ SIGNATURES: dict[str, list] = {
     "nfk_flow1d_bwd": [_vp] * 9 + [_i] * 5 + [_vp],
     "nfk_affine_rows": [_vp] * 7 + [_i, _i, _f, _vp],
     "nfk_gemm_nt_bf16_ranged": [_vp, _ll, _vp, _ll, _i, _i, _i, _i, _vp, _ll, _vp, _vp, _ll, _vp, _i, _vp, _vp, _vp],
+    "nfk_cnet_fused_supported": [_i, _i],
     "nfk_cnet_set_prof": [_vp],
     "nfk_cnet_fwd_fused": [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp],
     "nfk_cnet_bwd_fused": [_vp, _i, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _vp],

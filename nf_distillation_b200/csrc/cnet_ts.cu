@@ -4,13 +4,13 @@
 //   h1 = relu(col * B1^T + b1)       conv3x3 as im2col GEMM          (reference models/flows.py:27-28)
 //   h2 = relu(h1  * B2^T + b2)       conv1x1                         (:29-30)
 //
-// Why: the shared-memory variant (cnet_fused.cu) is bound by shared-memory bandwidth, not by the tensor pipe — per
-// 256x256x16 MMA each SM reads 4 KB of h1 + 4 KB of B2 while TMA refills 4 KB and the epilogue moves ~3 KB: 118 of the
-// 128 B/clk the SM has (measured 153 cycles per MMA against 128 in isolation, plus operand waits on a 4-slot ring that
-// the 128 KB of h1 panels leave no room to deepen). Here the epilogue warps write the bf16 activations back into TMEM
-// (tcgen05.st, two K elements per 32-bit column: 256 columns for K = 512) and conv#2 is issued with A = [tmem]:
-// shared memory only carries the weights (32 B/clk read + 32 B/clk refill) and the store staging, and the 128 KB that
-// the h1 panels used become a 12-16 slot weight ring.
+// Why h1 lives in TMEM and not in 128B-swizzled shared-memory panels: with h1 in shared memory as conv#2's A operand the
+// kernel is bound by shared-memory bandwidth, not by the tensor pipe — per 256x256x16 MMA each SM reads 4 KB of h1 +
+// 4 KB of B2 while TMA refills 4 KB and the epilogue moves ~3 KB: 118 of the 128 B/clk the SM has (measured 153 cycles
+// per MMA against 128 in isolation, plus operand waits on a 4-slot ring that 128 KB of h1 panels leave no room to
+// deepen). Here the epilogue warps write the bf16 activations back into TMEM (tcgen05.st, two K elements per 32-bit
+// column: 256 columns for K = 512) and conv#2 is issued with A = [tmem]: shared memory only carries the weights
+// (32 B/clk read + 32 B/clk refill) and the store staging, and the 128 KB the panels would take hold the weight ring.
 //
 //   TMEM   [0,256) h1 (bf16x2 per column) | [256,384) accumulator 0 | [384,512) accumulator 1
 //          -> a tile is 4 + 4 quarter-GEMMs of N = 128 (M = 256 over the CTA pair), ping-pong over the two accumulators
@@ -18,15 +18,17 @@
 //          4 KB | weight ring nslots x 8 KB (64 weight rows x 64 K per CTA and slot)
 //   warps  0: TMA producer, 1: MMA issuer (leader CTA) + TMEM alloc, 2-17: epilogue (4 per TMEM lane quadrant)
 //
-// MODE 0: forward (+ optional h1 / 1-bit ReLU mask outputs for training); MODE 1: the student's backward chain
-// d2 = mask .* (dhcol B3T^T), d1 = mask .* (d2 B2T^T) with both bias gradients (see cnet_fused.cu). Results are
-// bit-identical to cnet_fused.cu and to the two unfused GEMMs (same bf16 products, same K order in the fp32
+// MODE 0: forward (+ optional h1 / 1-bit ReLU mask outputs for training).
+// MODE 1: the student's backward chain, the two dgrads of Conv2dZeros input gradient -> ReLU mask of h2 -> conv1x1
+//         input gradient -> ReLU mask of h1:  d2 = mask_h2 .* (dhcol B3T^T),  d1 = mask_h1 .* (d2 B2T^T). Both are
+//         written out as bf16 (the weight-gradient GEMMs read them), and their column sums are the two bias gradients.
+//         Same tiles, same pipeline: d2 takes h1's place in TMEM as the A operand of the second GEMM.
+// Results are bit-identical to the two unfused GEMMs of gemm_tc.cu (same bf16 products, same K order in the fp32
 // accumulators; the N split does not enter the arithmetic).
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cstdint>
-#include <cstdlib>
 
 #include "../../include/nfk.h"
 #include "launch_util.h"
@@ -55,13 +57,16 @@ struct TsArgs {
   int nslots;
   const float* bias1;
   const float* bias2;
-  uint32_t* mask1;   // MODE 0: optional outputs; MODE 1: input masks of GEMM 1 / GEMM 2 outputs
-  uint32_t* mask2;
+  uint32_t* mask1;   // 1-bit ReLU masks, word-major [16][ldmask]. MODE 0: optional outputs; MODE 1: the masks applied
+  uint32_t* mask2;   // to the outputs of GEMM 1 / GEMM 2
   long long ldmask;
   int store_h1;
-  long long* prof;
-  int kb2_end[2];    // see cnet_fused.cu: structurally-zero k-blocks of B2 for output halves 0 / 1 are skipped
-  float* colsum1;
+  long long* prof;   // diagnostics: [grid][8] cycle counters of the MMA issuer
+  // GEMM-2 k-blocks (64 input channels each) that are not structurally zero for output half 0 / 1; 8 = all. MADE's
+  // degree-sorted hidden mask is block lower triangular: the low-degree half of the outputs never sees the high-degree
+  // inputs, so those B2 tiles are neither loaded nor multiplied (they are exact zeros: the result is bit-identical).
+  int kb2_end[2];
+  float* colsum1;    // MODE 1: column sums of the masked GEMM 1 / GEMM 2 outputs (the bias gradients), or NULL
   float* colsum2;
 };
 
@@ -524,65 +529,36 @@ cnet_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmCol, const __grid_const
   cnet_ts_body<1>(tmCol, tmB1, tmB2, tmH1, tmH2, g);
 }
 
-typedef CUresult (*EncodeTiledFn3)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-// bf16 [rows, cols] row-major (leading dimension ld elements), box = 64 columns (128 B, SWIZZLE_128B) x box_rows
-static int ts_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows) {
-  static EncodeTiledFn3 enc = nullptr;
-  if (!enc) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return NFK_ERR_DRIVER;
-    enc = reinterpret_cast<EncodeTiledFn3>(p);
-  }
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld * 2) % 16) return NFK_ERR_ALIGN;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * 2};
-  cuuint32_t box[2] = {64, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS
-             ? NFK_OK
-             : NFK_ERR_DRIVER;
-}
-
+// Shared-memory plan for a GEMM-1 A tile of kb1 k-blocks: the weight ring takes what the A tile, the store staging, the
+// barriers and the biases leave of the 227 KB, up to TS_MAX_SLOTS slots. Returns the bytes; *nslots = the ring's slots.
 static int ts_smem_plan(int kb1, int* nslots) {
   const int fixed = kb1 * TS_COLBLK + TS_STAGE_BYTES + TS_BAR_BYTES + TS_BIAS_BYTES;
   int n = (227 * 1024 - fixed) / TS_SLOT;
   if (n > TS_MAX_SLOTS) n = TS_MAX_SLOTS;
-  static const int cap = [] { const char* e = getenv("NFK_CNET_SLOTS"); return e ? atoi(e) : 0; }();   // experiments
-  if (cap >= 2 && n > cap) n = cap;
   *nslots = n;
   return fixed + n * TS_SLOT;
 }
 
 // Shared launcher: GEMM 1 = A [M, Ka] x W1 [512, Ka]^T, GEMM 2 = (epilogue of GEMM 1) x W2 [512, 512]^T; out1 (optional
-// in MODE 0) / out2 are the bf16 [M, 512] epilogue outputs of the two GEMMs.
+// in MODE 0) / out2 are the bf16 [M, 512] epilogue outputs of the two GEMMs. The shape has passed
+// nfk_cnet_fused_supported.
 template <int MODE>
 static int ts_launch(const void* A, int Ka, const void* W1, const void* W2, void* out1, void* out2, TsArgs g,
                      cudaStream_t stream) {
   int nslots = 0;
   const int smem_bytes = ts_smem_plan(Ka / 64, &nslots);
-  if (nslots < 2) return NFK_ERR_SHAPE;
   g.nslots = nslots;
   CUtensorMap tmA, tmW1, tmW2, tmO1, tmO2;
   int rc;
-  if ((rc = ts_tmap(&tmA, A, Ka, g.M, Ka, 128))) return rc;
-  if ((rc = ts_tmap(&tmW1, W1, Ka, TS_HID, Ka, 64))) return rc;
-  if ((rc = ts_tmap(&tmW2, W2, TS_HID, TS_HID, TS_HID, 64))) return rc;
-  if ((rc = ts_tmap(&tmO2, out2, TS_HID, g.M, TS_HID, 32))) return rc;
-  if (out1) { if ((rc = ts_tmap(&tmO1, out1, TS_HID, g.M, TS_HID, 32))) return rc; }
+  if ((rc = make_tmap_2d(&tmA, A, Ka, g.M, Ka, 128))) return rc;
+  if ((rc = make_tmap_2d(&tmW1, W1, Ka, TS_HID, Ka, 64))) return rc;
+  if ((rc = make_tmap_2d(&tmW2, W2, TS_HID, TS_HID, TS_HID, 64))) return rc;
+  if ((rc = make_tmap_2d(&tmO2, out2, TS_HID, g.M, TS_HID, 32))) return rc;
+  if (out1) { if ((rc = make_tmap_2d(&tmO1, out1, TS_HID, g.M, TS_HID, 32))) return rc; }
   else tmO1 = tmO2;
   auto kernel = MODE == 0 ? cnet_fwd_ts_kernel : cnet_bwd_ts_kernel;
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kernel), smem_bytes))) return rc;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int tiles = (g.M + 255) / 256;
   const int pairs = tiles < sms / 2 ? tiles : sms / 2;
   const cudaError_t le = launch_pdl(kernel, dim3(2 * pairs), dim3(TS_THREADS), smem_bytes, stream, tmA, tmW1, tmW2,
@@ -590,20 +566,49 @@ static int ts_launch(const void* A, int Ka, const void* W1, const void* W2, void
   return (le == cudaSuccess && cudaGetLastError() == cudaSuccess) ? NFK_OK : NFK_ERR_LAUNCH;
 }
 
-int cnet_ts_fwd(const void* col, int K1p, const void* B1, const void* B2, const float* bias1, const float* bias2,
-                void* h1, void* h2, void* mask1, void* mask2, long long ldmask, int M, int kb2_end_half0,
-                long long* prof, void* stream) {
+}  // namespace nfk
+
+using namespace nfk;
+
+extern "C" int nfk_cnet_fused_supported(int hid, int K) {
+  // (the k-block bound only keeps the plan's byte counts in range: 14 k-blocks alone fill the 227 KB)
+  if (hid != TS_HID || K < 64 || K % 64 || K / 64 > 227 * 1024 / TS_COLBLK) return 0;
+  int nslots = 0;
+  ts_smem_plan(K / 64, &nslots);
+  return nslots >= 2;     // K <= 448: at K = 512 the A tile leaves room for one weight slot
+}
+
+static long long* g_cnet_prof = nullptr;
+extern "C" int nfk_cnet_set_prof(void* buf) {
+  g_cnet_prof = static_cast<long long*>(buf);
+  return NFK_OK;
+}
+
+extern "C" int nfk_cnet_fwd_fused(const void* col, int K1p, const void* B1, const void* B2, const float* bias1,
+                                  const float* bias2, void* h1, void* h2, void* mask1, void* mask2,
+                                  long long ldmask, int M, int hid, void* stream) {
+  return nfk_cnet_fwd_fused_ranged(col, K1p, B1, B2, bias1, bias2, h1, h2, mask1, mask2, ldmask, M, hid, 8, stream);
+}
+
+extern "C" int nfk_cnet_fwd_fused_ranged(const void* col, int K1p, const void* B1, const void* B2, const float* bias1,
+                                         const float* bias2, void* h1, void* h2, void* mask1, void* mask2,
+                                         long long ldmask, int M, int hid, int kb2_end_half0, void* stream) {
+  if (M <= 0 || !nfk_cnet_fused_supported(hid, K1p)) return NFK_ERR_SHAPE;
+  if (kb2_end_half0 < 1 || kb2_end_half0 > 8) return NFK_ERR_ARG;
+  if (!col || !B1 || !B2 || !bias1 || !bias2 || !h2) return NFK_ERR_ARG;
+  if ((mask1 || mask2) && ldmask < M) return NFK_ERR_ARG;
   TsArgs g{M, K1p / 64, 0, bias1, bias2, static_cast<uint32_t*>(mask1), static_cast<uint32_t*>(mask2), ldmask,
-           h1 ? 1 : 0, prof, {kb2_end_half0, 8}, nullptr, nullptr};
+           h1 ? 1 : 0, g_cnet_prof, {kb2_end_half0, 8}, nullptr, nullptr};
   return ts_launch<0>(col, K1p, B1, B2, h1, h2, g, static_cast<cudaStream_t>(stream));
 }
 
-int cnet_ts_bwd(const void* dhcol, int K3p, const void* B3T, const void* B2T, const void* mask_h2,
-                const void* mask_h1, long long ldmask, void* dpre2, void* dpre1, float* dbias2, float* dbias1, int M,
-                void* stream) {
+extern "C" int nfk_cnet_bwd_fused(const void* dhcol, int K3p, const void* B3T, const void* B2T, const void* mask_h2,
+                                  const void* mask_h1, long long ldmask, void* dpre2, void* dpre1, float* dbias2,
+                                  float* dbias1, int M, int hid, void* stream) {
+  if (M <= 0 || !nfk_cnet_fused_supported(hid, K3p)) return NFK_ERR_SHAPE;
+  if (!dhcol || !B3T || !B2T || !mask_h2 || !mask_h1 || !dpre2 || !dpre1) return NFK_ERR_ARG;
+  if (ldmask < M) return NFK_ERR_ARG;
   TsArgs g{M, K3p / 64, 0, nullptr, nullptr, static_cast<uint32_t*>(const_cast<void*>(mask_h2)),
            static_cast<uint32_t*>(const_cast<void*>(mask_h1)), ldmask, 1, nullptr, {8, 8}, dbias2, dbias1};
   return ts_launch<1>(dhcol, K3p, B3T, B2T, dpre2, dpre1, g, static_cast<cudaStream_t>(stream));
 }
-
-}  // namespace nfk

@@ -349,9 +349,6 @@ conv1_dgrad_affine_bwd_kernel(const __grid_constant__ CUtensorMap tmW, const __g
   if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-// pconv_coupling.cu: bf16 [rows, cols] K-major tensor map, 64-column (128-byte, SWIZZLE_128B) boxes of box_rows rows
-int pc_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows);
-
 template <int C>
 static int dg_launch(const void* dpre1, const void* B1T, int K1p, int hid, DgArgs g, cudaStream_t st) {
   using Cfg = DgCfg<C>;
@@ -359,13 +356,11 @@ static int dg_launch(const void* dpre1, const void* B1T, int K1p, int hid, DgArg
   int rc;
   g.a_box_rows = K1p < 128 ? K1p : 128;
   const long long M = static_cast<long long>(g.B) << g.lgHW;
-  if ((rc = pc_tmap(&tmW, B1T, hid, K1p, hid, g.a_box_rows))) return rc;
-  if ((rc = pc_tmap(&tmD, dpre1, hid, static_cast<uint64_t>(M), hid, Cfg::NPIX))) return rc;
+  if ((rc = make_tmap_2d(&tmW, B1T, hid, K1p, hid, g.a_box_rows))) return rc;
+  if ((rc = make_tmap_2d(&tmD, dpre1, hid, static_cast<uint64_t>(M), hid, Cfg::NPIX))) return rc;
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv1_dgrad_affine_bwd_kernel<C>), DgSmem<C>::total)))
     return rc;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int ipt = Cfg::NPIX >> g.lgHW;
   const int tiles = (g.B + ipt - 1) / ipt;
   const cudaError_t le = launch_pdl(conv1_dgrad_affine_bwd_kernel<C>, dim3(tiles < sms ? tiles : sms),

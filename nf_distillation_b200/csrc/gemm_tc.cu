@@ -679,56 +679,6 @@ gemm_tn_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess)
-      return nullptr;
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
-// Row-major matrix [rows, cols] with leading dimension ld (elements); box = 128 bytes of columns x box_rows rows.
-static int make_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows,
-                     bool f32) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) return NFK_ERR_DRIVER;
-  const uint64_t es = f32 ? 4 : 2;
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld * es) % 16) return NFK_ERR_ALIGN;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * es};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(128 / es), box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                   const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? NFK_OK : NFK_ERR_DRIVER;
-}
-
-static int make_tmap_bf16(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld,
-                          uint32_t box_rows) {
-  return make_tmap(m, ptr, cols, rows, ld, box_rows, false);
-}
-
-static int num_sms() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-  }
-  return n;
-}
-
 static long long* g_prof_buffer = nullptr;   // set by nfk_gemm_set_prof (diagnostics only)
 
 static bool use_pairs() {
@@ -839,10 +789,10 @@ static int gemm_nt_launch(const void* A, long long lda, const void* B, long long
   g.prof = g_prof_buffer;
   CUtensorMap tmA, tmB, tmC;
   int rc;
-  if ((rc = make_tmap_bf16(&tmA, A, K, M, lda, BM)) != NFK_OK) return rc;
-  if ((rc = make_tmap_bf16(&tmB, B, K, N, ldb, pair ? g.BN / 2 : g.BN)) != NFK_OK) return rc;
+  if ((rc = make_tmap_2d(&tmA, A, K, M, lda, BM)) != NFK_OK) return rc;
+  if ((rc = make_tmap_2d(&tmB, B, K, N, ldb, pair ? g.BN / 2 : g.BN)) != NFK_OK) return rc;
   if (staged) {
-    if ((rc = make_tmap(&tmC, out, N, M, ldo, 32, f32)) != NFK_OK) return rc;
+    if ((rc = make_tmap_2d(&tmC, out, N, M, ldo, 32, f32)) != NFK_OK) return rc;
   } else {
     tmC = tmA;
   }
@@ -895,8 +845,8 @@ extern "C" int nfk_gemm_tn_bf16(const void* A, long long lda, const void* B, lon
     g.out = out; g.ldo = ldo;
     CUtensorMap ptmA, ptmB;
     int prc;
-    if ((prc = make_tmap_bf16(&ptmA, A, Mo, Kpix, lda, 64)) != NFK_OK) return prc;
-    if ((prc = make_tmap_bf16(&ptmB, B, No, Kpix, ldb, 64)) != NFK_OK) return prc;
+    if ((prc = make_tmap_2d(&ptmA, A, Mo, Kpix, lda, 64)) != NFK_OK) return prc;
+    if ((prc = make_tmap_2d(&ptmB, B, No, Kpix, ldb, 64)) != NFK_OK) return prc;
     const int psmem = g.stages * pstage + 1024 + 256;
     if ((prc = set_smem(gemm_tn_pair_kernel, psmem))) return prc;
     const cudaError_t ple = launch_pdl(gemm_tn_pair_kernel, dim3(2 * ptiles, psplits), dim3(TN_THREADS), psmem,
@@ -914,8 +864,8 @@ extern "C" int nfk_gemm_tn_bf16(const void* A, long long lda, const void* B, lon
   splits = (total_kb + g.kb_per_split - 1) / g.kb_per_split;
   CUtensorMap tmA, tmB;
   int rc;
-  if ((rc = make_tmap_bf16(&tmA, A, Mo, Kpix, lda, 64)) != NFK_OK) return rc;
-  if ((rc = make_tmap_bf16(&tmB, B, No, Kpix, ldb, 64)) != NFK_OK) return rc;
+  if ((rc = make_tmap_2d(&tmA, A, Mo, Kpix, lda, 64)) != NFK_OK) return rc;
+  if ((rc = make_tmap_2d(&tmB, B, No, Kpix, ldb, 64)) != NFK_OK) return rc;
   const int smem = g.stages * stage_bytes + 1024 + 256;
   if ((rc = set_smem(gemm_tn_kernel, smem))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);

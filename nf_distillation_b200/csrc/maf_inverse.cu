@@ -34,6 +34,7 @@
 #include <cstdint>
 
 #include "../../include/nfk.h"
+#include "launch_util.h"
 #include "ptx.cuh"
 
 namespace nfk {
@@ -1242,9 +1243,7 @@ static int mi_launch(MiArgs p, cudaStream_t st) {
   if (warps < 1) return NFK_ERR_SHAPE;
   const int wtiles = (p.B + MT * 16 - 1) / (MT * 16);
   if (warps > wtiles) warps = wtiles;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int smem = fixed + warps * per_warp;
   if (cudaFuncSetAttribute(made_inverse_resident_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) !=
       cudaSuccess)
@@ -1266,9 +1265,7 @@ static int mi_launch_push(MiArgs p, cudaStream_t st) {
   if (warps < 1) return NFK_ERR_SHAPE;
   const int wtiles = (p.B + 15) / 16;
   if (warps > wtiles) warps = wtiles;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int smem = fixed + warps * per_warp;
   if (cudaFuncSetAttribute(made_inverse_push_kernel<NO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) !=
       cudaSuccess)
@@ -1317,9 +1314,7 @@ static int mib_launch(MibArgs p, cudaStream_t st) {
   if (warps < 1) return NFK_ERR_SHAPE;
   const int wtiles = (p.B + MT * 16 - 1) / (MT * 16);
   if (warps > wtiles) warps = wtiles;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int smem = fixed + warps * per_warp;
   if (cudaFuncSetAttribute(made_inverse_bwd_resident_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) !=
       cudaSuccess)

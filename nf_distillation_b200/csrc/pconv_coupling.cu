@@ -294,44 +294,15 @@ pconv_coupling_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_cons
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-typedef CUresult (*EncodeTiledFn3)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-// bf16 [rows, cols] K-major tensor map, 64-column (128-byte, SWIZZLE_128B) boxes of box_rows rows; also used by
-// dgrad_col2im.cu
-int pc_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows) {
-  static EncodeTiledFn3 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return NFK_ERR_DRIVER;
-    fn = reinterpret_cast<EncodeTiledFn3>(p);
-  }
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld * 2) % 16) return NFK_ERR_ALIGN;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * 2};
-  cuuint32_t box[2] = {64, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? NFK_OK : NFK_ERR_DRIVER;
-}
-
 template <int C>
 static int pc_launch(const void* h2, const void* B3, int K3p, const PcArgs& g, int hid, cudaStream_t st) {
   using Cfg = PcCfg<C>;
   CUtensorMap tmW, tmH;
   int rc;
-  if ((rc = pc_tmap(&tmW, B3, hid, K3p, hid, 128))) return rc;
-  if ((rc = pc_tmap(&tmH, h2, hid, static_cast<uint64_t>(g.M), hid, Cfg::NPIX))) return rc;
+  if ((rc = make_tmap_2d(&tmW, B3, hid, K3p, hid, 128))) return rc;
+  if ((rc = make_tmap_2d(&tmH, h2, hid, static_cast<uint64_t>(g.M), hid, Cfg::NPIX))) return rc;
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(pconv_coupling_kernel<C>), PcSmem<C>::total))) return rc;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int tiles = g.banded ? g.B * g.nb : static_cast<int>((g.M + Cfg::NPIX - 1) / Cfg::NPIX);
   const cudaError_t le = launch_pdl(pconv_coupling_kernel<C>, dim3(tiles < sms ? tiles : sms), dim3(PC_THREADS),
                                     PcSmem<C>::total, st, tmW, tmH, g);

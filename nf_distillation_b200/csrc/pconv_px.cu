@@ -212,31 +212,6 @@ pconv_px_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-typedef CUresult (*EncodeTiledFn4)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int px_tmap(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t ld, uint32_t box_rows) {
-  static EncodeTiledFn4 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return NFK_ERR_DRIVER;
-    fn = reinterpret_cast<EncodeTiledFn4>(p);
-  }
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld * 2) % 16) return NFK_ERR_ALIGN;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld * 2};
-  cuuint32_t box[2] = {64, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? NFK_OK : NFK_ERR_DRIVER;
-}
-
 // C = 48 or 96, 4x4 maps, K3p >= 9 C rows of B3 [K3p, hid]. Returns NFK_ERR_SHAPE when the shape is not this kernel's.
 template <int C>
 static int px_launch(const void* h2, const void* B3, int K3p, const float* bias3, float* y, float* hsave, float* ld,
@@ -246,13 +221,11 @@ static int px_launch(const void* h2, const void* B3, int K3p, const float* bias3
   PxArgs g{static_cast<long long>(B) * 16, hid / 64, bias3, y, hsave, ld, reverse};
   CUtensorMap tmH, tmWA, tmWB;
   int rc;
-  if ((rc = px_tmap(&tmH, h2, hid, static_cast<uint64_t>(g.M), hid, 128))) return rc;
-  if ((rc = px_tmap(&tmWA, B3, hid, K3p, hid, Cfg::NA))) return rc;
-  if ((rc = px_tmap(&tmWB, B3, hid, K3p, hid, Cfg::NB))) return rc;
+  if ((rc = make_tmap_2d(&tmH, h2, hid, static_cast<uint64_t>(g.M), hid, 128))) return rc;
+  if ((rc = make_tmap_2d(&tmWA, B3, hid, K3p, hid, Cfg::NA))) return rc;
+  if ((rc = make_tmap_2d(&tmWB, B3, hid, K3p, hid, Cfg::NB))) return rc;
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(pconv_px_kernel<C>), PX_SMEM))) return rc;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = num_sms();
   const int tiles = static_cast<int>((g.M + 127) / 128);
   const cudaError_t le = launch_pdl(pconv_px_kernel<C>, dim3(tiles < sms ? tiles : sms), dim3(PX_THREADS), PX_SMEM, st,
                                     tmH, tmWA, tmWB, g);

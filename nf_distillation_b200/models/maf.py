@@ -281,7 +281,7 @@ class MADE(nn.Module):
         m2 = ops.relu_mask_like(Bn, H, dev) if keep else None
         h2 = torch.empty(Bn, H, device=dev, dtype=BF16)
         if ops.cnet_fused_supported(H, Dp) and Bn >= 8192:
-            # both masked linears in ONE kernel (the coupling net's fused conv#1 -> conv#2 kernel: h1 stays in shared
+            # both masked linears in ONE kernel (the coupling net's fused conv#1 -> conv#2 kernel: h1 stays in tensor
             # memory as the second GEMM's A operand and is only written out when training). The masks are zeros in the
             # bf16 weights here; skipping their k-blocks would save < what the h1 round trip through HBM costs.
             h1 = torch.empty(Bn, H, device=dev, dtype=BF16) if keep else None

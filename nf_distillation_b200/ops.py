@@ -456,8 +456,8 @@ def made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, wstream, jobs, g_u, 
                                             int(flip), int(mtiles), _st()), "nfk_made_inverse_bwd_resident")
 
 
-def cnet_fused_supported(hid, K1p) -> bool:
-    return hid == 512 and K1p % 64 == 0 and 64 <= K1p <= 512
+def cnet_fused_supported(hid, K) -> bool:
+    return bool(LIB.nfk_cnet_fused_supported(hid, K))
 
 
 def cnet_fwd_fused(col, K1p, B1, B2, bias1, bias2, h2, M, hid, h1=None, mask1=None, mask2=None, kb2_end_half0=8):

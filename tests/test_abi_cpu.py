@@ -36,6 +36,26 @@ def test_argument_errors_without_gpu():
     assert L.nfk_kd_mse_fwd(None, None, 4, 16, 1.0, None, None) == -3
 
 
+def test_fused_conv_kernel_shape_limits():
+    """nfk_cnet_fused_supported is the one statement of the fused conv kernel's shapes: hidden width 512 and a
+    first-GEMM depth K that is a multiple of 64 and leaves shared memory for two weight slots (K <= 448). The entry
+    points refuse K = 512 with NFK_ERR_SHAPE before any CUDA call, so callers take the two-GEMM path instead."""
+    from nf_distillation_b200 import _lib, ops
+    L = _lib.LIB
+    for K in (64, 128, 256, 448):
+        assert L.nfk_cnet_fused_supported(512, K) == 1 and ops.cnet_fused_supported(512, K), K
+    for hid, K in ((512, 512), (512, 100), (256, 128), (512, 0), (512, 1 << 30)):
+        assert L.nfk_cnet_fused_supported(hid, K) == 0 and not ops.cnet_fused_supported(hid, K), (hid, K)
+    M = 8192
+    assert L.nfk_cnet_fwd_fused(None, 512, None, None, None, None, None, None, None, None, M, M, 512, None) == -1
+    assert L.nfk_cnet_fwd_fused_ranged(None, 512, None, None, None, None, None, None, None, None, M, M, 512, 8,
+                                       None) == -1
+    assert L.nfk_cnet_bwd_fused(None, 512, None, None, None, None, M, None, None, None, None, M, 512, None) == -1
+    # a supported shape gets past the shape check to the argument checks (still no CUDA call)
+    assert L.nfk_cnet_fwd_fused(None, 448, None, None, None, None, None, None, None, None, M, M, 512, None) == -3
+    assert L.nfk_cnet_bwd_fused(None, 448, None, None, None, None, M, None, None, None, None, M, 512, None) == -3
+
+
 def test_state_dict_keys_and_module_tree():
     from nf_distillation_b200.models import FlowStep, SqueezeLayer, create_glow_model
     cfg = dict(image_shape=[32, 32, 3], hidden_channels=64, K=2, L=3, actnorm_scale=1.0,

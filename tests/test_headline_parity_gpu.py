@@ -164,10 +164,9 @@ def test_every_kernel_of_a_flowstep_is_exact_on_its_own_inputs(C, H, B):
 
 @pytest.mark.parametrize("M,K1p", [(8192, 64), (8200, 128), (33000, 256), (65536, 64)])
 def test_cnet_fused_kernel_is_bit_identical_to_the_two_gemms(M, K1p):
-    """The fused conv kernel the library dispatches to (csrc/cnet_ts.cu, h1 in tensor memory; NFK_CNET_TS=0:
-    csrc/cnet_fused.cu, h1 in shared-memory panels) against the two tcgen05 GEMMs it fuses (csrc/gemm_tc.cu): same bf16
-    products, same fp32 accumulation order per k-block -> h2 (both modes), h1 and both masks identical bit for bit;
-    ragged M included."""
+    """The fused conv kernel (csrc/cnet_ts.cu, h1 in tensor memory) against the two tcgen05 GEMMs it fuses
+    (csrc/gemm_tc.cu): same bf16 products, same fp32 accumulation order per k-block -> h2 (both modes), h1 and both
+    masks identical bit for bit; ragged M included."""
     from nf_distillation_b200 import ops
     hid = 512
     g = torch.Generator(device=dev).manual_seed(M + K1p)
@@ -188,18 +187,6 @@ def test_cnet_fused_kernel_is_bit_identical_to_the_two_gemms(M, K1p):
     assert torch.equal(m1a, m1b) and torch.equal(m2a, m2b)
     ref = torch.relu(col.float() @ B1.float().T + b1).bfloat16()
     assert rel(h1a, ref) < 1e-2
-
-
-def test_shared_memory_variant_of_the_fused_conv_kernels_stays_bit_identical():
-    """NFK_CNET_TS=0 (read once per process) selects the round-2 kernels of csrc/cnet_fused.cu; the forward and
-    backward bit-identity tests of this file are re-run against them in a child process."""
-    import subprocess
-    env = dict(os.environ, NFK_CNET_TS="0")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-m", "gpu", "-k",
-                        "bit_identical_to_the_two_gemms or matches_the_two_masked_gemms"], env=env, cwd=ROOT,
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "passed" in r.stdout and "failed" not in r.stdout
 
 
 # ------------------------------------------------------------------------------------------------ the KD step
@@ -599,7 +586,7 @@ def test_pipelined_trainer_makes_the_same_updates_as_the_sequential_one(use_grap
 
 @pytest.mark.parametrize("M,K3p", [(8192, 128), (8200, 256), (33000, 448), (65536, 128)])
 def test_cnet_bwd_fused_kernel_matches_the_two_masked_gemms(M, K3p):
-    """csrc/cnet_fused.cu in backward mode (both dgrads of the coupling net's chain in one kernel) against the two
+    """csrc/cnet_ts.cu in backward mode (both dgrads of the coupling net's chain in one kernel) against the two
     tcgen05 GEMMs with the ReLU-mask epilogue it replaces: same bf16 products, same k-block order -> dpre2 and dpre1
     identical bit for bit (ragged M included); the bias-gradient column sums agree to fp32 summation order."""
     from nf_distillation_b200 import ops

@@ -112,6 +112,32 @@ def test_resident_inverse_matches_paper_restatement(D, H, B, flip):
             assert none is None and torch.equal(x2, x)
 
 
+def test_made_forward_with_a_512_wide_input_runs_the_gemm_pair_at_a_large_batch():
+    """D = 500 pads to Dp = 512, deeper than the fused conv kernel takes (its A tile would leave shared memory for one
+    weight slot), so at a batch >= 8192 the forward runs the two GEMMs, in inference and in training (h1 and the ReLU
+    masks kept). Both against the fp32 restatement: u to 1e-3 of max; the log-det, a sum of 500 alphas computed by
+    the bf16 network, to 2e-3 of (max + 1) as in the resident-inverse test."""
+    from nf_distillation_b200 import ops
+    from nf_distillation_b200.models.maf import MADE
+    from oracle import maf_oracle as MO
+    D, H, B = 500, 512, 8192
+    torch.manual_seed(5)
+    made = MADE(D, H, flip=True)
+    with torch.no_grad():
+        made.fc3.bias.normal_(0, 0.1)
+    assert made.Dp == 512 and not ops.cnet_fused_supported(H, made.Dp)
+    sd = {"l." + k: v.clone() for k, v in made.state_dict().items()}
+    x = torch.randn(B, D)
+    u_o, ld_o = MO.made_forward(x, sd, "l.", D)
+    made = made.cuda()
+    with torch.no_grad():
+        u, ld = made(x.cuda(), logdet=torch.zeros(B, device="cuda"))
+    ld_tol = 2e-3 * (ld_o.abs().max().item() + 1)
+    assert rel(u, u_o) < 1e-3 and (ld.cpu() - ld_o).abs().max().item() < ld_tol
+    u2, ld2 = made(x.cuda(), logdet=torch.zeros(B, device="cuda"))
+    assert u2.requires_grad and rel(u2, u_o) < 1e-3 and (ld2.detach().cpu() - ld_o).abs().max().item() < ld_tol
+
+
 def test_masked_tile_skipping_is_exact():
     """The ranged GEMM (structurally-zero k-blocks never loaded) equals the full GEMM on the masked weight, bit for bit."""
     from nf_distillation_b200 import ops

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstdint>
+#include "../../nf_distillation_b200/csrc/launch_util.h"
 #include "../../nf_distillation_b200/csrc/ptx.cuh"
 using namespace nfk;
 
@@ -36,14 +37,7 @@ bench(const __grid_constant__ CUtensorMap tm, int rows, int slots, int iters, in
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 int main() {
-  void* fp = nullptr; cudaDriverEntryPointQueryResult q;
-  cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &q);
-  EncodeTiledFn enc = reinterpret_cast<EncodeTiledFn>(fp);
   void* w; cudaMalloc(&w, 512 * 512 * 2); cudaMemset(w, 0, 512 * 512 * 2);
   long long* d; cudaMalloc(&d, 148 * 8);
   cudaFuncSetAttribute(bench, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
@@ -51,9 +45,7 @@ int main() {
   for (int grid : {148}) for (int rows : {64}) for (int slots : {4}) for (int per : {1, 2}) for (int mode : {0, 1, 2}) {
     if (rows * 128 * slots * per > 190 * 1024) continue;
     CUtensorMap tm;
-    cuuint64_t dims[2] = {512, 512}; cuuint64_t strides[1] = {1024}; cuuint32_t box[2] = {64, (cuuint32_t)rows}; cuuint32_t es[2] = {1, 1};
-    enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (make_tmap_2d(&tm, w, 512, 512, 512, rows) != NFK_OK) { printf("tensor map encode failed\n"); return 1; }
     // phase bookkeeping above is simplistic: use iters multiple of slots
     for (int rep = 0; rep < 2; ++rep) {
       bench<<<grid, 64, 200 * 1024>>>(tm, rows, slots, iters, per, mode, d);

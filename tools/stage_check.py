@@ -89,7 +89,7 @@ def run(C, H, B, hid=512):
         stats("dhcol", dhcol[:, :9 * C], dhcol_r.to(BF), bf16=True)
         dpre2 = torch.empty(M, hid, device=dev, dtype=BF); dbias2 = torch.zeros(hid, device=dev)
         dpre1 = torch.empty(M, hid, device=dev, dtype=BF); dbias1 = torch.zeros(hid, device=dev)
-        fused_bwd = Fn.USE_FUSED_CNET_BWD and ops.cnet_fused_supported(hid, K3p) and M >= 8192
+        fused_bwd = ops.cnet_fused_supported(hid, K3p) and M >= 8192
         if fused_bwd:     # the path FlowStep2dFn.backward takes at this size: both dgrads in one kernel
             ops.cnet_bwd_fused(dhcol, K3p, k.B3T, k.B2T, m2, m1, dpre2, dpre1, dbias2, dbias1, M, hid)
         else:
