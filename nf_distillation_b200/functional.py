@@ -308,7 +308,7 @@ def _coupling_net(col, k: StepConsts, M, hid, K1p, K3p, keep):
     m2 = ops.relu_mask_like(M, hid, dev) if keep else None
     h1 = torch.empty(M, hid, device=dev, dtype=BF16) if keep else None
     h2 = torch.empty(M, hid, device=dev, dtype=BF16)
-    if ops.cnet_fused_supported(hid, K1p) and M >= 8192:
+    if ops.cnet_fused_supported(hid, K1p, M):
         # one kernel for conv#1 + conv#2: h1 stays in tensor memory (and is only written out when training)
         ops.cnet_fwd_fused(col, K1p, k.B1, k.B2, k.bias1, k.bias2, h2, M, hid, h1=h1, mask1=m1, mask2=m2)
     else:
@@ -392,7 +392,7 @@ def _coupling_net_backward(dhcol, col, h1, h2, m1, m2, B1T, B2T, B3T, dbias2, db
     dev = dhcol.device
     dpre2 = torch.empty(M, hid, device=dev, dtype=BF16)
     dpre1 = torch.empty(M, hid, device=dev, dtype=BF16)
-    if ops.cnet_fused_supported(hid, K3p) and M >= 8192:
+    if ops.cnet_fused_supported(hid, K3p, M):
         # both dgrads of the chain in ONE kernel: dpre2 stays in tensor memory as the second GEMM's A operand
         ops.cnet_bwd_fused(dhcol, K3p, B3T, B2T, m2, m1, dpre2, dpre1, dbias2, dbias1, M, hid)
     else:

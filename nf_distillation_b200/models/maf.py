@@ -63,11 +63,53 @@ def _kb_ranges_t(deg_out, deg_in, bn):
     return begins, ends
 
 
+class _MadePlan:
+    """What one degree assignment (deg1, deg2) fixes, derived on the host once per assignment (MADE._plan): sorted
+    (both ascending), resident_ok (sorted, no degree 0: what the resident inverse and the reverse solve need), the
+    k-block ranges of the H x H masked linear and of its transpose (full when unsorted), the fused kernel's
+    kb2_end_half0, the resident inverse's job table (on the degrees' device), push flag and stream bytes, and the
+    reverse solve's job table and stream bytes (None when not resident_ok or the shape does not fit the kernel).
+    It holds the degree tensors it was built from, so no pointer in `key` can be reused while it is alive."""
+
+    def __init__(self, made, key):
+        self.key, self.deg1, self.deg2 = key, made.deg1, made.deg2
+        d1, d2 = self.deg1.detach().cpu().long(), self.deg2.detach().cpu().long()
+        D, H, Dp, N3p, bn = made.D, made.H, made.Dp, made.N3p, made.bn
+        nkb = H // 64
+        self.sorted = bool((d1[1:] >= d1[:-1]).all() and (d2[1:] >= d2[:-1]).all())
+        self.resident_ok = self.sorted and bool(d1.min() >= 1 and d2.min() >= 1)
+        if self.sorted:
+            self.ranges, self.ranges_t = _kb_ranges(d2, d1, bn), _kb_ranges_t(d2, d1, bn)
+            self.kb2_end_half0 = _kb_ranges(d2, d1, 256)[1][0] if H == 512 else nkb
+        else:
+            nt = (H + bn - 1) // bn
+            self.ranges = self.ranges_t = ([0] * nt, [nkb] * nt)
+            self.kb2_end_half0 = nkb
+        self.jobs, self.push, self.nbytes, self.bwd_jobs, self.bwd_nbytes = None, False, 0, None, 0
+        if not self.resident_ok:
+            return
+        edges = torch.arange(D + 1)
+        cnt1, cnt2 = ((d[None, :] <= edges[:, None]).sum(1) for d in (d1, d2))   # cnt[d] = units of degree <= d
+        dev = self.deg1.device
+        if ops.made_inverse_resident_supported(D, H, Dp):
+            jobs = None
+            if made.push_inverse and ops.made_inverse_push_supported(D, H, Dp, N3p):
+                jobs = ops.made_inverse_jobs(cnt1, cnt2, D, H, Dp, N3p, push=True)
+                self.push = jobs is not None
+            if jobs is None:
+                jobs = ops.made_inverse_jobs(cnt1, cnt2, D, H, Dp)
+            self.jobs, self.nbytes = jobs.to(dev), int(jobs[:, 5].sum()) * 16
+        if ops.made_inverse_bwd_supported(D, H, N3p):
+            jobs = ops.made_inverse_bwd_jobs(cnt1, cnt2, D, H, N3p)
+            self.bwd_jobs, self.bwd_nbytes = jobs.to(dev), int(jobs[:, 5].sum()) * 16
+
+
 class _MadeFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, ld_in, made, flip, xb, w1, b1, w2, b2, w3, b3):
         x = x.contiguous()
-        u, ld_out, ub, saved = made._run_forward(x, ld_in.contiguous(), (w1, b1, w2, b2, w3, b3), flip, True, xb)
+        ops_ = made._operands((w1, b1, w2, b2, w3, b3), True)
+        u, ld_out, ub, saved = made._run_forward(x, ld_in.contiguous(), ops_, b1, b2, flip, True, xb)
         ctx.made, ctx.flip = made, flip
         ctx.save_for_backward(x, *saved)
         ctx.mark_non_differentiable(ub)
@@ -115,7 +157,7 @@ def _made_net_backward(made, dout, xb, h1, h2, m1, m2, B1T, B2T, B3T, grads, wan
     ops.gemm_nt(dout, B3T, B, H, N3p, ops.EPI_MASK_BF16, dpre2, aux=m2, colsum=db2)
     ops.gemm_tn(dout, h2, N3p, H, B, dB3)
     dpre1 = torch.empty(B, H, device=dev, dtype=BF16)
-    kb0, kb1 = made._ranges_t
+    kb0, kb1 = made._plan().ranges_t
     ops.gemm_nt_ranged(dpre2, B2T, B, H, H, ops.EPI_MASK_BF16, dpre1, made.bn, kb0, kb1, aux=m1, colsum=db1)
     ops.gemm_tn(dpre2, h1, H, H, B, dB2)
     dxn = None
@@ -181,80 +223,39 @@ class MADE(nn.Module):
         deg = hidden_degrees(D, H)
         self.register_buffer("deg1", deg.clone())
         self.register_buffer("deg2", deg.clone())
-        self._range_cache = None
-        self._cache = None
-        self._job_cache = None
-        self._bwd_job_cache = None
-        self._stream_cache = None
-        self._stream_bytes = 0
+        self._plan_cache = None   # _MadePlan of the current degree buffers
+        self._cache = None        # no-grad operands: [param_key, plan, operands, resident inverse's weight stream]
         self.push_inverse = True         # False: the pull kernel (h2 kept in shared memory) even for aligned degrees
         self.resident_inverse = True     # False: the D-pass GEMM inverse and reverse solve (the cross-checks in the tests)
         self.resident_mtiles = 0         # 16-sample tiles per warp in the resident inverse (0 = chosen by the library)
 
-    def _kb_ranges_now(self):
-        """(forward, transposed) k-block skip ranges of the H x H masked linear for the CURRENT degree buffers (a
-        loaded checkpoint may carry other degrees than the constructor's). Unsorted degrees have no block-triangular
-        structure to skip: full ranges."""
-        key = (self.deg1.data_ptr(), self.deg1._version, self.deg2.data_ptr(), self.deg2._version)
-        if self._range_cache is None or self._range_cache[0] != key:
-            d1, d2 = self.deg1.detach().cpu().long(), self.deg2.detach().cpu().long()
-            nkb = self.H // 64
-            if bool((d1[1:] >= d1[:-1]).all() and (d2[1:] >= d2[:-1]).all()):
-                r, rt = _kb_ranges(d2, d1, self.bn), _kb_ranges_t(d2, d1, self.bn)
-                half0 = _kb_ranges(d2, d1, 256)[1][0] if self.H == 512 else nkb   # fused kernel: outputs [0, 256)
-            else:
-                nt = (self.H + self.bn - 1) // self.bn
-                r = rt = ([0] * nt, [nkb] * nt)
-                half0 = nkb
-            self._range_cache = (key, (r, rt, half0))
-        return self._range_cache[1]
+    def _plan(self):
+        """The plan of the current degree buffers (a loaded checkpoint may carry other degrees than the constructor's)
+        and push_inverse. Building one reads the degrees to the host, so the first eager call builds it: a CUDA graph
+        captured after that finds it here."""
+        d1, d2 = self.deg1, self.deg2
+        key = (d1.data_ptr(), d1._version, d2.data_ptr(), d2._version, str(d1.device), self.push_inverse)
+        if self._plan_cache is None or self._plan_cache.key != key:
+            self._plan_cache = _MadePlan(self, key)
+        return self._plan_cache
 
-    @property
-    def _fused_kb_end_half0(self):
-        return self._kb_ranges_now()[2]
-
+    # views of the plan: (job table on `dev`, push?) of the resident inverse, (job table, stream bytes) or None of
+    # the reverse solve
     @property
     def _ranges(self):
-        return self._kb_ranges_now()[0]
-
-    @property
-    def _ranges_t(self):
-        return self._kb_ranges_now()[1]
+        return self._plan().ranges
 
     def _inverse_jobs(self, dev):
-        """(job table on `dev`, push?) of the resident inverse (ops.made_inverse_jobs), from cnt[d] = number of hidden
-        units with degree <= d (d = 0..D); (None, False) when the degrees are not sorted ascending (the resident
-        inverse walks the units in degree order). push = the degrees change on whole 8-unit tiles and 2D <= 128."""
-        key = (self.deg1.data_ptr(), self.deg1._version, self.deg2.data_ptr(), self.deg2._version, str(dev),
-               self.push_inverse)
-        if self._job_cache is None or self._job_cache[0] != key:
-            d1, d2 = self.deg1.detach().cpu().long(), self.deg2.detach().cpu().long()
-            ok = bool((d1[1:] >= d1[:-1]).all() and (d2[1:] >= d2[:-1]).all() and d1.min() >= 1 and d2.min() >= 1)
-            jobs, push = None, False
-            if ok:
-                edges = torch.arange(self.D + 1)
-                cnt1, cnt2 = ((d[None, :] <= edges[:, None]).sum(1) for d in (d1, d2))
-                if self.push_inverse and ops.made_inverse_push_supported(self.D, self.H, self.Dp, self.N3p):
-                    jobs = ops.made_inverse_jobs(cnt1, cnt2, self.D, self.H, self.Dp, self.N3p, push=True)
-                    push = jobs is not None
-                if jobs is None:
-                    jobs = ops.made_inverse_jobs(cnt1, cnt2, self.D, self.H, self.Dp)
-                self._stream_bytes = int(jobs[:, 5].sum()) * 16     # (host tensor: no device sync later)
-                jobs = jobs.to(dev)
-            self._job_cache = (key, (jobs, push))
-        return self._job_cache[1]
+        plan = self._plan()
+        return (None if plan.jobs is None else plan.jobs.to(dev)), plan.push
 
-    def _weight_stream(self, jobs, push, ops_):
-        """The packed weight stream of the resident inverse for the current operands (rebuilt when they change)."""
-        key = (jobs.data_ptr(), push, ops_[0].data_ptr(), ops_[0]._version)
-        if self._stream_cache is None or self._stream_cache[0] != key:
-            ws = self._pack_stream(jobs, push, ops_)
-            self._stream_cache = (key, ws, ops_[0])   # (keeps B1 alive so the pointer in the key cannot be reused)
-        return self._stream_cache[1]
+    def _inverse_bwd_jobs(self, dev):
+        plan = self._plan()
+        return None if plan.bwd_jobs is None else (plan.bwd_jobs.to(dev), plan.bwd_nbytes)
 
-    def _pack_stream(self, jobs, push, ops_):
-        ws = torch.zeros(max(self._stream_bytes, 128), device=jobs.device, dtype=torch.uint8)
-        ops.made_inverse_pack(jobs, ops_[0], ops_[2], ops_[4], self.N3p, self.D, self.H, self.Dp, push, ws)
+    def _pack_stream(self, plan, ops_):
+        ws = torch.zeros(max(plan.nbytes, 128), device=plan.jobs.device, dtype=torch.uint8)
+        ops.made_inverse_pack(plan.jobs, ops_[0], ops_[2], ops_[4], self.N3p, self.D, self.H, self.Dp, plan.push, ws)
         return ws
 
     def _params(self):
@@ -272,15 +273,32 @@ class MADE(nn.Module):
         b3p[:2 * D] = b3
         return B1, B1T, B2, B2T, B3, B3T, b3p
 
+    def _cached_operands(self):
+        """The operands of the current parameters for no-grad calls, cached on param_key and the plan: made_prep bakes
+        the degree masks into them."""
+        key, plan = Fn.param_key(self._params()), self._plan()
+        if self._cache is None or self._cache[0] != key or self._cache[1] is not plan:
+            self._cache = [key, plan, self._operands(tuple(p.detach() for p in self._params()), False), None]
+        return self._cache[2]
+
+    def _cached_stream(self):
+        """The resident inverse's packed weight stream of _cached_operands(), kept in the same cache entry, which holds
+        the plan and operands it was packed from."""
+        ops_ = self._cached_operands()
+        if self._cache[3] is None:
+            self._cache[3] = self._pack_stream(self._cache[1], ops_)
+        return self._cache[3]
+
     def _net(self, xb, Bn, ops_, b1, b2, keep=False):
         """(mu | alpha) = masked MLP(xb) on the tensor cores; returns h1, h2, out (+ 1-bit ReLU masks if keep)."""
         B1, _, B2, _, B3, _, b3p = ops_
         dev = xb.device
         H, Dp, N3p = self.H, self.Dp, self.N3p
+        plan = self._plan()
         m1 = ops.relu_mask_like(Bn, H, dev) if keep else None
         m2 = ops.relu_mask_like(Bn, H, dev) if keep else None
         h2 = torch.empty(Bn, H, device=dev, dtype=BF16)
-        if ops.cnet_fused_supported(H, Dp) and Bn >= 8192:
+        if ops.cnet_fused_supported(H, Dp, Bn):
             # both masked linears in ONE kernel (the coupling net's fused conv#1 -> conv#2 kernel: h1 stays in tensor
             # memory as the second GEMM's A operand and is only written out when training). The masks are zeros in the
             # bf16 weights here; skipping their k-blocks would save < what the h1 round trip through HBM costs.
@@ -288,11 +306,11 @@ class MADE(nn.Module):
             # k-blocks of the hidden weight that output channels [0, 256) can see (block-triangular mask): the rest
             # are exact zeros in B2 and are skipped
             ops.cnet_fwd_fused(xb, Dp, B1, B2, b1, b2, h2, Bn, H, h1=h1, mask1=m1, mask2=m2,
-                               kb2_end_half0=self._fused_kb_end_half0)
+                               kb2_end_half0=plan.kb2_end_half0)
         else:
             h1 = torch.empty(Bn, H, device=dev, dtype=BF16)
             ops.gemm_nt(xb, B1, Bn, H, Dp, ops.EPI_BIAS_RELU_BF16, h1, bias=b1, aux=m1)
-            kb0, kb1 = self._ranges
+            kb0, kb1 = plan.ranges
             ops.gemm_nt_ranged(h1, B2, Bn, H, H, ops.EPI_BIAS_RELU_BF16, h2, self.bn, kb0, kb1, bias=b2, aux=m2)
         out = torch.empty(Bn, N3p, device=dev, dtype=F32)
         ops.gemm_nt(h2, B3, Bn, N3p, H, ops.EPI_F32, out, bias=b3p)
@@ -308,24 +326,19 @@ class MADE(nn.Module):
         ops.rows_to_bf16(x, Bn, self.D, self.Dp, xb)
         return xb
 
-    def _run_forward(self, x, ld_in, params, flip, keep, xb=None):
+    def _run_forward(self, x, ld_in, ops_, b1, b2, flip, keep, xb=None):
+        """u = MADE(x) and ld_out = ld_in - sum alpha from the operands ops_; keep: also returns what _MadeFn's
+        backward saves. ub is u's bf16 copy for the next layer's first GEMM."""
         Bn = x.shape[0]
         dev = x.device
-        ops_ = self._operands(params, keep)
         xb = self._bf16_rows(x, xb)
-        res = self._net(xb, Bn, ops_, params[1], params[3], keep)
+        res = self._net(xb, Bn, ops_, b1, b2, keep)
         h1, h2, out = res[:3]
         u = torch.empty_like(x)
         ub = torch.empty(Bn, self.Dp, device=dev, dtype=BF16)   # the next layer's GEMM operand
         ld_out = torch.empty(Bn, device=dev, dtype=F32)
         ops.made_affine_fwd(x, out, self.N3p, u, ub, self.Dp, ld_in, ld_out, Bn, self.D, flip)
         return u, ld_out, ub, ((xb, h1, h2, res[3], res[4], out, ops_[1], ops_[3], ops_[5]) if keep else None)
-
-    def _cached_operands(self):
-        key = Fn.param_key(self._params())
-        if self._cache is None or self._cache[0] != key:
-            self._cache = (key, self._operands(tuple(p.detach() for p in self._params()), False))
-        return self._cache[1]
 
     def forward(self, input, y_onehot=None, logdet=None, reverse=False, **kwargs):
         _require_cuda(input, "MADE")
@@ -342,13 +355,9 @@ class MADE(nn.Module):
                 u, ld_out, ub = _MadeFn.apply(input, ld, self, self.flip, xb_in, *params)
             else:
                 x = input.contiguous()
-                ops_ = self._cached_operands()
-                xb = self._bf16_rows(x, xb_in if x is input else None)
-                _, _, out = self._net(xb, Bn, ops_, params[1].detach(), params[3].detach())
-                u = torch.empty_like(x)
-                ub = torch.empty(Bn, self.Dp, device=x.device, dtype=BF16)
-                ld_out = torch.empty(Bn, device=x.device, dtype=F32)
-                ops.made_affine_fwd(x, out, self.N3p, u, ub, self.Dp, ld.contiguous(), ld_out, Bn, self.D, self.flip)
+                u, ld_out, ub, _ = self._run_forward(x, ld.contiguous(), self._cached_operands(), params[1].detach(),
+                                                     params[3].detach(), self.flip, False,
+                                                     xb_in if x is input else None)
             u._nfk_bf16 = (ub, u._version)   # bf16 copy for the next MADE layer (saves its conversion pass)
             return u, (ld_out if want else None)
         if torch.is_grad_enabled() and (input.requires_grad or ld.requires_grad or any(p.requires_grad for p in params)):
@@ -358,22 +367,27 @@ class MADE(nn.Module):
 
     def _run_inverse(self, u_in, ld, want, params=None):
         """x = MADE^-1(u_in) and (want) ld_out = ld + sum alpha, without gradients. params=None (frozen modules:
-        no-grad calls): the operands and the packed weight stream come from the caches keyed by the parameters'
-        versions and the parameter epoch. Given params (the trainable path): both are rebuilt from them on every call,
-        as the forward's _MadeFn does, because an optimiser that writes the parameters through raw pointers (FlatAdam)
-        bumps no version, and a captured graph must contain the rebuild."""
+        no-grad calls): the operands and the packed weight stream come from _cached_operands / _cached_stream. Given
+        params (the trainable path): both are rebuilt from them on every call, as the forward's _MadeFn does, because
+        an optimiser that writes the parameters through raw pointers (FlatAdam) bumps no version, and a captured graph
+        must contain the rebuild."""
         Bn = u_in.shape[0]
-        cached = params is None
-        params = self._params() if cached else tuple(p.detach() for p in params)
-        ops_ = self._cached_operands() if cached else self._operands(params, False)
-        jobs, push = self._inverse_jobs(u_in.device)
-        if jobs is not None and self.resident_inverse and ops.made_inverse_resident_supported(self.D, self.H, self.Dp):
+        plan = self._plan()
+        resident = plan.jobs is not None and self.resident_inverse
+        if params is None:
+            params = self._params()
+            ops_ = self._cached_operands()
+            ws = self._cached_stream() if resident else None
+        else:
+            params = tuple(p.detach() for p in params)
+            ops_ = self._operands(params, False)
+            ws = self._pack_stream(plan, ops_) if resident else None
+        b1, b2 = params[1].detach(), params[3].detach()
+        if resident:
             # ONE launch: every hidden unit finalised once, in degree order, activations resident in shared memory
             x = torch.empty_like(u_in)
             ld_out = torch.empty(Bn, device=x.device, dtype=F32) if want else None
-            ws = self._weight_stream(jobs, push, ops_) if cached else self._pack_stream(jobs, push, ops_)
-            ops.made_inverse_resident(u_in, ws, params[1].detach(),
-                                      params[3].detach(), ops_[6], jobs, push, self.N3p, x,
+            ops.made_inverse_resident(u_in, ws, b1, b2, ops_[6], plan.jobs, plan.push, self.N3p, x,
                                       ld.contiguous() if want else None, ld_out, Bn, self.D, self.H, self.Dp,
                                       self.flip, self.resident_mtiles)
             return x, ld_out
@@ -384,49 +398,32 @@ class MADE(nn.Module):
         ld_out = torch.empty(Bn, device=x.device, dtype=F32)
         ldc = ld.contiguous()
         for i in range(self.D):
-            _, _, out = self._net(xb, Bn, ops_, params[1].detach(), params[3].detach())
+            _, _, out = self._net(xb, Bn, ops_, b1, b2)
             ops.made_inv_update(x, xb, self.Dp, u_in, out, self.N3p, ldc, ld_out, Bn, self.D, i, self.flip,
                                 i == self.D - 1)
         return x, (ld_out if want else None)
 
-    def _inverse_bwd_jobs(self, dev):
-        """Job table of the one-launch reverse solve on `dev` (ops.made_inverse_bwd_jobs), planned on the host once
-        per degree assignment; None when the degrees are not sorted ascending or the shape does not fit."""
-        key = (self.deg1.data_ptr(), self.deg1._version, self.deg2.data_ptr(), self.deg2._version, str(dev))
-        if self._bwd_job_cache is None or self._bwd_job_cache[0] != key:
-            d1, d2 = self.deg1.detach().cpu().long(), self.deg2.detach().cpu().long()
-            jobs = None
-            if (bool((d1[1:] >= d1[:-1]).all() and (d2[1:] >= d2[:-1]).all() and d1.min() >= 1 and d2.min() >= 1)
-                    and ops.made_inverse_bwd_supported(self.D, self.H, self.N3p)):
-                edges = torch.arange(self.D + 1)
-                cnt1, cnt2 = ((d[None, :] <= edges[:, None]).sum(1) for d in (d1, d2))
-                jobs = ops.made_inverse_bwd_jobs(cnt1, cnt2, self.D, self.H, self.N3p)
-                jobs = (jobs.to(dev), int(jobs[:, 5].sum()) * 16)
-            self._bwd_job_cache = (key, jobs)
-        return self._bwd_job_cache[1]
-
     def _inverse_solve(self, g_x, g_ld, u_in, out, m1, m2, ops_, flip, g_u, dout, db3):
         """Reverse solve of the inverse's gradients at x (out, m1, m2 from the forward network recomputed at x):
-        writes g_u, dout = [mubar | alphabar | 0] and adds dout's column sums to db3. One launch when the degrees are
-        sorted and the shape fits (and resident_inverse is on); else D passes of the three dgrad GEMMs."""
+        writes g_u, dout = [mubar | alphabar | 0] and adds dout's column sums to db3. One launch when the plan has
+        the reverse solve's jobs (and resident_inverse is on); else D passes of the three dgrad GEMMs."""
         B = u_in.shape[0]
         D, H, Dp, N3p = self.D, self.H, self.Dp, self.N3p
         _, B1T, _, B2T, _, B3T, _ = ops_
-        plan = self._inverse_bwd_jobs(u_in.device) if self.resident_inverse else None
-        if plan is not None:
-            jobs, nbytes = plan
+        plan = self._plan()
+        if plan.bwd_jobs is not None and self.resident_inverse:
             # (no memset: the pack writes every row the kernel multiplies; the bytes it leaves alone are only read
             # into MMA columns the kernel discards)
-            ws = torch.empty(max(nbytes, 128), device=u_in.device, dtype=torch.uint8)
-            ops.made_inverse_bwd_pack(jobs, B1T, B2T, B3T, D, H, N3p, ws)
-            ops.made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, ws, jobs, g_u, dout, db3, B, D, H, N3p, flip,
-                                          self.resident_mtiles)
+            ws = torch.empty(max(plan.bwd_nbytes, 128), device=u_in.device, dtype=torch.uint8)
+            ops.made_inverse_bwd_pack(plan.bwd_jobs, B1T, B2T, B3T, D, H, N3p, ws)
+            ops.made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, ws, plan.bwd_jobs, g_u, dout, db3, B, D, H,
+                                          N3p, flip, self.resident_mtiles)
             return
         dout.zero_()
         c = torch.empty(B, Dp, device=u_in.device, dtype=F32)
         dpre2 = torch.empty(B, H, device=u_in.device, dtype=BF16)
         dpre1 = torch.empty(B, H, device=u_in.device, dtype=BF16)
-        kb0, kb1 = self._ranges_t
+        kb0, kb1 = plan.ranges_t
         for d in reversed(range(D)):
             if d < D - 1:   # c = the network's input gradient for the rows finished so far
                 ops.gemm_nt(dout, B3T, B, H, N3p, ops.EPI_MASK_BF16, dpre2, aux=m2)

@@ -456,8 +456,11 @@ def made_inverse_bwd_resident(g_x, g_ld, out, m1, m2, u_in, wstream, jobs, g_u, 
                                             int(flip), int(mtiles), _st()), "nfk_made_inverse_bwd_resident")
 
 
-def cnet_fused_supported(hid, K) -> bool:
-    return bool(LIB.nfk_cnet_fused_supported(hid, K))
+def cnet_fused_supported(hid, K, M=None) -> bool:
+    """Whether the coupling net (or MADE's two masked linears) on M rows of depth K at hidden width `hid` runs as the
+    fused conv#1 -> conv#2 kernel rather than two GEMMs: the kernel takes the shape (nfk_cnet_fused_supported) and
+    M >= 8192. M=None asks about the shape alone."""
+    return (M is None or M >= 8192) and bool(LIB.nfk_cnet_fused_supported(hid, K))
 
 
 def cnet_fwd_fused(col, K1p, B1, B2, bias1, bias2, h2, M, hid, h1=None, mask1=None, mask2=None, kb2_end_half0=8):

@@ -46,6 +46,9 @@ def test_fused_conv_kernel_shape_limits():
         assert L.nfk_cnet_fused_supported(512, K) == 1 and ops.cnet_fused_supported(512, K), K
     for hid, K in ((512, 512), (512, 100), (256, 128), (512, 0), (512, 1 << 30)):
         assert L.nfk_cnet_fused_supported(hid, K) == 0 and not ops.cnet_fused_supported(hid, K), (hid, K)
+    # the dispatch rule: a supported shape with at least 8192 rows; fewer rows run the two GEMMs
+    assert ops.cnet_fused_supported(512, 64, 8192) and ops.cnet_fused_supported(512, 448, 1 << 20)
+    assert not ops.cnet_fused_supported(512, 64, 8191) and not ops.cnet_fused_supported(512, 512, 1 << 20)
     M = 8192
     assert L.nfk_cnet_fwd_fused(None, 512, None, None, None, None, None, None, None, None, M, M, 512, None) == -1
     assert L.nfk_cnet_fwd_fused_ranged(None, 512, None, None, None, None, None, None, None, None, M, M, 512, 8,

@@ -80,7 +80,7 @@ def test_flowstep_hidden512_forward_backward_all_fused_variants(C, H, B):
     from nf_distillation_b200 import functional as Fn
     from nf_distillation_b200 import ops
     hid = 512
-    assert B * H * H >= 8192 and ops.cnet_fused_supported(hid, ops.round_up(9 * C // 2, 64))
+    assert ops.cnet_fused_supported(hid, ops.round_up(9 * C // 2, 64), B * H * H)
     st, sd = make_step(C, hid, 100 + C)
     g = torch.Generator().manual_seed(C)
     x = torch.randn(B, C, H, H, generator=g)

@@ -112,6 +112,43 @@ def test_resident_inverse_matches_paper_restatement(D, H, B, flip):
             assert none is None and torch.equal(x2, x)
 
 
+def test_no_grad_calls_follow_degrees_written_in_place():
+    """A frozen layer's cached operands carry the masks of the degrees they were built with. After a no-grad forward
+    and inverse, another valid degree assignment is written into deg1 / deg2 in place, the weights untouched: the
+    next forward (fused kernel, B = 8192) and inverse (pull kernel: the new degrees do not change on whole 8-unit
+    tiles) compute with the new masks, against the fp32 restatement at the new degrees (u 1e-3, x 2e-3 of max,
+    log-dets 2e-3 of max + 1). fc3's weights are scaled by 3 so the old masks would miss those bounds several times
+    over."""
+    from nf_distillation_b200.models.maf import MADE
+    from oracle import maf_oracle as MO
+    D, H, B = 63, 512, 8192
+    torch.manual_seed(11)
+    made = MADE(D, H, flip=True)
+    with torch.no_grad():
+        made.fc3.weight.mul_(3.0)
+        made.fc3.bias.normal_(0, 0.1)
+    sd_old = {"l." + k: v.clone() for k, v in made.state_dict().items()}
+    g = torch.Generator().manual_seed(12)
+    x, u = torch.randn(B, D, generator=g), torch.randn(B, D, generator=g)
+    made = made.cuda()
+    with torch.no_grad():
+        made(x.cuda(), logdet=torch.zeros(B, device="cuda"))
+        made(u.cuda(), logdet=torch.zeros(B, device="cuda"), reverse=True)
+        made.deg1.copy_(torch.randint(1, D, (H,), generator=g).sort().values)
+        made.deg2.copy_(torch.randint(1, D, (H,), generator=g).sort().values)
+        u_p, ld_p = made(x.cuda(), logdet=torch.zeros(B, device="cuda"))
+        x_p, ldi_p = made(u.cuda(), logdet=torch.zeros(B, device="cuda"), reverse=True)
+    sd = {"l." + k: v.cpu().clone() for k, v in made.state_dict().items()}
+    u_o, ld_o = MO.made_forward(x, sd, "l.", D)
+    x_o, sa_o = MO.made_inverse(u, sd, "l.", D)
+    ld_err = lambda a, b: (a.cpu() - b).abs().max().item() / (b.abs().max().item() + 1)
+    u_old, ld_old = MO.made_forward(x, sd_old, "l.", D)
+    assert rel(u_old, u_o) > 5e-3 and ld_err(ld_old, ld_o) > 1e-2      # the old masks would fail the checks below
+    assert rel(u_p, u_o) < 1e-3 and ld_err(ld_p, ld_o) < 2e-3
+    assert rel(x_p, x_o) < 2e-3 and ld_err(ldi_p, sa_o) < 2e-3
+    assert not made._plan().push
+
+
 def test_made_forward_with_a_512_wide_input_runs_the_gemm_pair_at_a_large_batch():
     """D = 500 pads to Dp = 512, deeper than the fused conv kernel takes (its A tile would leave shared memory for one
     weight slot), so at a batch >= 8192 the forward runs the two GEMMs, in inference and in training (h1 and the ReLU

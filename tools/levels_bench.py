@@ -41,7 +41,7 @@ for (C, H) in ((12, 16), (24, 8), (48, 4)):
     B3 = (torch.randn(K3p, hid, device=dev) * 0.02).to(bf16)
     b1, b2, b3 = torch.zeros(hid, device=dev), torch.zeros(hid, device=dev), torch.zeros(C, device=dev)
     ta = time_graph(lambda i: ops.affine1x1_fwd(xs[i], Wf, bfv, sl, ys[i], cols[i], K1p, ld, ld1, B, C, H, W), 16, nb)
-    if ops.cnet_fused_supported(hid, K1p) and M >= 8192:
+    if ops.cnet_fused_supported(hid, K1p, M):
         tc = time_graph(lambda i: ops.cnet_fwd_fused(cols[i], K1p, W1, W2, b1, b2, h2[i], M, hid), 16, nb)
     else:
         tc = float("nan")
