@@ -406,7 +406,11 @@ int nfk_adam_step(float* p, const float* g, float* m, float* v, long long n, con
  *                        pattern 0 or 2 -> [M, terms*Kp]
  *   nfk_act_split3       mode 0: relu(pre); mode 1: pre where gate > 0 (gate: bf16, row stride ldg); pattern 0 or 2
  *                        -> [M, terms*N], and colsum[n] += column sums of the fp32 result (bias gradients)
- *   nfk_coupling_bwd_f32 backward of the affine coupling (models/flows.py:160-168) with an fp32 pixel-major dh [M, C] */
+ *   nfk_coupling_bwd_f32 backward of the affine coupling (models/flows.py:160-168) with an fp32 pixel-major dh [M, C]
+ *   nfk_coupling_inv_bwd_f32  backward of the INVERSE coupling (models/flows.py:185-193), the fp32-dh form of
+ *                        nfk_coupling_inv_bwd: g_zc = dL/dzc, zc = the post-coupling tensor, hsave its (shift, logit)
+ *                        pairs, g_ld [B] -> dz (z1 half = g_zc1, z2 half = g_zc2 / s), dh [M, C] (shift, logit
+ *                        interleaved), dbias3 += column sums of dh (zeroed by the caller). C in {12, 24, 48, 96} */
 int nfk_split3_rows(const float* src, long long lds, long long rows, int K, int Ksrc, int pattern, void* out,
                     void* stream);
 int nfk_im2col3x3_split3(const float* src, int layout, int Ctot, int c0, int Cc, int B, int H, int W, int flip,
@@ -415,6 +419,8 @@ int nfk_act_split3(const float* pre, long long M, int N, int mode, const void* g
                    void* out, float* colsum, void* stream);
 int nfk_coupling_bwd_f32(const float* g_out, const float* g_ld, const float* z_out, const float* hsave, float* dy,
                          float* dh, float* dbias3, int B, int C, int H, int W, void* stream);
+int nfk_coupling_inv_bwd_f32(const float* g_zc, const float* g_ld, const float* zc, const float* hsave, float* dz,
+                             float* dh, float* dbias3, int B, int C, int H, int W, void* stream);
 
 #ifdef __cplusplus
 }

@@ -129,6 +129,7 @@ SIGNATURES: dict[str, list] = {
     "nfk_im2col3x3_split3": [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "nfk_act_split3": [_vp, _ll, _i, _i, _vp, _ll, _i, _vp, _vp, _vp],
     "nfk_coupling_bwd_f32": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "nfk_coupling_inv_bwd_f32": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
 }
 
 

@@ -131,6 +131,43 @@ __global__ void coupling_bwd_f32_kernel(const float* __restrict__ g_out, const f
   for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(dbias3 + i, sb[i]);
 }
 
+// Backward of the INVERSE affine coupling (models/flows.py:185-193: zc2 = z2 / s - shift, ld -= sum log s) in fp32, the
+// mirror of coupling_bwd_f32_kernel (arithmetic of coupling_bwd_kernel<C, INV = true> in zpath.cu); zc = the
+// post-coupling tensor, g_zc its gradient:
+//   dz1 = g1, dz2 = g2 / s, dh[m, 2j] = -g2 (shift), dh[m, 2j+1] = -(g2 * (zc2 + shift) + g_ld) * (1 - s) (logit),
+//   s = sigmoid(logit + 2), z2 / s = zc2 + shift; dbias3[c] += sum_m dh[m, c].
+__global__ void coupling_inv_bwd_f32_kernel(const float* __restrict__ g_zc, const float* __restrict__ g_ld,
+                                            const float* __restrict__ zc, const float* __restrict__ hsave,
+                                            float* __restrict__ dz, float* __restrict__ dh,
+                                            float* __restrict__ dbias3, int B, int C, int HW) {
+  extern __shared__ float sb[];   // [C]
+  const int J = C / 2;
+  for (int i = threadIdx.x; i < C; i += blockDim.x) sb[i] = 0.f;
+  __syncthreads();
+  const long long total = static_cast<long long>(B) * HW * J;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long m = i / J;               // pixel (channel pair fastest: hsave / dh rows are contiguous)
+    const int j = static_cast<int>(i - m * J);
+    const int b = static_cast<int>(m / HW), rem = static_cast<int>(m - static_cast<long long>(b) * HW);
+    const long long lo = (static_cast<long long>(b) * C + j) * HW + rem, hi = lo + static_cast<long long>(J) * HW;
+    const float2 h = *reinterpret_cast<const float2*>(hsave + m * C + 2 * j);
+    const float t = h.y + 2.f;
+    const float e = expf(-fabsf(t));
+    const float sg = t >= 0.f ? 1.f / (1.f + e) : e / (1.f + e);
+    const float g2 = g_zc[hi];
+    const float dsh = -g2;
+    const float dlg = -(g2 * (zc[hi] + h.x) + g_ld[b]) * (1.f - sg);
+    dz[lo] = g_zc[lo];
+    dz[hi] = g2 / sg;
+    *reinterpret_cast<float2*>(dh + m * C + 2 * j) = make_float2(dsh, dlg);
+    atomicAdd(&sb[2 * j], dsh);
+    atomicAdd(&sb[2 * j + 1], dlg);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < C; i += blockDim.x) atomicAdd(dbias3 + i, sb[i]);
+}
+
 }  // namespace nfk
 
 using namespace nfk;
@@ -180,5 +217,19 @@ extern "C" int nfk_coupling_bwd_f32(const float* g_out, const float* g_ld, const
   const unsigned grid = static_cast<unsigned>(want < 4 * 148 ? want : 4 * 148);
   coupling_bwd_f32_kernel<<<grid, S3T, C * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
       g_out, g_ld, z_out, hsave, dy, dh, dbias3, B, C, H * W);
+  return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
+}
+
+extern "C" int nfk_coupling_inv_bwd_f32(const float* g_zc, const float* g_ld, const float* zc, const float* hsave,
+                                        float* dz, float* dh, float* dbias3, int B, int C, int H, int W,
+                                        void* stream) {
+  // the channel counts of the z-path kernels that produce zc / hsave (nfk_coupling_fwd, nfk_affine1x1_fwd)
+  if (B <= 0 || H <= 0 || W <= 0 || (C != 12 && C != 24 && C != 48 && C != 96)) return NFK_ERR_SHAPE;
+  if (!g_zc || !g_ld || !zc || !hsave || !dz || !dh || !dbias3) return NFK_ERR_ARG;
+  const long long total = static_cast<long long>(B) * H * W * (C / 2);
+  const long long want = (total + S3T - 1) / S3T;
+  const unsigned grid = static_cast<unsigned>(want < 4 * 148 ? want : 4 * 148);
+  coupling_inv_bwd_f32_kernel<<<grid, S3T, C * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
+      g_zc, g_ld, zc, hsave, dz, dh, dbias3, B, C, H * W);
   return cudaGetLastError() == cudaSuccess ? NFK_OK : NFK_ERR_LAUNCH;
 }

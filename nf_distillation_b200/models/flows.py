@@ -242,21 +242,22 @@ class FlowStep(nn.Module):
         return z, (ld_out if want_ld else None)
 
     def _forward_precise(self, input, ld, want_ld, reverse, needs_grad):
-        """fp32-class mode (precise.py): split-bf16 products on the same tensor-core tiles."""
+        """fp32-class mode (precise.py): split-bf16 products on the same tensor-core tiles. Additive steps run the
+        affine arithmetic with the pinned logit rows of _coupling_params_2d, as in the bf16 mode."""
         from .. import precise
-        if self.flow_coupling != "affine":
-            raise NotImplementedError("bf16x3 precision is built for the affine coupling")
         with torch.set_grad_enabled(needs_grad):
-            fp = precise.folded_params(self)
             if not reverse:
-                z, ld_out = precise.FlowStep2dX3Fn.apply(input, ld, self.hidden_channels, *fp)
+                z, ld_out = precise.FlowStep2dX3Fn.apply(input, ld, self.hidden_channels, *precise.folded_params(self))
+            elif needs_grad:
+                # the perceptual term's gradient reaches the student through its inverse pass (pl_module.py:229-243);
+                # the inverse-direction affine and its chain rule come from the batched prep, as in the bf16 mode
+                pctx, idx, token = Fn.prep_for(self, True)
+                z, ld_out = precise.FlowStep2dReverseX3Fn.apply(input, ld, self.hidden_channels, token, pctx, idx,
+                                                                *precise.folded_coupling(self))
             else:
-                if needs_grad:
-                    raise NotImplementedError("gradients through the 2-D inverse pass are built for the bf16 "
-                                              "precision only")
                 k = self._consts(True)
                 z, ld_out = precise.flowstep2d_reverse_x3(input.contiguous(), ld.contiguous(), self.hidden_channels,
-                                                          (k.Wf, k.bf, k.sl), *fp[3:])
+                                                          (k.Wf, k.bf, k.sl), *precise.folded_coupling(self))
         return z, (ld_out if want_ld else None)
 
     def normal_flow(self, input, y_onehot, logdet):
