@@ -55,11 +55,22 @@ int nfk_gemm_set_prof(void* buf);
 int nfk_gemm_tn_bf16(const void* A, long long lda, const void* B, long long ldb, int Mo, int No, int Kpix,
                      float* out, long long ldo, int sm_count, void* stream);
 
-/* ---- batched parameter-space prep: every FlowStep of a model in one launch (one CTA per step) ----------------
- * An item is the argument list of nfk_invconv_prep below; a backward item adds the incoming gradients of the
- * fused matrix (dWf, row stride dWf_ld >= C; fwd.outW must hold the forward's outW) and the outputs.
+/* ---- parameter-space prep ("K0"): every FlowStep of a model in one launch -----------------------------------
  * Items are read on the host at launch time (they travel in the kernel parameter block), so the arrays may be
- * temporaries; the device pointers inside them must stay valid until the stream reaches the kernel. */
+ * temporaries; the device pointers inside them must stay valid until the stream reaches the kernel.
+ *
+ * nfk_invconv_prep_batch: one CTA per item builds the fused ActNorm o InvertibleConv1x1 matrix of one FlowStep
+ * (models/layers.py:376-397 get_weight + :101-142), C <= 104:
+ *   forward (reverse=0):  outW = W diag(exp(logs)), outb = outW * an_bias, W = P (L o tril + I)(U o triu + diag(s))
+ *   inverse (reverse=1):  outW = diag(exp(-logs)) W^-1 (triangular solves in shared memory), outb = -an_bias
+ *   out_sl[0] = +-(sum(an_logs) + sum(log_s))   (multiply by H*W for the per-sample log-det)
+ *   transpose=1 selects the 1-D convention z = x @ W (models/layers.py:410-411).
+ *   weight != NULL selects the non-LU branch (models/layers.py:366-375): in-kernel Gauss-Jordan slogdet/inverse;
+ *   lower, upper, log_s, p, sign_s are then unused.
+ * nfk_invconv_prep_bwd_batch: chain rule of that prep in either direction, (dWf, dbf, g_ld[B] or NULL) -> gradients
+ * of actnorm.{bias,logs} and invconv.{lower,upper,log_s} (or invconv.weight); the inverse direction goes through
+ * dW = -W^-T dW^-1 W^-T. dWf has row stride dWf_ld >= C, fwd.outW must hold the forward's outW, `pixels` = H*W (1 in
+ * 1-D) scales the log-det gradient. Outputs are overwritten. */
 typedef struct nfk_invconv_item {
   const float *an_bias, *an_logs, *lower, *upper, *log_s, *p, *sign_s, *weight;
   int C, reverse, transpose;
@@ -78,29 +89,12 @@ typedef struct nfk_invconv_bwd_item {
 int nfk_invconv_prep_batch(int n, const nfk_invconv_item* items, void* stream);
 int nfk_invconv_prep_bwd_batch(int n, const nfk_invconv_bwd_item* items, void* stream);
 
-/* ---- parameter-space prep ("K0") ---------------------------------------------------------------------------
- * Fused ActNorm o InvertibleConv1x1 matrix of one FlowStep (models/layers.py:376-397 get_weight + :101-142).
- *   forward (reverse=0):  outW = W diag(exp(logs)), outb = outW * an_bias, W = P (L o tril + I)(U o triu + diag(s))
- *   inverse (reverse=1):  outW = diag(exp(-logs)) W^-1 (triangular solves in shared memory), outb = -an_bias
- *   out_sl[0] = +-(sum(an_logs) + sum(log_s))   (multiply by H*W for the per-sample log-det)
- *   transpose=1 selects the 1-D convention z = x @ W (models/layers.py:410-411).
- *   weight != NULL selects the non-LU branch (models/layers.py:366-375): in-kernel Gauss-Jordan slogdet/inverse. */
-int nfk_invconv_prep(const float* an_bias, const float* an_logs, const float* lower, const float* upper,
-                     const float* log_s, const float* p, const float* sign_s, const float* weight, int C, int reverse,
-                     int transpose, float* outW, float* outb, float* out_sl, void* stream);
-
-/* Chain rule of the prep in either direction: (dWf, dbf, g_ld[B] or NULL) -> gradients of actnorm.{bias,logs}
- * and invconv.{lower,upper,log_s} (or invconv.weight); the inverse direction goes through
- * dW = -W^-T dW^-1 W^-T. `pixels` = H*W (1 in 1-D). Outputs are overwritten. */
-int nfk_invconv_prep_bwd(const float* an_bias, const float* an_logs, const float* lower, const float* upper,
-                         const float* log_s, const float* p, const float* sign_s, const float* weight, int C,
-                         int reverse, int transpose, const float* Wf, const float* dWf, const float* dbf,
-                         const float* g_ld, int B,
-                         float pixels, float* d_bias, float* d_logs, float* d_lower, float* d_upper, float* d_log_s,
-                         float* d_weight, void* stream);
-
-/* Batched forms of nfk_coupling_prep / nfk_coupling_prep_bwd below (one grid row of CTAs per FlowStep): an item is
- * that call's argument list. Same lifetime rules as nfk_invconv_item. */
+/* nfk_coupling_prep_batch: one grid row of CTAs per item turns the coupling-network weights of one FlowStep into bf16
+ * GEMM operands with the ActNorm affine (models/layers.py:223-228) and the Conv2dZeros exp(3*logs) scale (:257-260)
+ * folded in. K1p / K3p = 9*cin / 9*cout rounded up to 64.
+ *   B1 [hid,K1p] (k = tap*cin+ci), B2 [hid,hid], B3 [K3p,hid] (row = tap*cout+co), bias1..3 the folded biases;
+ *   with_transposed = 1 also writes B1T, B2T, B3T (the transposes the dgrads read).
+ * nfk_coupling_prep_bwd_batch maps the gradients of those operands back to the reference parameters. */
 typedef struct nfk_coupling_item {
   const float *w1, *b1, *l1, *w2, *b2, *l2, *w3, *b3, *l3;
   int cin, hid, cout, K1p, K3p, with_transposed;
@@ -114,21 +108,6 @@ typedef struct nfk_coupling_bwd_item {
 } nfk_coupling_bwd_item;
 int nfk_coupling_prep_batch(int n, const nfk_coupling_item* items, void* stream);
 int nfk_coupling_prep_bwd_batch(int n, const nfk_coupling_bwd_item* items, void* stream);
-
-/* Coupling-network weights -> bf16 GEMM operands with the ActNorm affine (models/layers.py:223-228) and the
- * Conv2dZeros exp(3*logs) scale (:257-260) folded in. K1p / K3p = 9*cin / 9*cout rounded up to 64.
- *   B1 [hid,K1p] (k = tap*cin+ci), B2 [hid,hid], B3 [K3p,hid] (row = tap*cout+co); *T = transposes for dgrads. */
-int nfk_coupling_prep(const float* w1, const float* b1, const float* l1, const float* w2, const float* b2,
-                      const float* l2, const float* w3, const float* b3, const float* l3, int cin, int hid, int cout,
-                      int K1p, int K3p, void* B1, void* B1T, void* B2, void* B2T, void* B3, void* B3T, float* bias1,
-                      float* bias2, float* bias3, int with_transposed, void* stream);
-
-int nfk_coupling_prep_bwd(const float* w1, const float* b1, const float* l1, const float* w2, const float* b2,
-                          const float* l2, const float* w3, const float* b3, const float* l3, int cin, int hid,
-                          int cout, int K1p, int K3p, const float* dB1, const float* dbias1, const float* dB2,
-                          const float* dbias2, const float* dB3, const float* dbias3, float* dw1, float* db1,
-                          float* dl1, float* dw2, float* db2, float* dl2, float* dw3, float* db3, float* dl3,
-                          void* stream);
 
 /* ---- fp32 z path of a 2-D FlowStep (models/flows.py:142-202) ------------------------------------------------
  * y = Wf x + bf per pixel (ActNorm + invconv, models/layers.py:129-142,404-421); ld_out = ld_in + H*W*sl[0];
@@ -196,7 +175,7 @@ int nfk_kd_mse_bwd(const float* s, const float* t, const float* g, int B, int n,
  * models/flows.py:150-171 / :173-190): P^T = B3 * h2^T on tcgen05 with whole images as the N tile, col2im over the nine
  * taps, bias, then z2 <- (z2 + shift) * sigmoid(logit + 2) (reverse: z2 / sigmoid - shift) in place on y's upper C/2
  * channels, ld[b] += (-)sum log sigmoid. h2 [B*H*W, hid] bf16, B3 [K3p, hid] bf16 (rows tap*C + c, as built by
- * nfk_coupling_prep), hsave (optional, [B*H*W, C] fp32) keeps the conv output for nfk_coupling_bwd.
+ * nfk_coupling_prep_batch), hsave (optional, [B*H*W, C] fp32) keeps the conv output for nfk_coupling_bwd.
  * Supported shapes (nfk_pconv_coupling_supported): C = 12 with maps of 256 pixels (W <= 16) or <= 128 pixels, C = 24
  * with <= 64 pixels, C = 48 with <= 32 pixels; H, W powers of two; hid % 64 == 0. */
 int nfk_pconv_coupling_supported(int C, int H, int W, int hid);
@@ -207,8 +186,8 @@ int nfk_pconv_coupling_fwd(const void* h2, const void* B3, int K3p, const float*
  * (csrc/dgrad_col2im.cu): P^T = B1T * dpre1^T on tcgen05 with whole images as the N tile, then per pixel
  * dys = dy + col2im(P) on the y1 half (dy on the y2 half), dx = W'^T dys, dWf += dys x^T, dbf += sum dys.
  * dpre1 [B*H*W, hid] bf16 (the masked gradient at the first conv's output), B1T [K1p, hid] bf16 (rows tap*(C/2) + ci,
- * as built by nfk_coupling_prep), K1p = round_up(9*C/2, 64); dy, x, dx [B,C,H,W] fp32, Wf [C,C]; dWf, dbf are
- * accumulated (zeroed by the caller). dx is bit-identical to nfk_gemm_nt_bf16 (NFK_EPI_F32) + nfk_affine1x1_bwd.
+ * as built by nfk_coupling_prep_batch), K1p = round_up(9*C/2, 64); dy, x, dx [B,C,H,W] fp32, Wf [C,C]; dWf, dbf
+ * are accumulated (zeroed by the caller). dx is bit-identical to nfk_gemm_nt_bf16 (NFK_EPI_F32) + nfk_affine1x1_bwd.
  * Supported shapes (nfk_conv1_dgrad_affine_bwd_supported): C = 12 with maps of <= 256 pixels, C = 24 with <= 128,
  * C = 48 with <= 64; H, W powers of two; hid % 64 == 0. */
 int nfk_conv1_dgrad_affine_bwd_supported(int C, int H, int W, int hid);
@@ -217,8 +196,8 @@ int nfk_conv1_dgrad_affine_bwd(const void* dpre1, const void* B1T, int K1p, cons
                                void* stream);
 
 /* ---- 1-D (tabular) FlowStep, fused (is_1d branches of models/flows.py:37-52,142-202, models/layers.py:410-411) --
- * Weights are packed once per optimiser step by nfk_flow1d_pack from the fused affine (nfk_invconv_prep with
- * transpose=1, forward or inverse direction) and the six nn.Linear layers of get_block_1d:
+ * Weights are packed once per optimiser step by nfk_flow1d_pack from the fused affine (nfk_invconv_prep_batch
+ * with transpose=1, forward or inverse direction) and the six nn.Linear layers of get_block_1d:
  *   PF: per layer WT [nin][nout8] + bias [nout8] (forward), PB: per layer W [nout][nin8] (backward).
  * nfk_flow1d_sizes reports the block sizes and the per-layer offsets of the gradient block G
  * (dW_l [nout][nin8] at offG, db_l at offGB). x / y / dx are [B, D] row-major, cond is [B, Cc] (y_onehot). */
@@ -326,8 +305,8 @@ int nfk_made_inverse_bwd_resident(const float* g_x, const float* g_ld, const flo
 
 /* Fused conv#1 -> conv#2 of the coupling network: h2 = relu(relu(col*B1^T + b1)*B2^T + b2) in ONE kernel (CTA
  * pairs; h1 stays in tensor memory as the tcgen05 A operand of conv#2; csrc/cnet_ts.cu). col [M,K1p] bf16, B1 [512,K1p],
- * B2 [512,512] bf16 (nfk_coupling_prep), h2 [M,512] bf16. Training additionally passes h1 [M,512] and the two 1-bit
- * ReLU mask buffers (word-major, [16][ldmask >= M]); inference passes NULL for them.
+ * B2 [512,512] bf16 (nfk_coupling_prep_batch), h2 [M,512] bf16. Training additionally passes h1 [M,512] and the two
+ * 1-bit ReLU mask buffers (word-major, [16][ldmask >= M]); inference passes NULL for them.
  * nfk_cnet_fused_supported: 1 if the kernels take hidden width hid and first-GEMM depth K (K1p / K3p): hid = 512 and
  * K a multiple of 64 up to 448 (the GEMM-1 A tile must leave shared memory for a weight ring of two slots). The entry
  * points return NFK_ERR_SHAPE otherwise; callers run the two nfk_gemm_nt_bf16 GEMMs instead. */
@@ -340,9 +319,9 @@ int nfk_cnet_fwd_fused(const void* col, int K1p, const void* B1, const void* B2,
  * the Conv2dZeros input gradient through the ReLU mask of h2 — stays in tensor memory as the A operand of
  * d1 = relu'(h1) .* (d2 B2T^T); both are written out as bf16 [M, 512] (the weight-gradient GEMMs read them) and their
  * column sums are added into dbias2 / dbias1 (fp32 [512], caller-zeroed; NULL = not needed). dhcol [M, K3p] bf16
- * (nfk_coupling_bwd), B3T [512, K3p], B2T [512, 512] bf16 (nfk_coupling_prep, transposed operands), masks as written by
- * nfk_cnet_fwd_fused / nfk_gemm_nt_bf16 (word-major, [16][ldmask >= M]). Replaces two nfk_gemm_nt_bf16 calls with
- * NFK_EPI_MASK_BF16 (autograd of models/flows.py:25-34). Shapes: nfk_cnet_fused_supported(hid, K3p). */
+ * (nfk_coupling_bwd), B3T [512, K3p], B2T [512, 512] bf16 (nfk_coupling_prep_batch, transposed operands), masks as
+ * written by nfk_cnet_fwd_fused / nfk_gemm_nt_bf16 (word-major, [16][ldmask >= M]). Replaces two nfk_gemm_nt_bf16
+ * calls with NFK_EPI_MASK_BF16 (autograd of models/flows.py:25-34). Shapes: nfk_cnet_fused_supported(hid, K3p). */
 int nfk_cnet_bwd_fused(const void* dhcol, int K3p, const void* B3T, const void* B2T, const void* mask_h2,
                        const void* mask_h1, long long ldmask, void* dpre2, void* dpre1, float* dbias2, float* dbias1,
                        int M, int hid, void* stream);

@@ -65,12 +65,8 @@ SIGNATURES: dict[str, list] = {
     "nfk_gemm_tn_bf16": [_vp, _ll, _vp, _ll, _i, _i, _i, _vp, _ll, _i, _vp],
     "nfk_invconv_prep_batch": [_i, _vp, _vp],
     "nfk_invconv_prep_bwd_batch": [_i, _vp, _vp],
-    "nfk_invconv_prep": [_vp] * 8 + [_i, _i, _i, _vp, _vp, _vp, _vp],
-    "nfk_invconv_prep_bwd": [_vp] * 8 + [_i, _i, _i, _vp, _vp, _vp, _vp, _i, _f] + [_vp] * 6 + [_vp],
     "nfk_coupling_prep_batch": [_i, _vp, _vp],
     "nfk_coupling_prep_bwd_batch": [_i, _vp, _vp],
-    "nfk_coupling_prep": [_vp] * 9 + [_i] * 5 + [_vp] * 9 + [_i, _vp],
-    "nfk_coupling_prep_bwd": [_vp] * 9 + [_i] * 5 + [_vp] * 6 + [_vp] * 9 + [_vp],
     "nfk_affine1x1_fwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _i, _i, _i, _vp],
     "nfk_coupling_fwd": [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "nfk_coupling_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp],

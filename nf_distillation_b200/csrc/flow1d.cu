@@ -4,7 +4,7 @@
 // A persistent CTA (one per SM) walks tiles of NT samples with every weight of the step resident in shared memory.
 // Activations live in shared memory feature-major ([feature][NT+4]); each layer is a small fp32 GEMM over the tile,
 // register-blocked 8 outputs x 4 samples per thread (3 LDS.128 per 32 FMAs):
-//   y = W' x + b'            (ActNorm1d + x @ W folded by nfk_invconv_prep with transpose=1)
+//   y = W' x + b'            (ActNorm1d + x @ W folded by nfk_invconv_prep_batch with transpose=1)
 //   h = MLP(y1 [, cond])     Linear-ReLU x4, Linear-Tanh, Linear
 //   y2 = (y2 + h[0::2]) * sigmoid(h[1::2] + 2),  logdet += sum log sigmoid          (or the inverse order / formulas)
 // The backward kernel reloads the saved MLP activations, walks the chain in reverse with the same tile GEMM for the

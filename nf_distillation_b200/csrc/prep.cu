@@ -1,14 +1,15 @@
 // Parameter-space kernels ("K0"): everything that depends only on the weights, once per optimiser step.
 //
-//  * invconv_prep: builds the fused ActNorm o InvertibleConv1x1 matrix of one FlowStep from the LU
+//  * invconv_prep_kernel: builds the fused ActNorm o InvertibleConv1x1 matrix of a FlowStep from the LU
 //    parametrisation (reference: models/layers.py:376-397 get_weight, :101-142 ActNorm) — forward
 //    W' = P L U diag(e^logs), b' = W' b, and inverse diag(e^-logs) U^-1 L^-1 P^T via in-SM triangular solves
 //    (replaces three torch.inverse calls) — plus log|det| = sum(logs) + sum(log_s). The non-LU branch
 //    (:366-375) runs a Gauss-Jordan slogdet/inverse in shared memory.
-//  * invconv_prep_bwd: chain rule from (dW', db') back to actnorm.{bias,logs}, invconv.{lower,upper,log_s}.
-//  * coupling_prep: folds the ActNorm affine of Conv2d (models/layers.py:223-228) and the exp(3*logs) output
-//    scale of Conv2dZeros (:257-260) into bf16 GEMM operands laid out for the tcgen05 tiles; coupling_prep_bwd
-//    maps GEMM-operand gradients back to the reference parameters.
+//  * invconv_prep_bwd_kernel: chain rule from (dW', db') back to actnorm.{bias,logs}, invconv.{lower,upper,log_s}.
+//  * coupling_prep_kernel: folds the ActNorm affine of Conv2d (models/layers.py:223-228) and the exp(3*logs)
+//    output scale of Conv2dZeros (:257-260) into bf16 GEMM operands laid out for the tcgen05 tiles;
+//    coupling_prep_bwd_kernel maps GEMM-operand gradients back to the reference parameters.
+// Each kernel takes a batch of items (one CTA, or one grid row of CTAs, per FlowStep): include/nfk.h.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cstdint>
@@ -566,32 +567,6 @@ extern "C" int nfk_invconv_prep_bwd_batch(int n, const nfk_invconv_bwd_item* ite
   return NFK_OK;
 }
 
-extern "C" int nfk_invconv_prep(const float* an_bias, const float* an_logs, const float* lower, const float* upper,
-                                const float* log_s, const float* p, const float* sign_s, const float* weight,
-                                int C, int reverse, int transpose, float* outW, float* outb, float* out_sl,
-                                void* stream) {
-  const nfk_invconv_item q{an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose,
-                           outW, outb, out_sl};
-  return nfk_invconv_prep_batch(1, &q, stream);
-}
-
-extern "C" int nfk_invconv_prep_bwd(const float* an_bias, const float* an_logs, const float* lower,
-                                    const float* upper, const float* log_s, const float* p, const float* sign_s,
-                                    const float* weight, int C, int reverse, int transpose, const float* Wf,
-                                    const float* dWf, const float* dbf, const float* g_ld, int B, float pixels,
-                                    float* d_bias,
-                                    float* d_logs, float* d_lower, float* d_upper, float* d_log_s, float* d_weight,
-                                    void* stream) {
-  if (!Wf) return NFK_ERR_ARG;
-  nfk_invconv_bwd_item g{};
-  g.fwd = nfk_invconv_item{an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose,
-                           const_cast<float*>(Wf), const_cast<float*>(Wf), const_cast<float*>(Wf)};
-  g.dWf = dWf; g.dWf_ld = C; g.dbf = dbf; g.g_ld = g_ld; g.B = B; g.pixels = pixels;
-  g.d_bias = d_bias; g.d_logs = d_logs; g.d_lower = d_lower; g.d_upper = d_upper; g.d_log_s = d_log_s;
-  g.d_weight = d_weight;
-  return nfk_invconv_prep_bwd_batch(1, &g, stream);
-}
-
 static int coupling_item_check(const nfk_coupling_item& c) {
   if (c.cin <= 0 || c.hid <= 0 || c.cout <= 0 || c.hid % 64 || c.K1p % 64 || c.K3p % 64 || c.K1p < 9 * c.cin ||
       c.K3p < 9 * c.cout)
@@ -660,28 +635,4 @@ extern "C" int nfk_coupling_prep_bwd_batch(int n, const nfk_coupling_bwd_item* i
     if (cudaGetLastError() != cudaSuccess) return NFK_ERR_LAUNCH;
   }
   return NFK_OK;
-}
-
-extern "C" int nfk_coupling_prep(const float* w1, const float* b1, const float* l1, const float* w2, const float* b2,
-                                 const float* l2, const float* w3, const float* b3, const float* l3, int cin, int hid,
-                                 int cout, int K1p, int K3p, void* B1, void* B1T, void* B2, void* B2T, void* B3,
-                                 void* B3T, float* bias1, float* bias2, float* bias3, int with_transposed,
-                                 void* stream) {
-  const nfk_coupling_item c{w1, b1, l1, w2, b2, l2, w3, b3, l3, cin, hid, cout, K1p, K3p, with_transposed,
-                            B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3};
-  return nfk_coupling_prep_batch(1, &c, stream);
-}
-
-extern "C" int nfk_coupling_prep_bwd(const float* w1, const float* b1, const float* l1, const float* w2,
-                                     const float* b2, const float* l2, const float* w3, const float* b3,
-                                     const float* l3, int cin, int hid, int cout, int K1p, int K3p, const float* dB1,
-                                     const float* dbias1, const float* dB2, const float* dbias2, const float* dB3,
-                                     const float* dbias3, float* dw1, float* db1, float* dl1, float* dw2, float* db2,
-                                     float* dl2, float* dw3, float* db3, float* dl3, void* stream) {
-  nfk_coupling_bwd_item g{};
-  g.fwd = nfk_coupling_item{w1, b1, l1, w2, b2, l2, w3, b3, l3, cin, hid, cout, K1p, K3p, 0,
-                            nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  g.dB1 = dB1; g.dbias1 = dbias1; g.dB2 = dB2; g.dbias2 = dbias2; g.dB3 = dB3; g.dbias3 = dbias3;
-  g.dw1 = dw1; g.db1 = db1; g.dl1 = dl1; g.dw2 = dw2; g.db2 = db2; g.dl2 = dl2; g.dw3 = dw3; g.db3 = db3; g.dl3 = dl3;
-  return nfk_coupling_prep_bwd_batch(1, &g, stream);
 }

@@ -26,7 +26,7 @@ def _mlp_params(step):
 
 
 def _pack(step, reverse, with_bwd, affine, ws, bs):
-    """affine = (Wf, bf, sl) of this direction (nfk_invconv_prep with transpose=1)."""
+    """affine = (Wf, bf, sl) of this direction (functional.affine_item with transpose=1)."""
     D, Cc, hid = step.in_channels, step.condition_features, step.hidden_channels
     Wf, bf, sl = affine
     tf, tb, tg, n_act, offs = ops.flow1d_sizes(D, Cc, hid)
@@ -39,17 +39,13 @@ def _pack(step, reverse, with_bwd, affine, ws, bs):
 
 def _consts(step, reverse):
     """No-grad path: packed weights cached until a parameter changes (frozen teacher, sampling)."""
-    key = (reverse, Fn.param_key(step._all_params()))
-    hit = step._cache.get(("1d", reverse))
-    if hit is not None and hit[0] == key:
-        return hit[1]
-    ws, bs = _mlp_params(step)
-    inv = tuple(None if t is None else t.detach() for t in step.invconv.lu_tensors())
-    affine = Fn.build_affine(step.actnorm.bias.detach(), step.actnorm.logs.detach(), inv, step.in_channels, reverse,
-                             True)
-    out = _pack(step, reverse, False, affine, [w.detach() for w in ws], [b.detach() for b in bs])
-    step._cache[("1d", reverse)] = (key, out)
-    return out
+    def build():
+        ws, bs = _mlp_params(step)
+        inv = tuple(None if t is None else t.detach() for t in step.invconv.lu_tensors())
+        affine = Fn.build_affine(step.actnorm.bias.detach(), step.actnorm.logs.detach(), inv, step.in_channels,
+                                 reverse, True)
+        return _pack(step, reverse, False, affine, [w.detach() for w in ws], [b.detach() for b in bs])
+    return Fn.cached(step, ("1d", reverse), build)
 
 
 class FlowStep1dFn(torch.autograd.Function):
@@ -106,27 +102,23 @@ class FlowStep1dFn(torch.autograd.Function):
 def _wide_consts(step, reverse):
     """Frozen wide step (hidden width a multiple of 64 that does not fit the fused kernel, e.g. conf/teacher/rich.yaml:
     256): fused affine of this direction + the six Linear layers as zero-padded bf16 GEMM operands. Cached."""
-    key = (reverse, Fn.param_key(step._all_params()))
-    hit = step._cache.get(("1dw", reverse))
-    if hit is not None and hit[0] == key:
-        return hit[1]
-    D = step.in_channels
-    inv = tuple(None if t is None else t.detach() for t in step.invconv.lu_tensors())
-    Wf, bf, sl = Fn.build_affine(step.actnorm.bias.detach(), step.actnorm.logs.detach(), inv, D, reverse, True)
-    ws, bs = _mlp_params(step)
-    Wb, bb = [], []
-    for w, b in zip(ws, bs):
-        nout, nin = w.shape
-        n_p, k_p = ops.round_up(nout, 16), ops.round_up(nin, 64)
-        wp = torch.zeros(n_p, k_p, device=w.device, dtype=torch.bfloat16)
-        wp[:nout, :nin] = w.detach()
-        bp = torch.zeros(n_p, device=w.device, dtype=F32)
-        bp[:nout] = b.detach()
-        Wb.append(wp)
-        bb.append(bp)
-    out = (Wf, bf, sl, Wb, bb)
-    step._cache[("1dw", reverse)] = (key, out)
-    return out
+    def build():
+        D = step.in_channels
+        inv = tuple(None if t is None else t.detach() for t in step.invconv.lu_tensors())
+        Wf, bf, sl = Fn.build_affine(step.actnorm.bias.detach(), step.actnorm.logs.detach(), inv, D, reverse, True)
+        ws, bs = _mlp_params(step)
+        Wb, bb = [], []
+        for w, b in zip(ws, bs):
+            nout, nin = w.shape
+            n_p, k_p = ops.round_up(nout, 16), ops.round_up(nin, 64)
+            wp = torch.zeros(n_p, k_p, device=w.device, dtype=torch.bfloat16)
+            wp[:nout, :nin] = w.detach()
+            bp = torch.zeros(n_p, device=w.device, dtype=F32)
+            bp[:nout] = b.detach()
+            Wb.append(wp)
+            bb.append(bp)
+        return Wf, bf, sl, Wb, bb
+    return Fn.cached(step, ("1dw", reverse), build)
 
 
 def _flowstep1d_wide(step, x, cond, ld, reverse):

@@ -65,6 +65,15 @@ def param_key(params) -> tuple:
     return (epoch, tuple((p.data_ptr(), p._version) for p in params))
 
 
+def cached(step, slot, build):
+    """step._cache[slot] for the no-grad paths: build() again whenever a parameter of the step changed."""
+    key = param_key(step._all_params())
+    hit = step._cache.get(slot)
+    if hit is None or hit[0] != key:
+        hit = step._cache[slot] = (key, build())
+    return hit[1]
+
+
 # ------------------------------------------------------------------------------------------------ derived weights
 @dataclass
 class StepConsts:
@@ -83,15 +92,37 @@ class StepConsts:
     bias3: torch.Tensor = None
 
 
+def affine_item(an_bias, an_logs, inv, C, reverse, transpose, Wf, bf, sl):
+    """The nfk_invconv_item that writes one step's fused ActNorm o invconv affine of direction `reverse` into Wf [C,C],
+    bf [C], sl [1] (transpose: the 1-D convention). inv = (lower, upper, log_s, p, sign_s, weight) with unused
+    entries None, as InvertibleConv1x1.lu_tensors() gives it."""
+    lower, upper, log_s, p, sign_s, weight = inv
+    return ops.invconv_item(an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose, Wf, bf, sl)
+
+
 def build_affine(an_bias, an_logs, inv, C, reverse, transpose):
-    """inv = (lower, upper, log_s, p, sign_s, weight) with unused entries None."""
+    """(Wf, bf, sl) of one step or stand-alone layer, built by its own launch (see affine_item)."""
     dev = an_bias.device
     Wf = torch.empty(C, C, device=dev, dtype=F32)
     bf = torch.empty(C, device=dev, dtype=F32)
     sl = torch.empty(1, device=dev, dtype=F32)
-    lower, upper, log_s, p, sign_s, weight = inv
-    ops.invconv_prep(an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose, Wf, bf, sl)
+    ops.invconv_prep_batch([affine_item(an_bias, an_logs, inv, C, reverse, transpose, Wf, bf, sl)])
     return Wf, bf, sl
+
+
+def coupling_operands(cw, C, hid, with_t):
+    """The coupling-net GEMM operands of a 2-D step with C channels and their nfk_coupling_item: B1 [hid, K1p],
+    B2 [hid, hid], B3 [K3p, hid] bf16 with K1p, K3p = 9*C/2, 9*C rounded up to 64, their transposes B1T, B2T, B3T
+    when with_t (the backward's dgrads read them, else None) and the folded biases, all three in one buffer.
+    cw = FlowStep._coupling_params_2d(). Returns (item, (B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3))."""
+    dev = cw[0].device
+    K1p, K3p = ops.round_up(9 * (C // 2), 64), ops.round_up(9 * C, 64)
+    e = lambda *s: torch.empty(*s, device=dev, dtype=BF16)
+    B1, B2, B3 = e(hid, K1p), e(hid, hid), e(K3p, hid)
+    B1T, B2T, B3T = (e(K1p, hid), e(hid, hid), e(hid, K3p)) if with_t else (None, None, None)
+    bias = torch.empty(2 * hid + ops.round_up(C, 4), device=dev, dtype=F32)
+    cops = (B1, B1T, B2, B2T, B3, B3T, bias[:hid], bias[hid:2 * hid], bias[2 * hid:2 * hid + C])
+    return ops.coupling_item(cw, C // 2, hid, C, K1p, K3p, with_t, *cops), cops
 
 
 # ------------------------------------------------------------------------------------ batched affine build (K0)
@@ -120,6 +151,7 @@ class PrepCtx:
     def build(self):
         flat = []
         for st in self.steps:
+            st._sync_permutation()
             iv = st.invconv
             if iv.LU_decomposed:
                 flat += [st.actnorm.bias, st.actnorm.logs, iv.lower, iv.upper, iv.log_s]
@@ -172,10 +204,10 @@ def prep_for(step, reverse):
 def prepare_steps(layers, reverse):
     """Batch every trainable FlowStep in `layers` (called by FlowNet.encode/decode under grad); reverse=True builds the
     inverse-direction matrices, and PrepAllFn.backward then applies the inverse's chain rule."""
+    from .models.flows import FlowStep
     if not torch.is_grad_enabled():
         return None
-    steps = [l for l in layers if getattr(l, "_batched_prep_ok", None) is not None and l._batched_prep_ok()
-             and l.actnorm.logs.requires_grad]
+    steps = [l for l in layers if isinstance(l, FlowStep) and l.actnorm.logs.requires_grad]
     if len(steps) < 2:
         return None
     return PrepCtx(steps, reverse).build()
@@ -195,37 +227,21 @@ class PrepAllFn(torch.autograd.Function):
             Wf = buf[off:off + C * C].view(C, C); off += ops.round_up(C * C, 4)
             bf = buf[off:off + C]; off += ops.round_up(C, 4)
             sl = buf[off:off + 1]; off += 4
-            an_bias, an_logs, lower, upper, log_s = flat[5 * i:5 * i + 5]
-            if st.invconv.LU_decomposed:
-                it = ops.invconv_item(an_bias, an_logs, lower, upper, log_s, st.invconv.p, st.invconv.sign_s, None, C,
-                                      pctx.reverse, st.is_1d, Wf, bf, sl)
-            else:
-                it = ops.invconv_item(an_bias, an_logs, None, None, None, None, None, lower, C, pctx.reverse,
-                                      st.is_1d, Wf, bf, sl)
+            # (the invconv tensors of lu_tensors() are the ones PrepCtx.build put in this step's slots of `flat`)
+            it = affine_item(flat[5 * i], flat[5 * i + 1], st.invconv.lu_tensors(), C, pctx.reverse, st.is_1d,
+                             Wf, bf, sl)
             items.append(it)
             pctx.consts[i] = (Wf, bf, sl)
             pctx.items[i] = it
         ops.invconv_prep_batch(items)
         # coupling-net GEMM operands of the 2-D steps, one launch
         off = 5 * len(pctx.steps)
-        citems = []
         for i, st in enumerate(pctx.steps):
-            if st.is_1d:
-                continue
-            cw = flat[off:off + 9]; off += 9
-            C, hid = st.in_channels, st.hidden_channels
-            cin, cout = C // 2, C
-            K1p, K3p = ops.round_up(9 * cin, 64), ops.round_up(9 * cout, 64)
-            e = lambda *s_: torch.empty(*s_, device=dev, dtype=BF16)
-            B1, B2, B3 = e(hid, K1p), e(hid, hid), e(K3p, hid)
-            B1T, B2T, B3T = e(K1p, hid), e(hid, hid), e(hid, K3p)
-            bias = torch.empty(2 * hid + ops.round_up(cout, 4), device=dev, dtype=F32)
-            bias1, bias2, bias3 = bias[:hid], bias[hid:2 * hid], bias[2 * hid:2 * hid + cout]
-            it = ops.coupling_item(cw, cin, hid, cout, K1p, K3p, True, B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3)
-            citems.append(it)
-            pctx.citems[i] = it
-            pctx.cops[i] = (B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3)
-        ops.coupling_prep_batch(citems)
+            if not st.is_1d:
+                pctx.citems[i], pctx.cops[i] = coupling_operands(flat[off:off + 9], st.in_channels,
+                                                                 st.hidden_channels, True)
+                off += 9
+        ops.coupling_prep_batch([it for it in pctx.citems if it is not None])
         ctx.pctx = pctx
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(*flat)
@@ -285,20 +301,6 @@ class PrepAllFn(torch.autograd.Function):
         ops.coupling_prep_bwd_batch(citems)
         pctx.cgrads = [None] * n
         return (None, *out, *cout_grads)
-
-
-def build_coupling_ops(cw, cin, hid, cout, with_t):
-    """cw = (w1, b1, l1, w2, b2, l2, w3, b3, l3) reference parameters of get_block_2d."""
-    dev = cw[0].device
-    K1p, K3p = ops.round_up(9 * cin, 64), ops.round_up(9 * cout, 64)
-    e = lambda *s: torch.empty(*s, device=dev, dtype=BF16)
-    B1, B2, B3 = e(hid, K1p), e(hid, hid), e(K3p, hid)
-    B1T, B2T, B3T = (e(K1p, hid), e(hid, hid), e(hid, K3p)) if with_t else (None, None, None)
-    bias1 = torch.empty(hid, device=dev, dtype=F32)
-    bias2 = torch.empty(hid, device=dev, dtype=F32)
-    bias3 = torch.empty(cout, device=dev, dtype=F32)
-    ops.coupling_prep(*cw, cin, hid, cout, K1p, K3p, B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3, with_t)
-    return B1, B1T, B2, B2T, B3, B3T, bias1, bias2, bias3
 
 
 def _coupling_net(col, k: StepConsts, M, hid, K1p, K3p, keep):

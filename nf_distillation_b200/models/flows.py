@@ -12,6 +12,7 @@ import torch
 import torch.nn as nn
 
 from .. import functional as Fn
+from .. import ops
 from .layers import (ActNorm1d, ActNorm2d, Conv2d, Conv2dZeros, InvertibleConv1x1, LinearZeros, Permute2d, Split2d,
                      SqueezeLayer, _as_logdet, _require_cuda, gaussian_likelihood, gaussian_sample)
 from .utils import (can_fuse_dequant_squeeze, dequantize_and_squeeze, split_feature,
@@ -143,27 +144,17 @@ class FlowStep(nn.Module):
 
     def _consts(self, reverse: bool) -> Fn.StepConsts:
         """Derived tensors for the no-grad path (frozen teacher, sampling): rebuilt only when a parameter changed."""
-        key = (reverse, Fn.param_key(self._all_params()))
-        hit = self._cache.get(reverse)
-        if hit is not None and hit[0] == key:
-            return hit[1]
-        C = self.in_channels
-        inv = tuple(None if t is None else t.detach() for t in self.invconv.lu_tensors())
-        Wf, bf, sl = Fn.build_affine(self.actnorm.bias.detach(), self.actnorm.logs.detach(), inv, C, reverse,
-                                     self.is_1d)
-        if self.is_1d:
-            k = Fn.StepConsts(Wf, bf, sl)
-        else:
+        def build():
+            inv = tuple(None if t is None else t.detach() for t in self.invconv.lu_tensors())
+            Wf, bf, sl = Fn.build_affine(self.actnorm.bias.detach(), self.actnorm.logs.detach(), inv,
+                                         self.in_channels, reverse, self.is_1d)
+            if self.is_1d:
+                return Fn.StepConsts(Wf, bf, sl)
             cw = tuple(t.detach() for t in self._coupling_params_2d())
-            k = Fn.StepConsts(Wf, bf, sl, *Fn.build_coupling_ops(cw, C // 2, self.hidden_channels, C, False))
-        self._cache[reverse] = (key, k)
-        return k
-
-    def _batched_prep_ok(self):
-        """True when this step's fused affine can be built by the batched K0 launch (functional.PrepCtx): LU-parametrised
-        steps, fixed permutations (an LU with frozen factors) and plain-weight steps (LU_decomposed=False) alike."""
-        self._sync_permutation()
-        return True
+            item, cops = Fn.coupling_operands(cw, self.in_channels, self.hidden_channels, False)
+            ops.coupling_prep_batch([item])
+            return Fn.StepConsts(Wf, bf, sl, *cops)
+        return Fn.cached(self, reverse, build)
 
     def _check_actnorm_inited(self, input):
         """Reference layers.py:129-133: an ActNorm that was never initialised runs its data-dependent init on the first
@@ -189,7 +180,6 @@ class FlowStep(nn.Module):
             raise NotImplementedError("additive coupling is built for the 2-D steps only (every 1-D config is affine)")
         self._sync_permutation()
         if self.is_1d:
-            from .. import ops
             training = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
             wide_ok = not training and self.hidden_channels % 64 == 0      # GEMM path of flow1d._flowstep1d_wide
             if not wide_ok and not ops.flow1d_supported(self.in_channels, self.condition_features,
@@ -206,8 +196,6 @@ class FlowStep(nn.Module):
             if self.hidden_channels % 64 or self.in_channels not in (12, 24, 48, 96):
                 raise NotImplementedError("2-D FlowStep kernels need hidden_channels % 64 == 0 and "
                                           "C in {12, 24, 48, 96}")
-            if not self.invconv.LU_decomposed and torch.is_grad_enabled():
-                pass
 
     def forward(self, input, y_onehot=None, logdet=None, reverse=False):
         self._check_supported(input)

@@ -73,25 +73,8 @@ def sm_count() -> int:
     return _SM[d]
 
 
-def invconv_prep(an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose, outW, outb, out_sl):
-    _count()
-    check(LIB.nfk_invconv_prep(_p(an_bias), _p(an_logs), _p(lower), _p(upper), _p(log_s), _p(p), _p(sign_s),
-                               _p(weight), C, int(reverse), int(transpose), _p(outW), _p(outb), _p(out_sl), _st()),
-          "nfk_invconv_prep")
-
-
-def invconv_prep_bwd(an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose, Wf, dWf, dbf,
-                     g_ld, B, pixels, d_bias, d_logs, d_lower, d_upper, d_log_s, d_weight):
-    _count()
-    check(LIB.nfk_invconv_prep_bwd(_p(an_bias), _p(an_logs), _p(lower), _p(upper), _p(log_s), _p(p), _p(sign_s),
-                                   _p(weight), C, int(reverse), int(transpose), _p(Wf), _p(dWf), _p(dbf), _p(g_ld),
-                                   B,
-                                   float(pixels), _p(d_bias), _p(d_logs), _p(d_lower), _p(d_upper), _p(d_log_s),
-                                   _p(d_weight), _st()), "nfk_invconv_prep_bwd")
-
-
 def invconv_item(an_bias, an_logs, lower, upper, log_s, p, sign_s, weight, C, reverse, transpose, outW, outb, out_sl):
-    """One nfk_invconv_item (the argument list of invconv_prep) for the batched launch."""
+    """One nfk_invconv_item (include/nfk.h) for invconv_prep_batch."""
     from ._lib import InvconvItem
     return InvconvItem(_p(an_bias), _p(an_logs), _p(lower), _p(upper), _p(log_s), _p(p), _p(sign_s), _p(weight), C,
                        int(reverse), int(transpose), _p(outW), _p(outb), _p(out_sl))
@@ -155,23 +138,6 @@ def coupling_prep_bwd_batch(items):
     arr = (CouplingBwdItem * n)(*items)
     _count((n + 11) // 12)
     check(LIB.nfk_coupling_prep_bwd_batch(n, ctypes.addressof(arr), _st()), "nfk_coupling_prep_bwd_batch")
-
-
-def coupling_prep(w1, b1, l1, w2, b2, l2, w3, b3, l3, cin, hid, cout, K1p, K3p, B1, B1T, B2, B2T, B3, B3T, bias1,
-                  bias2, bias3, with_t):
-    _count()
-    check(LIB.nfk_coupling_prep(_p(w1), _p(b1), _p(l1), _p(w2), _p(b2), _p(l2), _p(w3), _p(b3), _p(l3), cin, hid,
-                                cout, K1p, K3p, _p(B1), _p(B1T), _p(B2), _p(B2T), _p(B3), _p(B3T), _p(bias1),
-                                _p(bias2), _p(bias3), int(with_t), _st()), "nfk_coupling_prep")
-
-
-def coupling_prep_bwd(w1, b1, l1, w2, b2, l2, w3, b3, l3, cin, hid, cout, K1p, K3p, dB1, dbias1, dB2, dbias2, dB3,
-                      dbias3, dw1, db1, dl1, dw2, db2, dl2, dw3, db3, dl3):
-    _count()
-    check(LIB.nfk_coupling_prep_bwd(_p(w1), _p(b1), _p(l1), _p(w2), _p(b2), _p(l2), _p(w3), _p(b3), _p(l3), cin, hid,
-                                    cout, K1p, K3p, _p(dB1), _p(dbias1), _p(dB2), _p(dbias2), _p(dB3), _p(dbias3),
-                                    _p(dw1), _p(db1), _p(dl1), _p(dw2), _p(db2), _p(dl2), _p(dw3), _p(db3), _p(dl3),
-                                    _st()), "nfk_coupling_prep_bwd")
 
 
 def affine1x1_fwd(x, Wf, bf, sl, y, col, K1p, ld_in, ld_out, B, C, H, W):

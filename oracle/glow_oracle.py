@@ -165,7 +165,7 @@ def invconv(x: Tensor, sd: SD, pre: str, logdet, reverse: bool) -> Tuple[Tensor,
 def conv_actnorm(x: Tensor, sd: SD, pre: str) -> Tensor:
     """Conv2d: zero-pad 'same' -> bias-free conv -> ActNorm affine (models/layers.py:190-228)."""
     w = sd[pre + "conv.weight"]
-    if _BF16["on"]:   # folded operand bf16(w * exp(logs)) and fp32 bias b * exp(logs) (csrc/prep.cu::coupling_prep)
+    if _BF16["on"]:   # folded operand bf16(w * exp(logs)) and fp32 bias b * exp(logs) (prep.cu coupling_prep_kernel)
         e = torch.exp(sd[pre + "actnorm.logs"])                      # [1, Cout, 1, 1]
         wf = _q(w * e.view(-1, 1, 1, 1))
         y = F.conv2d(_q(x), wf, padding=(w.shape[2] // 2, w.shape[3] // 2))

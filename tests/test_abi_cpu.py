@@ -31,7 +31,14 @@ def test_argument_errors_without_gpu():
     L = _lib.LIB
     assert L.nfk_gemm_nt_bf16(None, 64, None, 64, 128, 100, 64, 0, None, 64, None, None, 0, None, None) == -1
     assert L.nfk_gemm_nt_bf16(None, 64, None, 64, 128, 64, 60, 0, None, 64, None, None, 0, None, None) == -1
-    assert L.nfk_invconv_prep(None, None, None, None, None, None, None, None, 12, 0, 0, None, None, None, None) == -3
+    inv = _lib.InvconvItem(C=12)                        # every pointer NULL
+    assert L.nfk_invconv_prep_batch(1, ctypes.addressof(inv), None) == -3
+    inv.C = 105                                         # C <= 104
+    assert L.nfk_invconv_prep_batch(1, ctypes.addressof(inv), None) == -1
+    cp = _lib.CouplingItem(cin=6, hid=512, cout=12, K1p=64, K3p=128)
+    assert L.nfk_coupling_prep_batch(1, ctypes.addressof(cp), None) == -3
+    cp.K3p = 64                                         # K3p < 9 * cout
+    assert L.nfk_coupling_prep_batch(1, ctypes.addressof(cp), None) == -1
     assert L.nfk_affine1x1_fwd(None, None, None, None, None, None, 0, None, None, 0, 12, 4, 4, None) == -1
     assert L.nfk_kd_mse_fwd(None, None, 4, 16, 1.0, None, None) == -3
 
